@@ -289,6 +289,32 @@ int ssb200_radsurf_sp(const ssb200_config *config,
                       ssb200_canopy_flux_sp *lw_internal,
                       ssb200_canopy_flux_sp *lw_norm);
 
+/* ssb200_radsurf_fluxes for a `-DSINGLE_PRECISION` host: the reference driver's sequence
+ * (driver/spartacus_surface_driver.F90:206-261, as ssb200_radsurf_fluxes above) with float arrays.
+ * ssb200_driver_inputs_sp has the members of ssb200_driver_inputs as `const float *`.  NULL members
+ * take read_input's defaults and the LW emission is derived from the temperatures exactly as in
+ * ssb200_radsurf_fluxes.  The arrays cross PCIe as float (half the bytes of the double entry), are
+ * widened on the device, the solve, the sigma T^4 emission and the scale + sum run in FP64, and every
+ * output is the FP64 result rounded to nearest float: bit-equal to ssb200_radsurf_fluxes on the widened
+ * inputs followed by a cast.  HOST pointers; same return convention as ssb200_radsurf. */
+typedef struct ssb200_driver_inputs_sp {
+  const float *top_flux_dn_sw;
+  const float *top_flux_dn_direct_sw;
+  const float *top_flux_dn_lw;
+  const float *ground_temperature;
+  const float *roof_temperature, *wall_temperature;
+  const float *clear_air_temperature, *veg_temperature, *veg_air_temperature;
+} ssb200_driver_inputs_sp;
+
+int ssb200_radsurf_fluxes_sp(const ssb200_config *config,
+                             const ssb200_canopy_properties_sp *canopy_props,
+                             const ssb200_sw_spectral_properties_sp *sw_spectral_props,
+                             const ssb200_lw_spectral_properties_sp *lw_spectral_props,
+                             const ssb200_driver_inputs_sp *driver_inputs,
+                             ssb200_boundary_conds_out_sp *bc_out,
+                             int32_t istartcol, int32_t iendcol,
+                             ssb200_canopy_flux_sp *sw_flux, ssb200_canopy_flux_sp *lw_flux);
+
 /* Device-resident variant.  The three per-column index arrays of
  * `canopy_props` (nlay, istartlay, i_representation) stay HOST pointers (they
  * define the launch plan, which is cached between calls while they do not
@@ -311,6 +337,31 @@ int ssb200_radsurf_device(const ssb200_config *config,
                           ssb200_canopy_flux *lw_internal,
                           ssb200_canopy_flux *lw_norm,
                           void *stream, int32_t *status_out);
+
+/* ssb200_radsurf_device for float device arrays: replaces the body of `radsurf`
+ * (radsurf/radsurf_interface.F90:20-317) for a `-DSINGLE_PRECISION` caller whose arrays live in HBM.
+ * Every float array is a DEVICE pointer; nlay, istartlay and i_representation stay HOST arrays.  The
+ * call is asynchronous on `stream`, shares the one context of the other entries and is ordered against
+ * calls from other streams exactly as ssb200_radsurf_device.  The solve runs in FP64 and every output
+ * is the FP64 result rounded to nearest float: bit-equal to ssb200_radsurf_device on the widened inputs
+ * followed by a cast; entries the solve leaves untouched keep the caller's value, and columns outside
+ * istartcol..iendcol are not written.  No full double copy of the inputs is made when every per-layer
+ * read of the call goes through the level-major staging ("stage_layers", the register-resident kernels
+ * of 1-4 streams, no "fused_kernels", no SimpleUrban / InfiniteStreet column): the staging widens and
+ * rounds the per-layer arrays as it moves them, and only the per-column members are widened into
+ * double buffers of the context.  Otherwise the per-layer arrays of the call's packed layers are
+ * widened into double buffers too and rounded back.  Same return convention as ssb200_radsurf_device. */
+int ssb200_radsurf_device_sp(const ssb200_config *config,
+                             const ssb200_canopy_properties_sp *canopy_props,
+                             const ssb200_sw_spectral_properties_sp *sw_spectral_props,
+                             const ssb200_lw_spectral_properties_sp *lw_spectral_props,
+                             ssb200_boundary_conds_out_sp *bc_out,
+                             int32_t istartcol, int32_t iendcol,
+                             ssb200_canopy_flux_sp *sw_norm_dir,
+                             ssb200_canopy_flux_sp *sw_norm_diff,
+                             ssb200_canopy_flux_sp *lw_internal,
+                             ssb200_canopy_flux_sp *lw_norm,
+                             void *stream, int32_t *status_out);
 
 /* Number of kernels launched by this process through the library so far
  * (bench.py reports the per-step delta as `gpu_launches`). */

@@ -40,6 +40,11 @@ def _declare(lib):
     lib.ssb200_radsurf_fluxes.argtypes = (radsurf_args[:4] + [P(_abi.DriverInputs)] + radsurf_args[4:7]
                                           + [P(_abi.CanopyFlux), P(_abi.CanopyFlux)])
     lib.ssb200_radsurf_fluxes.restype = C.c_int
+    # (the _sp structs, ssb200_driver_inputs_sp included, are layout-identical to the double ones)
+    lib.ssb200_radsurf_fluxes_sp.argtypes = lib.ssb200_radsurf_fluxes.argtypes
+    lib.ssb200_radsurf_fluxes_sp.restype = C.c_int
+    lib.ssb200_radsurf_device_sp.argtypes = lib.ssb200_radsurf_device.argtypes
+    lib.ssb200_radsurf_device_sp.restype = C.c_int
     lib.ssb200_kernel_launch_count.restype = C.c_int64
     lib.ssb200_set_profiling.argtypes = [C.c_int]
     lib.ssb200_last_kernel_times_ms.argtypes = [P(C.c_double)]

@@ -46,12 +46,13 @@ __global__ void k_surface(ssb::SurfaceArgs s, int nsw_threads, int nlw_threads) 
 // The key is packed into as few bits as it needs - `lbits` for the segment pattern (one bit per
 // layer; night-time columns get the largest value) below the group index - so that the radix sort
 // runs 3 passes instead of 8: at 131,072 columns per GPU (8-GPU sharding) the sort is latency, not
-// bandwidth.
+// bandwidth.  T: element type of the per-layer fractions (float: ssb200_radsurf_device_sp).
+template <class T>
 __global__ void k_column_keys(ssb::ClassArgs a, unsigned long long *keys, int group, int lbits) {
   const int ic = blockIdx.x * blockDim.x + threadIdx.x;
   if (ic >= a.ncols) return;
   const unsigned long long all = (1ull << lbits) - 1ull;
-  const unsigned pattern = ssb::column_segment_key(a, a.cols[ic]);
+  const unsigned pattern = ssb::column_segment_key<T>(a, a.cols[ic]);
   const unsigned long long k = (pattern == 0xffffffffu) ? all : ((unsigned long long)pattern & (all >> 1));
   keys[ic] = ((unsigned long long)(ic / group) << lbits) | k;
 }
@@ -139,6 +140,35 @@ __global__ void k_f2d(double *dst, const float *src, size_t n) {
 __global__ void k_d2f(float *dst, const double *src, size_t n) {
   const size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x;
   if (i < n) dst[i] = (float)src[i];  // round to nearest even
+}
+
+// ---- ssb200_radsurf_device_sp: float device arrays around the FP64 solve ----------------------
+// element ranges [lo, hi) of a list of arrays, widened (d = f, exact) before the solve or rounded to
+// nearest (f = d) after it, one launch per direction
+constexpr int kConvMax = 48;
+struct ConvList {
+  float *f[kConvMax];
+  double *d[kConvMax];
+  long lo[kConvMax], hi[kConvMax];
+  int n;
+};
+struct ConvArray {
+  float *f;
+  double *d;
+  long lo, hi;
+  bool out;  // rounded back after the solve
+};
+template <bool ROUND>
+__global__ void k_convert(ConvList cl) {
+  const long t = blockIdx.x * (long)blockDim.x + threadIdx.x;
+  for (int k = 0; k < cl.n; ++k) {
+    const long i = cl.lo[k] + t;
+    if (i >= cl.hi[k]) continue;
+    if (ROUND)
+      cl.f[k][i] = __double2float_rn(cl.d[k][i]);
+    else
+      cl.d[k][i] = (double)cl.f[k][i];
+  }
 }
 
 // ---- stages around radsurf for ssb200_radsurf_fluxes ----------------------------------------
@@ -236,6 +266,7 @@ struct Context {
   int pipeline = 1;
   int pipeline_max_blocks = 16;
   std::vector<DevBuf> stage;  // staging mirrors of host arrays for ssb200_radsurf
+  std::vector<DevBuf> wide;   // double copies of float device arrays for ssb200_radsurf_device_sp
   cudaStream_t stream = nullptr;
   cudaStream_t own_stream = nullptr;
   size_t budget_doubles = 0;
@@ -286,6 +317,7 @@ struct CudaBackend {
   bool forked = false;
   size_t budget;
   bool layer_was_fast = false;  // the chunk's layer kernels were the register-resident ones
+  bool f32_layers = false;      // per-layer members are the caller's float arrays (ssb200_radsurf_device_sp)
   explicit CudaBackend(Context &c, int lane_ = 0, size_t budget_ = 0)
       : cx(c), lane(lane_), pass_lane(lane_), main_stream(c.stream), budget(budget_ ? budget_ : c.budget_doubles) {}
   // Shortwave pass on the stream of the call, longwave pass on an auxiliary stream with its own
@@ -343,7 +375,10 @@ struct CudaBackend {
     int gbits = 0;
     for (size_t ngroups = (n + (size_t)group - 1) / (size_t)group; ((size_t)1 << gbits) < ngroups; ++gbits) {
     }
-    k_column_keys<<<(unsigned)((n + 127) / 128), 128, 0, cx.stream>>>(a, keys, group, lbits);
+    if (f32_layers)
+      k_column_keys<float><<<(unsigned)((n + 127) / 128), 128, 0, cx.stream>>>(a, keys, group, lbits);
+    else
+      k_column_keys<double><<<(unsigned)((n + 127) / 128), 128, 0, cx.stream>>>(a, keys, group, lbits);
     cub::DeviceRadixSort::SortPairs(base, temp_bytes, keys, keys_out, a.cols, cols_out, (int)n, 0, lbits + gbits,
                                     cx.stream);
     g_launches += 2;
@@ -586,6 +621,33 @@ int upload_plan(Context &cx, const ssb200_canopy_properties &cp) {
   return 0;
 }
 
+// Runs the prepared plan on cx.stream.  f32_layers: the per-layer members of `ca` are float arrays that
+// only the level-major staging touches (ssb200_radsurf_device_sp, staged route).
+int dispatch_call(Context &cx, const ssb::CallArgs &ca, bool f32_layers) {
+  std::string err;
+  CudaBackend be(cx);
+  be.f32_layers = f32_layers;
+  ssb::Dispatcher<CudaBackend> disp(be);
+  disp.f32_layers = f32_layers;
+  const int rc = disp.run(ca, cx.plan, err);
+  if (rc) return fail(rc, err);
+  if (cx.first_error != cudaSuccess)
+    return fail(SSB200_ERR_CUDA, std::string("kernel launch / scratch allocation: ") + cudaGetErrorString(cx.first_error));
+  return 0;
+}
+
+// End of a device-entry call: status word to the caller, and the event that a later call on another
+// stream waits for before it reuses the context's buffers.
+int finish_device_call(Context &cx, cudaStream_t stream, int32_t *status_out) {
+  if (status_out)
+    SSB_CUDA(cudaMemcpyAsync(status_out, cx.d_status.p, sizeof(int), cudaMemcpyDeviceToDevice, stream));
+  if (!cx.ev_done) SSB_CUDA(cudaEventCreateWithFlags(&cx.ev_done, cudaEventDisableTiming));
+  SSB_CUDA(cudaEventRecord(cx.ev_done, stream));
+  cx.last_stream = stream;
+  cx.last_stream_valid = true;
+  return 0;
+}
+
 // Core of both entry points; all double arrays are device pointers here.
 // `blocks`: when non-null the call only prepares (plan, status, budget) and returns the
 // clamped 1-based column range in blocks[0..1]; the caller then dispatches column
@@ -641,19 +703,9 @@ int radsurf_device_locked(Context &cx, const ssb::CallArgs &ca, int istartcol, i
     blocks[1] = c2;
     return 0;
   }
-  CudaBackend be(cx);
-  ssb::Dispatcher<CudaBackend> disp(be);
-  rc = disp.run(ca, cx.plan, err);
-  if (rc) return fail(rc, err);
-  if (cx.first_error != cudaSuccess)
-    return fail(SSB200_ERR_CUDA, std::string("kernel launch / scratch allocation: ") + cudaGetErrorString(cx.first_error));
-  if (status_out)
-    SSB_CUDA(cudaMemcpyAsync(status_out, cx.d_status.p, sizeof(int), cudaMemcpyDeviceToDevice, stream));
-  if (!cx.ev_done) SSB_CUDA(cudaEventCreateWithFlags(&cx.ev_done, cudaEventDisableTiming));
-  SSB_CUDA(cudaEventRecord(cx.ev_done, stream));
-  cx.last_stream = stream;
-  cx.last_stream_valid = true;
-  return 0;
+  rc = dispatch_call(cx, ca, false);
+  if (rc) return rc;
+  return finish_device_call(cx, stream, status_out);
 }
 
 // dispatch the columns [col_lo, col_hi) (0-based) of the prepared plan on one lane
@@ -716,6 +768,39 @@ static int collect_fields(ssb200_canopy_flux *o, const ssb200_canopy_flux *a, co
   }
 #undef F
   return fl.n;
+}
+
+// widen every array of `v` (round = false) or round its outputs back (true) on `st`, kConvMax arrays per launch
+int convert_arrays(const std::vector<ConvArray> &v, bool round, cudaStream_t st) {
+  ConvList cl;
+  cl.n = 0;
+  long most = 0;
+  auto flush = [&]() -> int {
+    if (cl.n > 0 && most > 0) {
+      const unsigned blocks = (unsigned)((most + 255) / 256);
+      if (round)
+        k_convert<true><<<blocks, 256, 0, st>>>(cl);
+      else
+        k_convert<false><<<blocks, 256, 0, st>>>(cl);
+      ++g_launches;
+      SSB_CUDA(cudaGetLastError());
+    }
+    cl.n = 0;
+    most = 0;
+    return 0;
+  };
+  for (const ConvArray &c : v) {
+    if ((round && !c.out) || c.hi <= c.lo) continue;
+    cl.f[cl.n] = c.f;
+    cl.d[cl.n] = c.d;
+    cl.lo[cl.n] = c.lo;
+    cl.hi[cl.n] = c.hi;
+    ++cl.n;
+    most = std::max(most, c.hi - c.lo);
+    if (cl.n == kConvMax)
+      if (int rc = flush()) return rc;
+  }
+  return flush();
 }
 
 // --- host-pointer staging --------------------------------------------------
@@ -907,6 +992,166 @@ int ssb200_radsurf_device(const ssb200_config *config, const ssb200_canopy_prope
   std::lock_guard<std::mutex> lock(g_mutex);
   ssb::CallArgs ca{config, canopy_props, sw, lw, bc_out, sw_norm_dir, sw_norm_diff, lw_internal, lw_norm};
   return radsurf_device_locked(g_ctx, ca, istartcol, iendcol, (cudaStream_t)stream, status_out);
+}
+
+// Body of ssb200_radsurf_device_sp: every real array of `ca` is a float device array.  The per-column
+// members (cos_sza, ground_*, bc_out, the per-column flux members: 1/16 of the data at 16 layers) are
+// widened into double buffers of the context for the call's columns and rounded back after the solve.
+// The per-layer members take one of two routes, chosen per call from the plan:
+//   staged:   every class and pass reads and writes them through the level-major staging only, whose
+//             gather widens (float -> double) and whose scatter rounds (double -> float): no double copy;
+//   fallback: some read happens outside the staging (generic kernels, stage_layers = 0, column-resident
+//             kernels, single-layer urban columns on the surface kernel): the packed layers of the call's
+//             columns are widened into double copies and rounded back, as ssb200_radsurf_sp does.
+// Either way the kernels see the doubles the double entry sees on widened inputs, and entries the
+// solve leaves untouched round back to the caller's value.
+static int radsurf_device_sp_locked(Context &cx, const ssb::CallArgs &ca, int32_t istartcol, int32_t iendcol,
+                                    cudaStream_t stream, int32_t *status_out) {
+  int range[2] = {1, 0};
+  int rc = radsurf_device_locked(cx, ca, istartcol, iendcol, stream, nullptr, range);
+  if (rc || range[0] > range[1]) return rc;
+  const ssb200_config &cfg = *ca.config;
+  const ssb200_canopy_properties &cp = *ca.cp;
+  CudaBackend probe(cx);
+  ssb::Dispatcher<CudaBackend> route(probe);
+  const bool staged = route.all_layers_staged(ca, cx.plan);
+  const size_t ncol = (size_t)cp.ncol, ntot = (size_t)cp.ntotlay;
+  const size_t c0 = (size_t)range[0] - 1, c1 = (size_t)range[1];
+  size_t l0 = ntot, l1 = 0;  // packed layers of the call's columns (fallback route)
+  if (!staged)
+    for (size_t j = c0; j < c1; ++j)
+      if (cp.i_representation[j] != SSB200_TILE_FLAT && cp.nlay[j] > 0) {
+        l0 = std::min(l0, (size_t)cp.istartlay[j] - 1);
+        l1 = std::max(l1, (size_t)cp.istartlay[j] - 1 + (size_t)cp.nlay[j]);
+      }
+  if (l1 < l0) l0 = l1 = 0;
+  std::vector<ConvArray> conv;
+  size_t next = 0;
+  int err_rc = 0;
+  // double buffer for the float array p of `rows` x `width` values; rows [r0, r1) are converted
+  auto wide = [&](const void *p, size_t rows, size_t width, size_t r0, size_t r1, bool out) -> double * {
+    if (!p || err_rc) return nullptr;
+    if (next >= cx.wide.size()) cx.wide.resize(next + 16);
+    DevBuf &b = cx.wide[next++];
+    const cudaError_t e = b.reserve(std::max(rows * width, (size_t)1) * sizeof(double));
+    if (e != cudaSuccess) {
+      err_rc = fail(SSB200_ERR_CUDA, std::string("double copies: ") + cudaGetErrorString(e));
+      return nullptr;
+    }
+    conv.push_back(ConvArray{(float *)p, (double *)b.p, (long)(r0 * width), (long)(r1 * width), out});
+    return (double *)b.p;
+  };
+  auto C = [&](const void *p, size_t w, bool out) { return wide(p, ncol, w, c0, c1, out); };
+  auto L = [&](const void *p, size_t w, bool out) { return staged ? (double *)p : wide(p, ntot, w, l0, l1, out); };
+  ssb200_canopy_properties dcp = cp;
+  dcp.cos_sza = C(cp.cos_sza, 1, false);
+  dcp.dz = L(cp.dz, 1, false);
+  dcp.building_fraction = L(cp.building_fraction, 1, false);
+  dcp.building_scale = L(cp.building_scale, 1, false);
+  dcp.veg_fraction = L(cp.veg_fraction, 1, false);
+  dcp.veg_scale = L(cp.veg_scale, 1, false);
+  dcp.veg_ext = L(cp.veg_ext, 1, false);
+  dcp.veg_fsd = L(cp.veg_fsd, 1, false);
+  dcp.veg_contact_fraction = L(cp.veg_contact_fraction, 1, false);
+  ssb200_sw_spectral_properties dsw;
+  ssb200_lw_spectral_properties dlw;
+  ssb200_boundary_conds_out dbc;
+  memset(&dsw, 0, sizeof(dsw));
+  memset(&dlw, 0, sizeof(dlw));
+  memset(&dbc, 0, sizeof(dbc));
+  if (cfg.do_sw) {
+    const ssb200_sw_spectral_properties &sw = *ca.sw;
+    const size_t g = (size_t)cfg.nsw;
+    dsw.nspec = sw.nspec;
+    dsw.air_ext = L(sw.air_ext, g, false);
+    dsw.air_ssa = L(sw.air_ssa, g, false);
+    dsw.veg_ssa = L(sw.veg_ssa, g, false);
+    dsw.ground_albedo = C(sw.ground_albedo, g, false);
+    dsw.roof_albedo = L(sw.roof_albedo, g, false);
+    dsw.wall_albedo = L(sw.wall_albedo, g, false);
+    dsw.wall_specular_frac = L(sw.wall_specular_frac, g, false);
+    dsw.ground_albedo_dir = C(sw.ground_albedo_dir, g, false);
+    dsw.roof_albedo_dir = L(sw.roof_albedo_dir, g, false);
+    dbc.sw_albedo = C(ca.bc->sw_albedo, g, true);
+    dbc.sw_albedo_dir = C(ca.bc->sw_albedo_dir, g, true);
+  }
+  if (cfg.do_lw) {
+    const ssb200_lw_spectral_properties &lw = *ca.lw;
+    const size_t g = (size_t)cfg.nlw;
+    dlw.nspec = lw.nspec;
+    dlw.air_ext = L(lw.air_ext, g, false);
+    dlw.air_ssa = L(lw.air_ssa, g, false);
+    dlw.clear_air_planck = L(lw.clear_air_planck, g, false);
+    dlw.veg_ssa = L(lw.veg_ssa, g, false);
+    dlw.veg_planck = L(lw.veg_planck, g, false);
+    dlw.veg_air_planck = L(lw.veg_air_planck, g, false);
+    dlw.ground_emissivity = C(lw.ground_emissivity, g, false);
+    dlw.ground_emission = C(lw.ground_emission, g, false);
+    dlw.roof_emissivity = L(lw.roof_emissivity, g, false);
+    dlw.wall_emissivity = L(lw.wall_emissivity, g, false);
+    dlw.roof_emission = L(lw.roof_emission, g, false);
+    dlw.wall_emission = L(lw.wall_emission, g, false);
+    dbc.lw_emissivity = C(ca.bc->lw_emissivity, g, true);
+    dbc.lw_emission = C(ca.bc->lw_emission, g, true);
+  }
+  auto flux = [&](const ssb200_canopy_flux *h, ssb200_canopy_flux &d) {
+    d = *h;
+    const size_t g = (size_t)h->nspec;
+    d.ground_dn = C(h->ground_dn, g, true);
+    d.ground_net = C(h->ground_net, g, true);
+    d.ground_vertical_diff = C(h->ground_vertical_diff, g, true);
+    d.top_dn = C(h->top_dn, g, true);
+    d.top_net = C(h->top_net, g, true);
+    d.ground_dn_dir = C(h->ground_dn_dir, g, true);
+    d.top_dn_dir = C(h->top_dn_dir, g, true);
+    d.ground_sunlit_frac = C(h->ground_sunlit_frac, 1, true);
+    d.roof_in = L(h->roof_in, g, true);
+    d.roof_net = L(h->roof_net, g, true);
+    d.wall_in = L(h->wall_in, g, true);
+    d.wall_net = L(h->wall_net, g, true);
+    d.roof_in_dir = L(h->roof_in_dir, g, true);
+    d.wall_in_dir = L(h->wall_in_dir, g, true);
+    d.roof_sunlit_frac = L(h->roof_sunlit_frac, 1, true);
+    d.wall_sunlit_frac = L(h->wall_sunlit_frac, 1, true);
+    d.clear_air_abs = L(h->clear_air_abs, g, true);
+    d.veg_abs = L(h->veg_abs, g, true);
+    d.veg_air_abs = L(h->veg_air_abs, g, true);
+    d.veg_abs_dir = L(h->veg_abs_dir, g, true);
+    d.veg_sunlit_frac = L(h->veg_sunlit_frac, 1, true);
+    d.flux_dn_layer_top = L(h->flux_dn_layer_top, g, true);
+    d.flux_up_layer_top = L(h->flux_up_layer_top, g, true);
+    d.flux_dn_layer_base = L(h->flux_dn_layer_base, g, true);
+    d.flux_up_layer_base = L(h->flux_up_layer_base, g, true);
+    d.flux_dn_dir_layer_top = L(h->flux_dn_dir_layer_top, g, true);
+    d.flux_dn_dir_layer_base = L(h->flux_dn_dir_layer_base, g, true);
+  };
+  ssb200_canopy_flux d1, d2, d3, d4;
+  if (cfg.do_sw) {
+    flux(ca.sw_dir, d1);
+    flux(ca.sw_diff, d2);
+  }
+  if (cfg.do_lw) {
+    flux(ca.lw_int, d3);
+    flux(ca.lw_norm, d4);
+  }
+  if (err_rc) return err_rc;
+  ssb::CallArgs wca{ca.config, &dcp, cfg.do_sw ? &dsw : nullptr, cfg.do_lw ? &dlw : nullptr, &dbc,
+                    cfg.do_sw ? &d1 : nullptr, cfg.do_sw ? &d2 : nullptr,
+                    cfg.do_lw ? &d3 : nullptr, cfg.do_lw ? &d4 : nullptr};
+  // an error return after the first launch must not leave work queued on the context's buffers (a later
+  // call on another stream, or ssb200_release, would not wait for it)
+  struct Drain {
+    cudaStream_t s;
+    bool armed = true;
+    ~Drain() {
+      if (armed) cudaStreamSynchronize(s);
+    }
+  } drain{stream};
+  if ((rc = convert_arrays(conv, false, stream))) return rc;
+  if ((rc = dispatch_call(cx, wca, staged))) return rc;
+  if ((rc = convert_arrays(conv, true, stream))) return rc;
+  drain.armed = false;
+  return finish_device_call(cx, stream, status_out);
 }
 
 // Body of both host entries.  drv == NULL: ssb200_radsurf (the four normalised flux objects are
@@ -1321,7 +1566,8 @@ int ssb200_radsurf_sp(const ssb200_config *config, const ssb200_canopy_propertie
                     sizeof(ssb200_sw_spectral_properties_sp) == sizeof(ssb200_sw_spectral_properties) &&
                     sizeof(ssb200_lw_spectral_properties_sp) == sizeof(ssb200_lw_spectral_properties) &&
                     sizeof(ssb200_canopy_flux_sp) == sizeof(ssb200_canopy_flux) &&
-                    sizeof(ssb200_boundary_conds_out_sp) == sizeof(ssb200_boundary_conds_out),
+                    sizeof(ssb200_boundary_conds_out_sp) == sizeof(ssb200_boundary_conds_out) &&
+                    sizeof(ssb200_driver_inputs_sp) == sizeof(ssb200_driver_inputs),
                 "single-precision structs must mirror the double-precision ones");
   return radsurf_host(config, reinterpret_cast<const ssb200_canopy_properties *>(cp),
                       reinterpret_cast<const ssb200_sw_spectral_properties *>(sw),
@@ -1330,6 +1576,40 @@ int ssb200_radsurf_sp(const ssb200_config *config, const ssb200_canopy_propertie
                       reinterpret_cast<ssb200_canopy_flux *>(sw_dir), reinterpret_cast<ssb200_canopy_flux *>(sw_diff),
                       reinterpret_cast<ssb200_canopy_flux *>(lw_int), reinterpret_cast<ssb200_canopy_flux *>(lw_norm), nullptr,
                       nullptr, true);
+}
+
+int ssb200_radsurf_fluxes_sp(const ssb200_config *config, const ssb200_canopy_properties_sp *cp,
+                             const ssb200_sw_spectral_properties_sp *sw, const ssb200_lw_spectral_properties_sp *lw,
+                             const ssb200_driver_inputs_sp *drv, ssb200_boundary_conds_out_sp *bc, int32_t istartcol,
+                             int32_t iendcol, ssb200_canopy_flux_sp *sw_flux, ssb200_canopy_flux_sp *lw_flux) {
+  if (!drv) return fail(SSB200_ERR_ARG, "driver_inputs must not be NULL");
+  return radsurf_host(config, reinterpret_cast<const ssb200_canopy_properties *>(cp),
+                      reinterpret_cast<const ssb200_sw_spectral_properties *>(sw),
+                      reinterpret_cast<const ssb200_lw_spectral_properties *>(lw),
+                      reinterpret_cast<const ssb200_driver_inputs *>(drv), reinterpret_cast<ssb200_boundary_conds_out *>(bc),
+                      istartcol, iendcol, nullptr, nullptr, nullptr, nullptr, reinterpret_cast<ssb200_canopy_flux *>(sw_flux),
+                      reinterpret_cast<ssb200_canopy_flux *>(lw_flux), true);
+}
+
+int ssb200_radsurf_device_sp(const ssb200_config *config, const ssb200_canopy_properties_sp *cp,
+                             const ssb200_sw_spectral_properties_sp *sw, const ssb200_lw_spectral_properties_sp *lw,
+                             ssb200_boundary_conds_out_sp *bc, int32_t istartcol, int32_t iendcol,
+                             ssb200_canopy_flux_sp *sw_norm_dir, ssb200_canopy_flux_sp *sw_norm_diff,
+                             ssb200_canopy_flux_sp *lw_internal, ssb200_canopy_flux_sp *lw_norm, void *stream,
+                             int32_t *status_out) {
+  int rc = ensure_device();
+  if (rc) return rc;
+  std::lock_guard<std::mutex> lock(g_mutex);
+  ssb::CallArgs ca{config,
+                   reinterpret_cast<const ssb200_canopy_properties *>(cp),
+                   reinterpret_cast<const ssb200_sw_spectral_properties *>(sw),
+                   reinterpret_cast<const ssb200_lw_spectral_properties *>(lw),
+                   reinterpret_cast<ssb200_boundary_conds_out *>(bc),
+                   reinterpret_cast<ssb200_canopy_flux *>(sw_norm_dir),
+                   reinterpret_cast<ssb200_canopy_flux *>(sw_norm_diff),
+                   reinterpret_cast<ssb200_canopy_flux *>(lw_internal),
+                   reinterpret_cast<ssb200_canopy_flux *>(lw_norm)};
+  return radsurf_device_sp_locked(g_ctx, ca, istartcol, iendcol, (cudaStream_t)stream, status_out);
 }
 
 int64_t ssb200_kernel_launch_count(void) { return (int64_t)g_launches; }
@@ -1434,6 +1714,7 @@ int ssb200_release(void) {
       cx.d_sort[l].release();
     }
     for (DevBuf &b : cx.stage) b.release();
+    for (DevBuf &b : cx.wide) b.release();
   }
   cx.plan = ssb::Plan();
   cx.plan_uploaded = false;

@@ -22,7 +22,9 @@ namespace ssb {
 
 // Lists the per-layer arrays of a pass and redirects the members of `b` to their level-major staging
 // buffers (ssb_stage.cuh), carved from `cursor` (NULL: only count).  Returns doubles per (level, column).
-inline size_t stage_plan(ClassArgs &b, bool lw, size_t per_elem, double *cursor, StageList *in, StageList *out) {
+// f32: the members of `b` are the caller's float arrays (ssb200_radsurf_device_sp).
+inline size_t stage_plan(ClassArgs &b, bool lw, size_t per_elem, double *cursor, StageList *in, StageList *out,
+                         bool f32 = false) {
   size_t elems = 0;
   auto add = [&](StageList *list, double *&member, int ns) {
     if (!member) return;
@@ -31,6 +33,7 @@ inline size_t stage_plan(ClassArgs &b, bool lw, size_t per_elem, double *cursor,
     list->ref[list->n] = member;
     list->staged[list->n] = cursor;
     list->nspec[list->n] = ns;
+    list->f32[list->n] = f32 ? 1 : 0;
     ++list->n;
     member = cursor;
     cursor += (size_t)ns * per_elem;
@@ -248,7 +251,45 @@ struct Dispatcher {
   // optional window of global column indices [col_lo, col_hi): lets the host entry
   // pipeline transfers and kernels over blocks of columns without rebuilding the plan
   int col_lo = 0, col_hi = 0x7fffffff;
+  // the per-layer members of the call are the caller's float arrays, read and written through the
+  // level-major staging only (ssb200_radsurf_device_sp; see all_layers_staged)
+  bool f32_layers = false;
   explicit Dispatcher(Backend &b) : be(b) {}
+
+  static SolveCfg class_cfg(const ssb200_config &cfg, const ColumnClass &k, bool lw) {
+    const ssb200_legendre_gauss &lgs =
+        lw ? (k.urban ? cfg.lg_lw_urban : cfg.lg_lw_forest) : (k.urban ? cfg.lg_sw_urban : cfg.lg_sw_forest);
+    SolveCfg c;
+    std::memset(&c, 0, sizeof(c));
+    c.urban = k.urban;
+    c.lw = lw ? 1 : 0;
+    c.nreg = k.nreg;
+    c.ns = lgs.nstream;
+    c.nspec = lw ? cfg.nlw : cfg.nsw;
+    c.symmetric_scale = k.urban ? cfg.use_symmetric_vegetation_scale_urban : cfg.use_symmetric_vegetation_scale_forest;
+    c.isolation = k.urban ? cfg.vegetation_isolation_factor_urban : cfg.vegetation_isolation_factor_forest;
+    c.min_veg = cfg.min_vegetation_fraction;
+    c.min_bld = cfg.min_building_fraction;
+    return c;
+  }
+
+  // True when every read and write of a per-layer member in the plan goes through the level-major
+  // staging: each class and pass is staged (no column-resident kernels, no unstaged split kernels) and
+  // no single-layer urban column is present (the surface kernel reads and writes its layer in place).
+  bool all_layers_staged(const CallArgs &ca, const Plan &plan) {
+    const ssb200_config &cfg = *ca.config;
+    for (int j : plan.surface_cols)
+      if (plan.irep[j] == SSB200_TILE_SIMPLE_URBAN || plan.irep[j] == SSB200_TILE_INFINITE_STREET) return false;
+    for (const ColumnClass &k : plan.classes)
+      for (int pass = 0; pass < 2; ++pass) {
+        const bool lw = (pass == 1);
+        if (k.cols.empty() || (lw ? !cfg.do_lw : !cfg.do_sw)) continue;
+        const SolveCfg c = class_cfg(cfg, k, lw);
+        int pe = 0, oe = 0, geo = 0;
+        if (be.fused_shape(c, lw, &pe, &oe, &geo) || !be.stage_supported(c)) return false;
+      }
+    return true;
+  }
 
   template <int NS>
   void run_class(ClassArgs a, bool lw, const Plan &plan, const ColumnClass &k, size_t col_offset) {
@@ -328,7 +369,7 @@ struct Dispatcher {
       if (staged) {
         double *cursor = a.sweep + (rec ? scratch_doubles((size_t)r_op, (size_t)lmax, width)
                                         : scratch_doubles(es, (size_t)lmax + 1, width));
-        stage_plan(b, lw, (size_t)lmax * cnt, cursor, &sin.list, &sout.list);
+        stage_plan(b, lw, (size_t)lmax * cnt, cursor, &sin.list, &sout.list, f32_layers);
         b.lstride = (int)cnt;
         sin.cols = sout.cols = a.cols;
         sin.nlay = sout.nlay = a.nlay;
@@ -374,16 +415,7 @@ struct Dispatcher {
         }
         ClassArgs a;
         std::memset(&a, 0, sizeof(a));
-        a.cfg.urban = k.urban;
-        a.cfg.lw = lw ? 1 : 0;
-        a.cfg.nreg = k.nreg;
-        a.cfg.ns = lgs.nstream;
-        a.cfg.nspec = lw ? cfg.nlw : cfg.nsw;
-        a.cfg.symmetric_scale =
-            k.urban ? cfg.use_symmetric_vegetation_scale_urban : cfg.use_symmetric_vegetation_scale_forest;
-        a.cfg.isolation = k.urban ? cfg.vegetation_isolation_factor_urban : cfg.vegetation_isolation_factor_forest;
-        a.cfg.min_veg = cfg.min_vegetation_fraction;
-        a.cfg.min_bld = cfg.min_building_fraction;
+        a.cfg = class_cfg(cfg, k, lw);
         a.lg = make_lg(lgs);
         a.nlay = be.dev_nlay();
         a.istartlay = be.dev_istartlay();

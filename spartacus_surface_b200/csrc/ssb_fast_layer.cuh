@@ -272,7 +272,9 @@ SSB_HD inline void fast_layer_problem_lw(const ClassArgs &a, int q, int lev, con
 // only a sub-block of its regions (same rule as layer_geometry: radsurf_urban_sw.F90:512-583).
 // Columns with equal keys take the same code path layer by layer, so ordering the columns of
 // a launch by this key makes warps uniform: the segment kernels write, and the sweeps skip,
-// whole 32-byte sectors.  Night-time columns (shortwave) go last.
+// whole 32-byte sectors.  Night-time columns (shortwave) go last.  T: element type of the
+// per-layer fractions (float for the caller's arrays of ssb200_radsurf_device_sp).
+template <class T = double>
 SSB_HDI unsigned column_segment_key(const ClassArgs &a, int col) {
   const SolveCfg &c = a.cfg;
   if (!c.lw && !(a.cp.cos_sza[col] > 0.0)) return 0xffffffffu;
@@ -282,8 +284,8 @@ SSB_HDI unsigned column_segment_key(const ClassArgs &a, int col) {
   const bool veg = c.nreg > 1 || !c.urban;
   unsigned key = 0u;
   for (int l = 0; l < nlay && l < 31; ++l) {
-    const double bf = c.urban ? a.cp.building_fraction[il1 + l] : 0.0;
-    const double vf = (veg && a.cp.veg_fraction) ? a.cp.veg_fraction[il1 + l] : 0.0;
+    const double bf = c.urban ? (double)((const T *)a.cp.building_fraction)[il1 + l] : 0.0;
+    const double vf = (veg && a.cp.veg_fraction) ? (double)((const T *)a.cp.veg_fraction)[il1 + l] : 0.0;
     double frac[3];
     region_fractions(c, bf, vf, frac);
     if (vf <= c.min_veg || frac[0] <= c.min_veg) key |= 1u << l;

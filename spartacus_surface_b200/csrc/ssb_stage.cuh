@@ -22,6 +22,9 @@ struct StageList {
   double *ref[kStageMaxArrays];     // the caller's array, reference layout (inputs are not written)
   double *staged[kStageMaxArrays];  // [lev][ic][g] buffer of the chunk
   int nspec[kStageMaxArrays];
+  // 1: `ref` really holds float (ssb200_radsurf_device_sp): the gather widens exactly, the scatter
+  // rounds to nearest, so the kernels see the same doubles as the double entry on widened inputs
+  unsigned char f32[kStageMaxArrays];
 };
 struct StageArgs {
   StageList list;
@@ -37,12 +40,21 @@ inline void stage_host(const StageArgs &s, bool scatter) {
       const int col = s.cols[ic], il1 = s.istartlay[col] - 1;
       for (int lev = 0; lev < s.nlay[col]; ++lev)
         for (int g = 0; g < ns; ++g) {
-          double &r = s.list.ref[k][(size_t)g + (size_t)ns * (size_t)(il1 + lev)];
+          const size_t ri = (size_t)g + (size_t)ns * (size_t)(il1 + lev);
           double &t = s.list.staged[k][(size_t)g + (size_t)ns * ((size_t)ic + (size_t)lev * (size_t)s.ncols)];
-          if (scatter)
-            r = t;
-          else
-            t = r;
+          if (s.list.f32[k]) {
+            float &r = reinterpret_cast<float *>(s.list.ref[k])[ri];
+            if (scatter)
+              r = (float)t;  // round to nearest even
+            else
+              t = (double)r;
+          } else {
+            double &r = s.list.ref[k][ri];
+            if (scatter)
+              r = t;
+            else
+              t = r;
+          }
         }
     }
   }
@@ -51,12 +63,18 @@ inline void stage_host(const StageArgs &s, bool scatter) {
 #if defined(__CUDACC__)
 constexpr int kStageBlock = 256;
 constexpr int kStageTile = 4096;  // doubles of shared memory per block
+// store of a staged double on the caller's side: unchanged, or rounded to nearest float
+__device__ __forceinline__ double stage_out(double *, double v) { return v; }
+__device__ __forceinline__ float stage_out(float *, double v) { return __double2float_rn(v); }
+
 // blockIdx.x: tile of `tc` chunk columns, blockIdx.y: array.  `lb` levels per pass of the tile.
-template <bool SCATTER>
+// R: element type of the caller's side (double, or float for the single-precision device entry).
+template <bool SCATTER, class R>
 __global__ void __launch_bounds__(kStageBlock) k_stage(StageArgs s, int tc, int lb) {
   __shared__ double tile[kStageTile + 2 * 64];
   const int k = blockIdx.y, ns = s.list.nspec[k];
-  double *ref = s.list.ref[k], *stg = s.list.staged[k];
+  R *ref = reinterpret_cast<R *>(s.list.ref[k]);
+  double *stg = s.list.staged[k];
   const int ic0 = blockIdx.x * tc;
   const int ncl = min(tc, s.ncols - ic0);
   if (ncl <= 0) return;
@@ -69,7 +87,7 @@ __global__ void __launch_bounds__(kStageBlock) k_stage(StageArgs s, int tc, int 
         const int c = idx / (nl * ns), r = idx % (nl * ns), l = r / ns, g = r % ns;
         const int col = s.cols[ic0 + c];
         if (l0 + l < s.nlay[col])
-          tile[l * pitch + c * ns + g] = ref[(size_t)g + (size_t)ns * (size_t)(s.istartlay[col] - 1 + l0 + l)];
+          tile[l * pitch + c * ns + g] = (double)ref[(size_t)g + (size_t)ns * (size_t)(s.istartlay[col] - 1 + l0 + l)];
       }
       __syncthreads();
       for (int idx = threadIdx.x; idx < total; idx += kStageBlock) {  // (c, g) fastest: contiguous in `stg`
@@ -88,7 +106,7 @@ __global__ void __launch_bounds__(kStageBlock) k_stage(StageArgs s, int tc, int 
         const int c = idx / (nl * ns), r = idx % (nl * ns), l = r / ns, g = r % ns;
         const int col = s.cols[ic0 + c];
         if (l0 + l < s.nlay[col])
-          ref[(size_t)g + (size_t)ns * (size_t)(s.istartlay[col] - 1 + l0 + l)] = tile[l * pitch + c * ns + g];
+          ref[(size_t)g + (size_t)ns * (size_t)(s.istartlay[col] - 1 + l0 + l)] = stage_out(ref, tile[l * pitch + c * ns + g]);
       }
     }
     __syncthreads();
@@ -97,8 +115,9 @@ __global__ void __launch_bounds__(kStageBlock) k_stage(StageArgs s, int tc, int 
 
 // Arrays with one value per layer (every array when nsw = nlw = 1): no tile needed.  A thread moves four
 // vertically adjacent layers of one column of every array: on the reference side that is one full 32-byte
-// sector per array, on the staged side four rows in which neighbouring threads are neighbouring columns.
-template <bool SCATTER>
+// sector per array (16 bytes for float), on the staged side four rows in which neighbouring threads are
+// neighbouring columns.
+template <bool SCATTER, class R>
 __global__ void __launch_bounds__(kStageBlock) k_stage1(StageArgs s) {
   // neighbouring threads take neighbouring groups of four layers of ONE column: on the reference side a
   // warp then covers whole 128-byte lines (8 columns x 16 layers when every column has 16 layers)
@@ -115,37 +134,86 @@ __global__ void __launch_bounds__(kStageBlock) k_stage1(StageArgs s) {
   const bool vec = cnt >= 4 && (rbase & 1) == 0;  // two aligned 16-byte accesses on the reference side
 #pragma unroll 4
   for (int k = 0; k < s.list.n; ++k) {
-    double *ref = s.list.ref[k] + rbase, *stg = s.list.staged[k] + sbase;
+    R *ref = reinterpret_cast<R *>(s.list.ref[k]) + rbase;
+    double *stg = s.list.staged[k] + sbase;
     double v[4];
-    if (!SCATTER) {
-      if (vec) {
-        const double2 a = __ldcs((const double2 *)ref), b = __ldcs((const double2 *)ref + 1);
-        v[0] = a.x, v[1] = a.y, v[2] = b.x, v[3] = b.y;
+    if constexpr (sizeof(R) == sizeof(float)) {
+      // four floats are one 16-byte access when the ADDRESS is 16-byte aligned (the caller's base
+      // address is not assumed to be)
+      const bool vec4 = cnt >= 4 && ((size_t)ref & 15) == 0;
+      if (!SCATTER) {
+        if (vec4) {
+          const float4 a = __ldcs((const float4 *)ref);
+          v[0] = a.x, v[1] = a.y, v[2] = a.z, v[3] = a.w;
+        } else {
+#pragma unroll
+          for (int j = 0; j < 4; ++j)
+            if (j < cnt) v[j] = (double)__ldcs(ref + j);
+        }
+#pragma unroll
+        for (int j = 0; j < 4; ++j)
+          if (j < cnt) stg[j * pitch] = v[j];
       } else {
 #pragma unroll
         for (int j = 0; j < 4; ++j)
-          if (j < cnt) v[j] = __ldcs(ref + j);
+          if (j < cnt) v[j] = __ldcs(stg + j * pitch);
+        if (vec4) {
+          __stcs((float4 *)ref, make_float4(__double2float_rn(v[0]), __double2float_rn(v[1]), __double2float_rn(v[2]),
+                                            __double2float_rn(v[3])));
+        } else {
+#pragma unroll
+          for (int j = 0; j < 4; ++j)
+            if (j < cnt) __stcs(ref + j, __double2float_rn(v[j]));
+        }
       }
-#pragma unroll
-      for (int j = 0; j < 4; ++j)
-        if (j < cnt) stg[j * pitch] = v[j];
     } else {
+      if (!SCATTER) {
+        if (vec) {
+          const double2 a = __ldcs((const double2 *)ref), b = __ldcs((const double2 *)ref + 1);
+          v[0] = a.x, v[1] = a.y, v[2] = b.x, v[3] = b.y;
+        } else {
 #pragma unroll
-      for (int j = 0; j < 4; ++j)
-        if (j < cnt) v[j] = __ldcs(stg + j * pitch);
-      if (vec) {
-        __stcs((double2 *)ref, make_double2(v[0], v[1]));
-        __stcs((double2 *)ref + 1, make_double2(v[2], v[3]));
+          for (int j = 0; j < 4; ++j)
+            if (j < cnt) v[j] = __ldcs(ref + j);
+        }
+#pragma unroll
+        for (int j = 0; j < 4; ++j)
+          if (j < cnt) stg[j * pitch] = v[j];
       } else {
 #pragma unroll
         for (int j = 0; j < 4; ++j)
-          if (j < cnt) __stcs(ref + j, v[j]);
+          if (j < cnt) v[j] = __ldcs(stg + j * pitch);
+        if (vec) {
+          __stcs((double2 *)ref, make_double2(v[0], v[1]));
+          __stcs((double2 *)ref + 1, make_double2(v[2], v[3]));
+        } else {
+#pragma unroll
+          for (int j = 0; j < 4; ++j)
+            if (j < cnt) __stcs(ref + j, v[j]);
+        }
       }
     }
   }
 }
 
-// launches one grid per group of arrays with the same spectral width (the tile shape depends on it)
+template <bool SCATTER, class R>
+inline void stage_launch_group(const StageArgs &g, int ns, cudaStream_t st) {
+  if (ns == 1) {
+    const long nthreads = (long)g.ncols * ((g.lmax + 3) / 4);
+    const unsigned blocks = (unsigned)((nthreads + kStageBlock - 1) / kStageBlock);
+    k_stage1<SCATTER, R><<<blocks, kStageBlock, 0, st>>>(g);
+    return;
+  }
+  int lb = g.lmax < 32 ? g.lmax : 32;
+  while (lb > 1 && lb * ns > kStageTile) lb /= 2;  // (stage_supported caps the spectral width at kStageTile)
+  int tc = kStageTile / (lb * ns);
+  tc = tc > 64 ? 64 : (tc < 1 ? 1 : tc);
+  const dim3 grid((unsigned)((g.ncols + tc - 1) / tc), (unsigned)g.list.n);
+  k_stage<SCATTER, R><<<grid, kStageBlock, 0, st>>>(g, tc, lb);
+}
+
+// launches one grid per group of arrays with the same spectral width (the tile shape depends on it) and
+// the same element type on the caller's side
 inline void stage_launch(const StageArgs &s, bool scatter, cudaStream_t st, long *launches) {
   if (s.list.n == 0 || s.ncols <= 0 || s.lmax <= 0) return;
   int done[kStageMaxArrays] = {0};
@@ -154,33 +222,20 @@ inline void stage_launch(const StageArgs &s, bool scatter, cudaStream_t st, long
     StageArgs g = s;
     g.list.n = 0;
     const int ns = s.list.nspec[k0];
+    const unsigned char f32 = s.list.f32[k0];
     for (int k = k0; k < s.list.n; ++k)
-      if (!done[k] && s.list.nspec[k] == ns) {
+      if (!done[k] && s.list.nspec[k] == ns && s.list.f32[k] == f32) {
         g.list.ref[g.list.n] = s.list.ref[k];
         g.list.staged[g.list.n] = s.list.staged[k];
         g.list.nspec[g.list.n] = ns;
+        g.list.f32[g.list.n] = f32;
         ++g.list.n;
         done[k] = 1;
       }
-    if (ns == 1) {
-      const long nthreads = (long)s.ncols * ((s.lmax + 3) / 4);
-      const unsigned blocks = (unsigned)((nthreads + kStageBlock - 1) / kStageBlock);
-      if (scatter)
-        k_stage1<true><<<blocks, kStageBlock, 0, st>>>(g);
-      else
-        k_stage1<false><<<blocks, kStageBlock, 0, st>>>(g);
-      if (launches) ++*launches;
-      continue;
-    }
-    int lb = s.lmax < 32 ? s.lmax : 32;
-    while (lb > 1 && lb * ns > kStageTile) lb /= 2;  // (stage_supported caps the spectral width at kStageTile)
-    int tc = kStageTile / (lb * ns);
-    tc = tc > 64 ? 64 : (tc < 1 ? 1 : tc);
-    const dim3 grid((unsigned)((s.ncols + tc - 1) / tc), (unsigned)g.list.n);
-    if (scatter)
-      k_stage<true><<<grid, kStageBlock, 0, st>>>(g, tc, lb);
+    if (f32)
+      scatter ? stage_launch_group<true, float>(g, ns, st) : stage_launch_group<false, float>(g, ns, st);
     else
-      k_stage<false><<<grid, kStageBlock, 0, st>>>(g, tc, lb);
+      scatter ? stage_launch_group<true, double>(g, ns, st) : stage_launch_group<false, double>(g, ns, st);
     if (launches) ++*launches;
   }
 }

@@ -16,8 +16,9 @@ class boundary_conds_out_type:
             self.lw_emission = zeros((ncol, nlw), device=device)
         return self
 
-    def as_struct(self):
+    def as_struct(self, ptr=dptr):
+        """C struct of the members; `ptr` maps an array to the address stored (default: dptr)."""
         c = _abi.BoundaryCondsOut()
         for name in ("sw_albedo", "sw_albedo_dir", "lw_emissivity", "lw_emission"):
-            setattr(c, name, dptr(getattr(self, name)))
+            setattr(c, name, ptr(getattr(self, name)))
         return c

@@ -94,11 +94,12 @@ class canopy_flux_type:
     def is_device(self):
         return is_torch(self.ground_dn)
 
-    def as_struct(self):
+    def as_struct(self, ptr=dptr):
+        """C struct of the members; `ptr` maps an array to the address stored (default: dptr)."""
         c = _abi.CanopyFlux()
         c.nspec, c.ncol, c.ntotlay = int(self.nspec), int(self.ncol), int(self.ntotlay)
         for name in ALL_FIELDS:
-            setattr(c, name, dptr(getattr(self, name)))
+            setattr(c, name, ptr(getattr(self, name)))
         return c
 
     # -- scale_canopy_flux (radsurf_canopy_flux.F90:212-282) -----------------

@@ -42,12 +42,13 @@ class canopy_properties_type:
         self.istartlay = start.astype(np.int32)
         return self
 
-    def as_struct(self):
+    def as_struct(self, ptr=dptr):
+        """C struct of the members; `ptr` maps an array to the address stored (default: dptr)."""
         c = _abi.CanopyProperties()
         c.ncol, c.ntotlay = int(self.ncol), int(self.ntotlay)
         c.nlay, c.istartlay = iptr(self.nlay), iptr(self.istartlay)
         c.i_representation = iptr(self.i_representation)
-        c.cos_sza = dptr(self.cos_sza)
+        c.cos_sza = ptr(self.cos_sza)
         for name in _REAL_LAYER:
-            setattr(c, name, dptr(getattr(self, name)))
+            setattr(c, name, ptr(getattr(self, name)))
         return c

@@ -2,12 +2,12 @@
 
 Same argument list and meaning as the reference subroutine; the body is the
 B200 library (ssb200_radsurf for host arrays, ssb200_radsurf_device when the
-members are torch CUDA tensors).  The reference aborts on error
+members are torch CUDA tensors; the _sp wrappers below take float32 arrays).  The reference aborts on error
 (utilities/radiation_io.F90:46-54); here errors raise RadsurfError.
 """
 import ctypes as C
 
-from ._arrays import is_torch
+from ._arrays import dptr, is_torch
 from ._lib import load, last_error
 
 
@@ -16,22 +16,24 @@ class RadsurfError(RuntimeError):
 
 
 def marshal(config, canopy_props, sw_spectral_props, lw_spectral_props, bc_out,
-            sw_norm_dir=None, sw_norm_diff=None, lw_internal=None, lw_norm=None):
+            sw_norm_dir=None, sw_norm_diff=None, lw_internal=None, lw_norm=None, ptr=dptr):
     """Build the C structs of include/spartacus_b200.h from the API objects.
 
     Returned objects own no array memory: the caller's arrays must outlive
-    the call (same ownership rule as the Fortran allocatables).
+    the call (same ownership rule as the Fortran allocatables).  `ptr` maps
+    an array member to the address stored in its struct slot.
     """
+    s = lambda o: o.as_struct(ptr) if o is not None else None
     structs = dict(
         config=config.as_struct(),
-        canopy=canopy_props.as_struct(),
-        sw=sw_spectral_props.as_struct() if sw_spectral_props is not None else None,
-        lw=lw_spectral_props.as_struct() if lw_spectral_props is not None else None,
-        bc=bc_out.as_struct(),
-        sw_norm_dir=sw_norm_dir.as_struct() if sw_norm_dir is not None else None,
-        sw_norm_diff=sw_norm_diff.as_struct() if sw_norm_diff is not None else None,
-        lw_internal=lw_internal.as_struct() if lw_internal is not None else None,
-        lw_norm=lw_norm.as_struct() if lw_norm is not None else None,
+        canopy=canopy_props.as_struct(ptr),
+        sw=s(sw_spectral_props),
+        lw=s(lw_spectral_props),
+        bc=bc_out.as_struct(ptr),
+        sw_norm_dir=s(sw_norm_dir),
+        sw_norm_diff=s(sw_norm_diff),
+        lw_internal=s(lw_internal),
+        lw_norm=s(lw_norm),
     )
     return structs
 
@@ -94,14 +96,44 @@ def radsurf_fluxes(config, canopy_props, sw_spectral_props, lw_spectral_props, b
     return rc
 
 
-def _real_members(*objs):
+def _float_members(*objs):
+    """Every real array member of the objects: numpy arrays of a float dtype and floating torch tensors."""
     import numpy as np
     for o in objs:
         if o is None:
             continue
         for v in vars(o).values():
-            if isinstance(v, np.ndarray) and v.dtype.kind == "f":
+            if (isinstance(v, np.ndarray) and v.dtype.kind == "f") or (is_torch(v) and v.is_floating_point()):
                 yield v
+
+
+def _is_f32(a):
+    import numpy as np
+    if is_torch(a):
+        import torch
+        return a.dtype == torch.float32
+    return a.dtype == np.float32
+
+
+def f32_ptr(device, where):
+    """Address function for the single-precision entries: the _sp structs of the header are
+    layout-identical to the double-precision ones, so the same ctypes structs carry float32 addresses.
+    device=False accepts C-contiguous float32 numpy arrays, device=True contiguous float32 torch CUDA
+    tensors; anything else raises RadsurfError (the double-precision entries keep their own checks)."""
+    import numpy as np
+    _dp = C.POINTER(C.c_double)
+
+    def ptr(a):
+        if a is None:
+            return C.cast(None, _dp)
+        if device:
+            if is_torch(a) and a.is_cuda and _is_f32(a) and a.is_contiguous():
+                return C.cast(a.data_ptr(), _dp)
+            raise RadsurfError(f"{where}: every real member must be a contiguous float32 CUDA tensor")
+        if isinstance(a, np.ndarray) and a.dtype == np.float32 and a.flags["C_CONTIGUOUS"]:
+            return a.ctypes.data_as(_dp)
+        raise RadsurfError(f"{where}: every real member must be a C-contiguous float32 numpy array")
+    return ptr
 
 
 def to_single(obj):
@@ -118,17 +150,56 @@ def to_single(obj):
 
 def radsurf_sp(config, canopy_props, sw_spectral_props, lw_spectral_props, bc_out,
                istartcol=None, iendcol=None, sw_norm_dir=None, sw_norm_diff=None,
-               lw_internal=None, lw_norm=None):
-    """radsurf for single-precision (float32) host arrays: ssb200_radsurf_sp.  The arrays cross PCIe
-    as float32, the solve runs in FP64 on the device, outputs are the FP64 results rounded to float32."""
-    import numpy as np
+               lw_internal=None, lw_norm=None, stream=None):
+    """radsurf for single-precision (float32) arrays.  numpy members: ssb200_radsurf_sp (the arrays cross
+    PCIe as float32).  torch CUDA members: ssb200_radsurf_device_sp, enqueued on `stream` (cudaStream_t
+    as an int, None = default stream) without synchronising.  The solve runs in FP64 on the device and
+    every output is the FP64 result rounded to float32."""
     lib = load()
     objs = (canopy_props, sw_spectral_props, lw_spectral_props, bc_out, sw_norm_dir, sw_norm_diff, lw_internal, lw_norm)
-    if not all(v.dtype == np.float32 for v in _real_members(*objs)):
+    members = list(_float_members(*objs))
+    device = any(is_torch(v) for v in members)
+    if device and not all(is_torch(v) for v in members):
+        raise RadsurfError("radsurf_sp: members mix numpy arrays and torch tensors")
+    if not all(_is_f32(v) for v in members):
         raise RadsurfError("radsurf_sp: every real array member must be float32")
     structs = marshal(config, canopy_props, sw_spectral_props, lw_spectral_props, bc_out,
-                      sw_norm_dir, sw_norm_diff, lw_internal, lw_norm)
-    rc = call_radsurf(lib.ssb200_radsurf_sp, structs, istartcol, iendcol)
+                      sw_norm_dir, sw_norm_diff, lw_internal, lw_norm, ptr=f32_ptr(device, "radsurf_sp"))
+    if device:
+        rc = call_radsurf(lib.ssb200_radsurf_device_sp, structs, istartcol, iendcol,
+                          extra=(C.c_void_p(stream or 0), None))
+    else:
+        rc = call_radsurf(lib.ssb200_radsurf_sp, structs, istartcol, iendcol)
     if rc < 0:
-        raise RadsurfError(f"ssb200_radsurf_sp failed (rc={rc}): {last_error()}")
+        name = "ssb200_radsurf_device_sp" if device else "ssb200_radsurf_sp"
+        raise RadsurfError(f"{name} failed (rc={rc}): {last_error()}")
+    return rc
+
+
+def radsurf_fluxes_sp(config, canopy_props, sw_spectral_props, lw_spectral_props, bc_out, istartcol=None,
+                      iendcol=None, sw_flux=None, lw_flux=None, top_flux_dn_sw=None, top_flux_dn_direct_sw=None,
+                      top_flux_dn_lw=None, ground_temperature=None, roof_temperature=None, wall_temperature=None,
+                      clear_air_temperature=None, veg_temperature=None, veg_air_temperature=None):
+    """radsurf_fluxes for single-precision (float32) host arrays: ssb200_radsurf_fluxes_sp.  Same arguments
+    and defaults as radsurf_fluxes; every real member, top-of-canopy flux and temperature must be a float32
+    numpy array.  The arrays cross PCIe as float32, the solve, emission and scale + sum run in FP64 and
+    every output is the FP64 result rounded to float32."""
+    from . import _abi
+    lib = load()
+    ptr = f32_ptr(False, "radsurf_fluxes_sp")
+    members = list(_float_members(canopy_props, sw_spectral_props, lw_spectral_props, bc_out, sw_flux, lw_flux))
+    if not all(_is_f32(v) for v in members):
+        raise RadsurfError("radsurf_fluxes_sp: every real array member must be float32")
+    structs = marshal(config, canopy_props, sw_spectral_props, lw_spectral_props, bc_out, ptr=ptr)
+    drv = _abi.DriverInputs(*[ptr(a) for a in (top_flux_dn_sw, top_flux_dn_direct_sw, top_flux_dn_lw,
+                                               ground_temperature, roof_temperature, wall_temperature,
+                                               clear_air_temperature, veg_temperature, veg_air_temperature)])
+    fsw = sw_flux.as_struct(ptr) if sw_flux is not None else None
+    flw = lw_flux.as_struct(ptr) if lw_flux is not None else None
+    s = structs
+    rc = lib.ssb200_radsurf_fluxes_sp(_ref(s["config"]), _ref(s["canopy"]), _ref(s["sw"]), _ref(s["lw"]),
+                                      C.byref(drv), _ref(s["bc"]), int(istartcol or 0), int(iendcol or 0),
+                                      _ref(fsw), _ref(flw))
+    if rc < 0:
+        raise RadsurfError(f"ssb200_radsurf_fluxes_sp failed (rc={rc}): {last_error()}")
     return rc

@@ -27,9 +27,10 @@ class lw_spectral_properties_type:
             self.wall_emission = (StefanBoltzmann * self.wall_emissivity[:, :1]
                                   * cp.wall_temperature[:, None] ** 4).copy()
 
-    def as_struct(self):
+    def as_struct(self, ptr=dptr):
+        """C struct of the members; `ptr` maps an array to the address stored (default: dptr)."""
         c = _abi.LwSpectralProperties()
         c.nspec = int(self.nspec)
         for name in _MEMBERS:
-            setattr(c, name, dptr(getattr(self, name)))
+            setattr(c, name, ptr(getattr(self, name)))
         return c

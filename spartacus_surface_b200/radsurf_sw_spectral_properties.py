@@ -15,9 +15,10 @@ class sw_spectral_properties_type:
         for name in _MEMBERS:
             setattr(self, name, None)
 
-    def as_struct(self):
+    def as_struct(self, ptr=dptr):
+        """C struct of the members; `ptr` maps an array to the address stored (default: dptr)."""
         c = _abi.SwSpectralProperties()
         c.nspec = int(self.nspec)
         for name in _MEMBERS:
-            setattr(c, name, dptr(getattr(self, name)))
+            setattr(c, name, ptr(getattr(self, name)))
         return c
