@@ -363,6 +363,36 @@ int ssb200_radsurf_device_sp(const ssb200_config *config,
                              ssb200_canopy_flux_sp *lw_norm,
                              void *stream, int32_t *status_out);
 
+/* ssb200_radsurf_fluxes for a caller whose arrays live in HBM: the reference driver's sequence around
+ * radsurf (driver/spartacus_surface_driver.F90:206-261) - calc_simple_spectrum_lw, radsurf, scale of the
+ * normalised fluxes by the top-of-canopy fluxes and sum into sw_flux / lw_flux - in one asynchronous call.
+ * Same semantics as ssb200_radsurf_fluxes: the members of sw_flux / lw_flux that are allocated decide what
+ * is computed, NULL members of the property structs take read_input's defaults, and NULL emission /
+ * Planck members are sigma [emissivity] T^4 of the temperatures in `driver_inputs`.  Every array, the
+ * members of `driver_inputs` included, is a DEVICE pointer; nlay, istartlay and i_representation stay
+ * HOST arrays, as for ssb200_radsurf_device.  The call is enqueued on `stream`, shares the one context of
+ * the other entries, is ordered against calls from other streams and fills `status_out` exactly as
+ * ssb200_radsurf_device.  Columns outside istartcol..iendcol are not written, and per-layer entries only
+ * for the layers of in-range, non-Flat columns; unlike the host entry the packed layers of the selected
+ * columns need not be contiguous.  The caller's arrays are never written except the outputs: defaults and
+ * emission go to buffers of the context.
+ * The four normalised flux objects are never formed in the caller's layout.  When every per-layer write
+ * of the call goes through the level-major staging ("stage_layers", the register-resident kernels of 1-4
+ * streams, no "fused_kernels", no SimpleUrban / InfiniteStreet column), the staging scatter writes the
+ * scaled sum of both objects straight into sw_flux / lw_flux; otherwise the objects are held in buffers
+ * of the context for the call's columns and layers and summed after the solve.  Either way the result is
+ * bit-equal to ssb200_radsurf_fluxes on the same inputs, and to ssb200_radsurf_device followed by
+ * ssb200_canopy_flux_scale_device and ssb200_canopy_flux_sum_device on zeroed normalised objects. */
+int ssb200_radsurf_fluxes_device(const ssb200_config *config,
+                                 const ssb200_canopy_properties *canopy_props,
+                                 const ssb200_sw_spectral_properties *sw_spectral_props,
+                                 const ssb200_lw_spectral_properties *lw_spectral_props,
+                                 const ssb200_driver_inputs *driver_inputs,
+                                 ssb200_boundary_conds_out *bc_out,
+                                 int32_t istartcol, int32_t iendcol,
+                                 ssb200_canopy_flux *sw_flux, ssb200_canopy_flux *lw_flux,
+                                 void *stream, int32_t *status_out);
+
 /* Number of kernels launched by this process through the library so far
  * (bench.py reports the per-step delta as `gpu_launches`). */
 int64_t ssb200_kernel_launch_count(void);

@@ -190,7 +190,9 @@ __global__ void k_lay2col(const int *nlay, const int *istartlay, const int *irep
 // out = a * fa + b * fb per (interval, column) factor, every product and the sum rounded separately
 // so that the result equals canopy_flux_type%scale followed by %sum bit for bit
 // (radsurf/radsurf_canopy_flux.F90:212-282,399-460).  fa NULL: 1.  fb_minus non-NULL: fb - fb_minus.
-// Non-spectral members (sunlit fractions) are summed unscaled.  Window: columns [c0, c1), layers [l0, l1).
+// Non-spectral members (sunlit fractions) are summed unscaled.  Window: columns [c0, c1), layers [l0, l1);
+// a layer of the window is skipped unless a column of [c0, c1) owns it (lay2col: -1 for the layers of no
+// non-Flat column), so packed layouts whose layers are not contiguous leave other columns' layers alone.
 __global__ void k_scale_sum(FieldList fl, const double *fa, const double *fb, const double *fb_minus,
                             const int *lay2col, int nspec, long c0, long c1, long l0, long l1) {
   const long t = blockIdx.x * (long)blockDim.x + threadIdx.x;
@@ -199,14 +201,15 @@ __global__ void k_scale_sum(FieldList fl, const double *fa, const double *fb, co
     const long lo = (fl.per_layer[f] ? l0 : c0) * w, hi = (fl.per_layer[f] ? l1 : c1) * w;
     const long i = lo + t;
     if (i >= hi) continue;
+    const long idx = i / w;
+    const long col = fl.per_layer[f] ? lay2col[idx] : idx;
+    if (col < c0 || col >= c1) continue;
     const double a = fl.a[f][i], b = fl.b[f][i];
     if (!fl.spectral[f]) {
       fl.p[f][i] = __dadd_rn(a, b);
       continue;
     }
-    const long idx = i / nspec;
     const int g = (int)(i % nspec);
-    const long col = fl.per_layer[f] ? lay2col[idx] : idx;
     const size_t k = (size_t)g + (size_t)nspec * (size_t)col;
     const double xa = fa ? __dmul_rn(fa[k], a) : a;
     const double fbk = fb_minus ? __dadd_rn(fb[k], -fb_minus[k]) : fb[k];
@@ -267,6 +270,7 @@ struct Context {
   int pipeline_max_blocks = 16;
   std::vector<DevBuf> stage;  // staging mirrors of host arrays for ssb200_radsurf
   std::vector<DevBuf> wide;   // double copies of float device arrays for ssb200_radsurf_device_sp
+  std::vector<DevBuf> drv;    // defaulted inputs and normalised flux members of ssb200_radsurf_fluxes_device
   cudaStream_t stream = nullptr;
   cudaStream_t own_stream = nullptr;
   size_t budget_doubles = 0;
@@ -621,14 +625,20 @@ int upload_plan(Context &cx, const ssb200_canopy_properties &cp) {
   return 0;
 }
 
+typedef ssb::Dispatcher<CudaBackend>::PassSum PassSum;
+
 // Runs the prepared plan on cx.stream.  f32_layers: the per-layer members of `ca` are float arrays that
-// only the level-major staging touches (ssb200_radsurf_device_sp, staged route).
-int dispatch_call(Context &cx, const ssb::CallArgs &ca, bool f32_layers) {
+// only the level-major staging touches (ssb200_radsurf_device_sp, staged route).  sum_sw / sum_lw:
+// summing scatter of each pass (ssb200_radsurf_fluxes_device, staged route).
+int dispatch_call(Context &cx, const ssb::CallArgs &ca, bool f32_layers, const PassSum &sum_sw = PassSum(),
+                  const PassSum &sum_lw = PassSum()) {
   std::string err;
   CudaBackend be(cx);
   be.f32_layers = f32_layers;
   ssb::Dispatcher<CudaBackend> disp(be);
   disp.f32_layers = f32_layers;
+  disp.sum_sw = sum_sw;
+  disp.sum_lw = sum_lw;
   const int rc = disp.run(ca, cx.plan, err);
   if (rc) return fail(rc, err);
   if (cx.first_error != cudaSuccess)
@@ -720,6 +730,21 @@ int run_window(Context &cx, const ssb::CallArgs &ca, int lane, size_t budget, in
   if (rc) return fail(rc, err);
   if (cx.first_error != cudaSuccess)
     return fail(SSB200_ERR_CUDA, std::string("kernel launch / scratch allocation: ") + cudaGetErrorString(cx.first_error));
+  return 0;
+}
+
+// owner column of every packed layer of the uploaded plan (-1: no non-Flat column owns it), on `st`
+int ensure_lay2col(Context &cx, size_t ncol, size_t ntot, cudaStream_t st) {
+  if (cx.lay2col_generation == cx.plan.generation) return 0;
+  SSB_CUDA(cx.d_lay2col.reserve(sizeof(int) * (ntot + 1)));
+  SSB_CUDA(cudaMemsetAsync(cx.d_lay2col.p, 0xff, sizeof(int) * ntot, st));
+  if (ncol > 0) {
+    k_lay2col<<<(unsigned)((ncol + 127) / 128), 128, 0, st>>>((const int *)cx.d_nlay.p, (const int *)cx.d_istart.p,
+                                                               (const int *)cx.d_irep.p, (int)ncol, (int *)cx.d_lay2col.p);
+    ++g_launches;
+    SSB_CUDA(cudaGetLastError());
+  }
+  cx.lay2col_generation = cx.plan.generation;
   return 0;
 }
 
@@ -1154,6 +1179,241 @@ static int radsurf_device_sp_locked(Context &cx, const ssb::CallArgs &ca, int32_
   return finish_device_call(cx, stream, status_out);
 }
 
+// Body of ssb200_radsurf_fluxes_device: the sequence of radsurf_host with drv != NULL on device arrays.
+// Inputs the caller leaves NULL are filled in context buffers (read_input's defaults, sigma T^4 from the
+// temperatures) over the call's columns and packed layers.  The four normalised flux objects take one of
+// two routes, chosen per call from the plan:
+//   staged:   every per-layer write goes through the level-major staging, whose scatter writes
+//             fa * f1 + fb * f2 straight into sw_flux / lw_flux (StageList::sum): the per-layer members of
+//             the normalised objects exist in the staging buffers of a chunk only.  Their per-column
+//             members (written in place by the sweeps and the surface kernel) live in zeroed context
+//             buffers and are scaled and summed by one launch per pass after the solve;
+//   fallback: generic kernels, stage_layers = 0, column-resident kernels, single-layer urban columns:
+//             the four objects are materialised in zeroed context buffers for the call's columns and
+//             layers, and scaled and summed per column and per owned layer after the solve.
+// Both give the bits of ssb200_radsurf_fluxes: the same products and sums, each rounded once.
+static int radsurf_fluxes_device_locked(Context &cx, const ssb200_config *config, const ssb200_canopy_properties *cp,
+                                        const ssb200_sw_spectral_properties *sw, const ssb200_lw_spectral_properties *lw,
+                                        const ssb200_driver_inputs *drv, ssb200_boundary_conds_out *bc,
+                                        int32_t istartcol, int32_t iendcol, ssb200_canopy_flux *sw_flux,
+                                        ssb200_canopy_flux *lw_flux, cudaStream_t stream, int32_t *status_out) {
+  if (!config || !cp || !bc || !drv)
+    return fail(SSB200_ERR_ARG, "config, canopy_props, driver_inputs and bc_out must not be NULL");
+  if ((config->do_sw && (!sw_flux || !drv->top_flux_dn_sw || !drv->top_flux_dn_direct_sw)) ||
+      (config->do_lw && (!lw_flux || !drv->top_flux_dn_lw)))
+    return fail(SSB200_ERR_ARG, "radsurf_fluxes_device: flux object or top-of-canopy flux missing");
+  {
+    ssb::CallArgs probe{config, cp, sw, lw, bc, sw_flux, sw_flux, lw_flux, lw_flux};
+    std::string err;
+    const int rc = ssb::validate_call(probe, err);
+    if (rc) return fail(rc, err);
+  }
+  const size_t ncol = (size_t)cp->ncol, ntot = (size_t)cp->ntotlay;
+  int c1 = istartcol > 0 ? istartcol : 1, c2 = iendcol > 0 ? iendcol : cp->ncol;
+  if (c2 > cp->ncol) c2 = cp->ncol;
+  if (c1 > c2) return 0;
+  const size_t c0 = (size_t)c1 - 1, cN = (size_t)c2;  // 0-based column window [c0, cN)
+  // packed layers [l0, lN) spanned by the call's columns (ranges outside 1..ntotlay are refused by the plan)
+  size_t l0 = ntot, lN = 0;
+  for (size_t j = c0; j < cN; ++j) {
+    if (cp->i_representation[j] == SSB200_TILE_FLAT || cp->nlay[j] <= 0 || cp->istartlay[j] < 1) continue;
+    const size_t s = (size_t)cp->istartlay[j] - 1, e = s + (size_t)cp->nlay[j];
+    if (e > ntot) continue;
+    l0 = std::min(l0, s);
+    lN = std::max(lN, e);
+  }
+  if (lN < l0) l0 = lN = 0;
+  size_t next = 0;
+  int err_rc = 0;
+  auto buffer = [&](size_t n) -> double * {
+    if (err_rc) return nullptr;
+    if (next >= cx.drv.size()) cx.drv.resize(next + 16);
+    DevBuf &b = cx.drv[next++];
+    const cudaError_t e = b.reserve(std::max(n, (size_t)1) * sizeof(double));
+    if (e != cudaSuccess) {
+      err_rc = fail(SSB200_ERR_CUDA, std::string("context buffers: ") + cudaGetErrorString(e));
+      return nullptr;
+    }
+    return (double *)b.p;
+  };
+  // read_input's defaults and the emission stage, as in radsurf_host
+  struct Fill {
+    double *p;
+    double v;
+    long i0, i1;
+  };
+  struct Emis {
+    double *out;
+    const double *emissivity, *temperature;
+    long i0, i1;
+  };
+  std::vector<Fill> fills;
+  std::vector<Emis> emis;
+  auto filled = [&](size_t width, double v) -> const double * {
+    double *p = buffer(ntot * width);
+    fills.push_back(Fill{p, v, (long)(l0 * width), (long)(lN * width)});
+    return p;
+  };
+  ssb200_canopy_properties dcp = *cp;
+  double *vcf_default = nullptr;
+  if (!cp->veg_contact_fraction && cp->veg_fraction && cp->building_fraction) {
+    vcf_default = buffer(ntot);
+    dcp.veg_contact_fraction = vcf_default;
+  }
+  ssb200_sw_spectral_properties dsw;
+  ssb200_lw_spectral_properties dlw;
+  memset(&dsw, 0, sizeof(dsw));
+  memset(&dlw, 0, sizeof(dlw));
+  if (config->do_sw) {  // driver/spartacus_surface_read_input.F90:258-269,335-344
+    const size_t g = (size_t)config->nsw;
+    dsw = *sw;
+    if (!sw->air_ext) dsw.air_ext = filled(g, 1.0e-5);
+    if (!sw->air_ssa) dsw.air_ssa = filled(g, 0.999);
+    if (!sw->wall_specular_frac && sw->wall_albedo) dsw.wall_specular_frac = filled(g, 0.0);
+  }
+  if (config->do_lw) {  // driver/spartacus_surface_read_input.F90:362-365; radsurf_simple_spectrum.F90:41-66
+    const size_t g = (size_t)config->nlw;
+    dlw = *lw;
+    if (!lw->air_ext) dlw.air_ext = filled(g, 1.0e-5);
+    if (!lw->air_ssa) dlw.air_ssa = filled(g, 0.0);
+    const bool need_t = !lw->ground_emission || !lw->roof_emission || !lw->wall_emission || !lw->clear_air_planck ||
+                        !lw->veg_planck || !lw->veg_air_planck;
+    if (need_t && g != 1)
+      return fail(SSB200_ERR_ARG, "Simple longwave spectrum only possible with one input spectral interval");
+    if (!lw->ground_emission && drv->ground_temperature) {
+      dlw.ground_emission = buffer(ncol);
+      emis.push_back(Emis{const_cast<double *>(dlw.ground_emission), dlw.ground_emissivity, drv->ground_temperature,
+                          (long)c0, (long)cN});
+    }
+    auto layer_emis = [&](const double *given, const double *&slot, const double *emissivity, const double *t) {
+      if (given || !t) return;
+      slot = buffer(ntot);
+      emis.push_back(Emis{const_cast<double *>(slot), emissivity, t, (long)l0, (long)lN});
+    };
+    layer_emis(lw->roof_emission, dlw.roof_emission, dlw.roof_emissivity, drv->roof_temperature);
+    layer_emis(lw->wall_emission, dlw.wall_emission, dlw.wall_emissivity, drv->wall_temperature);
+    layer_emis(lw->clear_air_planck, dlw.clear_air_planck, nullptr, drv->clear_air_temperature);
+    layer_emis(lw->veg_planck, dlw.veg_planck, nullptr, drv->veg_temperature);
+    layer_emis(lw->veg_air_planck, dlw.veg_air_planck, nullptr, drv->veg_air_temperature);
+  }
+  if (err_rc) return err_rc;
+  // plan, argument checks, ordering against the previous call, status reset (the summed objects stand in
+  // for the normalised ones, whose shape they have)
+  ssb::CallArgs ca{config, &dcp, config->do_sw ? &dsw : nullptr, config->do_lw ? &dlw : nullptr, bc,
+                   sw_flux, sw_flux, lw_flux, lw_flux};
+  int range[2] = {1, 0};
+  int rc = radsurf_device_locked(cx, ca, c1, c2, stream, nullptr, range);
+  if (rc || range[0] > range[1]) return rc;
+  CudaBackend probe(cx);
+  ssb::Dispatcher<CudaBackend> route(probe);
+  const bool staged = route.all_layers_staged(ca, cx.plan);
+  // the normalised objects: context buffers shaped like the summed object, zeroed over the call's window
+  // (canopy_flux_type%zero_all, driver:184).  Staged route: per-column members only; the per-layer members
+  // keep the summed object's pointers, which only mark them present (stage_plan redirects them).
+  std::vector<std::pair<double *, size_t>> zeroed;
+  auto normalised = [&](const ssb200_canopy_flux *sum, ssb200_canopy_flux &d) {
+    d = *sum;
+    const size_t g = (size_t)sum->nspec;
+    auto make = [&](double *&m, bool per_layer, size_t w) {
+      if (!m || (per_layer && staged)) return;
+      double *p = buffer((per_layer ? ntot : ncol) * w);
+      if (p) zeroed.push_back({p + (per_layer ? l0 : c0) * w, ((per_layer ? lN - l0 : cN - c0)) * w});
+      m = p;
+    };
+    make(d.ground_dn, false, g); make(d.ground_net, false, g); make(d.ground_vertical_diff, false, g);
+    make(d.top_dn, false, g); make(d.top_net, false, g); make(d.ground_dn_dir, false, g); make(d.top_dn_dir, false, g);
+    make(d.ground_sunlit_frac, false, 1);
+    make(d.roof_in, true, g); make(d.roof_net, true, g); make(d.wall_in, true, g); make(d.wall_net, true, g);
+    make(d.roof_in_dir, true, g); make(d.wall_in_dir, true, g);
+    make(d.roof_sunlit_frac, true, 1); make(d.wall_sunlit_frac, true, 1);
+    make(d.clear_air_abs, true, g); make(d.veg_abs, true, g); make(d.veg_air_abs, true, g); make(d.veg_abs_dir, true, g);
+    make(d.veg_sunlit_frac, true, 1);
+    make(d.flux_dn_layer_top, true, g); make(d.flux_up_layer_top, true, g); make(d.flux_dn_layer_base, true, g);
+    make(d.flux_up_layer_base, true, g); make(d.flux_dn_dir_layer_top, true, g); make(d.flux_dn_dir_layer_base, true, g);
+  };
+  ssb200_canopy_flux d1, d2, d3, d4;
+  PassSum sum_sw, sum_lw;
+  if (config->do_sw) {
+    normalised(sw_flux, d1);
+    normalised(sw_flux, d2);
+    sum_sw.fa = drv->top_flux_dn_direct_sw;
+    sum_sw.fb = drv->top_flux_dn_sw;
+    sum_sw.fb_minus = drv->top_flux_dn_direct_sw;
+    if (staged) sum_sw.out = sw_flux;
+  }
+  if (config->do_lw) {
+    normalised(lw_flux, d3);
+    normalised(lw_flux, d4);
+    sum_lw.fb = drv->top_flux_dn_lw;
+    if (staged) sum_lw.out = lw_flux;
+  }
+  if (err_rc) return err_rc;
+  const ssb::CallArgs nca{config, &dcp, ca.sw, ca.lw, bc, config->do_sw ? &d1 : nullptr, config->do_sw ? &d2 : nullptr,
+                          config->do_lw ? &d3 : nullptr, config->do_lw ? &d4 : nullptr};
+  // an error return after the first launch must not leave work queued on the context's buffers
+  struct Drain {
+    cudaStream_t s;
+    bool armed = true;
+    ~Drain() {
+      if (armed) cudaStreamSynchronize(s);
+    }
+  } drain{stream};
+  CudaBackend be(cx);  // (profiling: the stages around the solve are booked with family 4)
+  be.tick(4, true);
+  for (const Fill &f : fills)
+    if (f.i1 > f.i0) {
+      k_fill<<<(unsigned)((f.i1 - f.i0 + 255) / 256), 256, 0, stream>>>(f.p, f.v, f.i0, f.i1);
+      ++g_launches;
+    }
+  if (vcf_default && lN > l0) {
+    k_vcf_default<<<(unsigned)((lN - l0 + 255) / 256), 256, 0, stream>>>(
+        vcf_default, cp->veg_fraction, cp->building_fraction, config->min_vegetation_fraction, (long)l0, (long)lN);
+    ++g_launches;
+  }
+  for (const Emis &e : emis)
+    if (e.i1 > e.i0) {
+      k_sigma_t4<<<(unsigned)((e.i1 - e.i0 + 255) / 256), 256, 0, stream>>>(e.out, e.emissivity, e.temperature, 1,
+                                                                              e.i0, e.i1);
+      ++g_launches;
+    }
+  for (const auto &z : zeroed)
+    if (z.second > 0) SSB_CUDA(cudaMemsetAsync(z.first, 0, z.second * sizeof(double), stream));
+  SSB_CUDA(cudaGetLastError());
+  be.tick(4, false);
+  if ((rc = dispatch_call(cx, nca, false, sum_sw, sum_lw))) return rc;
+  // scale + sum (driver:250-261) of what the solve left in the normalised objects: the per-column members
+  // (staged route), or every member over the call's columns and owned layers (fallback route)
+  if (!staged && (rc = ensure_lay2col(cx, ncol, ntot, stream))) return rc;
+  const long cnt = (long)std::max(cN - c0, staged ? (size_t)0 : lN - l0);
+  auto scale_sum = [&](ssb200_canopy_flux *o, const ssb200_canopy_flux &x, const ssb200_canopy_flux &y,
+                       const double *fa, const double *fb, const double *fbm, int nspec) {
+    FieldList all, fl;
+    collect_fields(o, &x, &y, all, true);
+    fl.n = 0;
+    for (int f = 0; f < all.n; ++f)
+      if (!staged || !all.per_layer[f]) {
+        fl.p[fl.n] = all.p[f];
+        fl.a[fl.n] = all.a[f];
+        fl.b[fl.n] = all.b[f];
+        fl.per_layer[fl.n] = all.per_layer[f];
+        fl.spectral[fl.n] = all.spectral[f];
+        ++fl.n;
+      }
+    const long nthr = cnt * nspec;
+    if (fl.n == 0 || nthr <= 0) return;
+    k_scale_sum<<<(unsigned)((nthr + 255) / 256), 256, 0, stream>>>(fl, fa, fb, fbm, (const int *)cx.d_lay2col.p,
+                                                                     nspec, (long)c0, (long)cN, (long)l0, (long)lN);
+    ++g_launches;
+  };
+  be.tick(4, true);
+  if (config->do_sw) scale_sum(sw_flux, d1, d2, sum_sw.fa, sum_sw.fb, sum_sw.fb_minus, config->nsw);
+  if (config->do_lw) scale_sum(lw_flux, d3, d4, nullptr, sum_lw.fb, nullptr, config->nlw);
+  SSB_CUDA(cudaGetLastError());
+  be.tick(4, false);
+  drain.armed = false;
+  return finish_device_call(cx, stream, status_out);
+}
+
 // Body of both host entries.  drv == NULL: ssb200_radsurf (the four normalised flux objects are
 // host arrays).  drv != NULL: ssb200_radsurf_fluxes - the normalised objects exist on the device
 // only (shaped like sw_flux / lw_flux), NULL inputs take read_input's defaults or are derived from
@@ -1437,13 +1697,7 @@ static int radsurf_host(const ssb200_config *config, const ssb200_canopy_propert
   int range[2];
   rc = radsurf_device_locked(cx, ca, c1, c2, st, nullptr, range);
   if (rc) return rc;
-  if (drv && cx.lay2col_generation != cx.plan.generation) {
-    SSB_CUDA(cx.d_lay2col.reserve(sizeof(int) * (ntot + 1)));
-    k_lay2col<<<(unsigned)((ncol + 127) / 128), 128, 0, st>>>((const int *)cx.d_nlay.p, (const int *)cx.d_istart.p,
-                                                               (const int *)cx.d_irep.p, (int)ncol, (int *)cx.d_lay2col.p);
-    ++g_launches;
-    cx.lay2col_generation = cx.plan.generation;
-  }
+  if (drv && (rc = ensure_lay2col(cx, ncol, ntot, st))) return rc;
   SSB_CUDA(cudaStreamSynchronize(st));  // plan upload and status reset are visible to every lane
   const size_t total_work = lN + cN;
   int nblk = 1;
@@ -1612,6 +1866,18 @@ int ssb200_radsurf_device_sp(const ssb200_config *config, const ssb200_canopy_pr
   return radsurf_device_sp_locked(g_ctx, ca, istartcol, iendcol, (cudaStream_t)stream, status_out);
 }
 
+int ssb200_radsurf_fluxes_device(const ssb200_config *config, const ssb200_canopy_properties *canopy_props,
+                                 const ssb200_sw_spectral_properties *sw, const ssb200_lw_spectral_properties *lw,
+                                 const ssb200_driver_inputs *driver_inputs, ssb200_boundary_conds_out *bc_out,
+                                 int32_t istartcol, int32_t iendcol, ssb200_canopy_flux *sw_flux,
+                                 ssb200_canopy_flux *lw_flux, void *stream, int32_t *status_out) {
+  int rc = ensure_device();
+  if (rc) return rc;
+  std::lock_guard<std::mutex> lock(g_mutex);
+  return radsurf_fluxes_device_locked(g_ctx, config, canopy_props, sw, lw, driver_inputs, bc_out, istartcol, iendcol,
+                                      sw_flux, lw_flux, (cudaStream_t)stream, status_out);
+}
+
 int64_t ssb200_kernel_launch_count(void) { return (int64_t)g_launches; }
 
 int ssb200_set_profiling(int enable) {
@@ -1715,6 +1981,7 @@ int ssb200_release(void) {
     }
     for (DevBuf &b : cx.stage) b.release();
     for (DevBuf &b : cx.wide) b.release();
+    for (DevBuf &b : cx.drv) b.release();
   }
   cx.plan = ssb::Plan();
   cx.plan_uploaded = false;
@@ -1738,6 +2005,7 @@ int ssb200_canopy_flux_scale_device(ssb200_canopy_flux *flux, const int32_t *nla
       lay2col[(size_t)il] = j;
     }
   SSB_CUDA(cx.d_lay2col.reserve(sizeof(int) * (lay2col.size() + 1)));
+  cx.lay2col_generation = -1;  // (the plan's map is rebuilt by the next call that needs it)
   SSB_CUDA(cudaMemcpyAsync(cx.d_lay2col.p, lay2col.data(), sizeof(int) * lay2col.size(), cudaMemcpyHostToDevice, st));
   SSB_CUDA(cudaStreamSynchronize(st));
   FieldList fl;

@@ -23,20 +23,29 @@ namespace ssb {
 // Lists the per-layer arrays of a pass and redirects the members of `b` to their level-major staging
 // buffers (ssb_stage.cuh), carved from `cursor` (NULL: only count).  Returns doubles per (level, column).
 // f32: the members of `b` are the caller's float arrays (ssb200_radsurf_device_sp).
+// sum: summing scatter (ssb200_radsurf_fluxes_device): both normalised objects f1 and f2 are still staged
+// (the kernels write both), and `out` pairs the staging buffers of each member with that member of *sum.
 inline size_t stage_plan(ClassArgs &b, bool lw, size_t per_elem, double *cursor, StageList *in, StageList *out,
-                         bool f32 = false) {
+                         bool f32 = false, const ssb200_canopy_flux *sum = nullptr) {
   size_t elems = 0;
-  auto add = [&](StageList *list, double *&member, int ns) {
-    if (!member) return;
+  // stages `member` (listed in `list` unless NULL); returns its staging buffer
+  auto add = [&](StageList *list, double *&member, int ns) -> double * {
+    if (!member) return nullptr;
     elems += (size_t)ns;
-    if (!cursor) return;
-    list->ref[list->n] = member;
-    list->staged[list->n] = cursor;
-    list->nspec[list->n] = ns;
-    list->f32[list->n] = f32 ? 1 : 0;
-    ++list->n;
+    if (!cursor) return nullptr;
+    double *staged = cursor;
+    if (list) {
+      list->ref[list->n] = member;
+      list->staged[list->n] = cursor;
+      list->staged2[list->n] = nullptr;
+      list->nspec[list->n] = ns;
+      list->f32[list->n] = f32 ? 1 : 0;
+      list->sum[list->n] = kSumNone;
+      ++list->n;
+    }
     member = cursor;
     cursor += (size_t)ns * per_elem;
+    return staged;
   };
   auto cin = [&](const double *&member, int ns) { add(in, const_cast<double *&>(member), ns); };
   if (in) in->n = 0;
@@ -70,27 +79,38 @@ inline size_t stage_plan(ClassArgs &b, bool lw, size_t per_elem, double *cursor,
     cin(b.sw.wall_specular_frac, ns);
     cin(b.sw.roof_albedo_dir, ns);
   }
-  for (ssb200_canopy_flux *f : {&b.f1, &b.f2}) {
-    add(out, f->roof_in, ns);
-    add(out, f->roof_net, ns);
-    add(out, f->wall_in, ns);
-    add(out, f->wall_net, ns);
-    add(out, f->roof_in_dir, ns);
-    add(out, f->wall_in_dir, ns);
-    add(out, f->clear_air_abs, ns);
-    add(out, f->veg_abs, ns);
-    add(out, f->veg_air_abs, ns);
-    add(out, f->veg_abs_dir, ns);
-    add(out, f->flux_dn_layer_top, ns);
-    add(out, f->flux_up_layer_top, ns);
-    add(out, f->flux_dn_layer_base, ns);
-    add(out, f->flux_up_layer_base, ns);
-    add(out, f->flux_dn_dir_layer_top, ns);
-    add(out, f->flux_dn_dir_layer_base, ns);
-    add(out, f->roof_sunlit_frac, 1);
-    add(out, f->wall_sunlit_frac, 1);
-    add(out, f->veg_sunlit_frac, 1);
+  typedef double *ssb200_canopy_flux::*Member;
+  static const Member spectral[] = {
+      &ssb200_canopy_flux::roof_in,           &ssb200_canopy_flux::roof_net,
+      &ssb200_canopy_flux::wall_in,           &ssb200_canopy_flux::wall_net,
+      &ssb200_canopy_flux::roof_in_dir,       &ssb200_canopy_flux::wall_in_dir,
+      &ssb200_canopy_flux::clear_air_abs,     &ssb200_canopy_flux::veg_abs,
+      &ssb200_canopy_flux::veg_air_abs,       &ssb200_canopy_flux::veg_abs_dir,
+      &ssb200_canopy_flux::flux_dn_layer_top, &ssb200_canopy_flux::flux_up_layer_top,
+      &ssb200_canopy_flux::flux_dn_layer_base, &ssb200_canopy_flux::flux_up_layer_base,
+      &ssb200_canopy_flux::flux_dn_dir_layer_top, &ssb200_canopy_flux::flux_dn_dir_layer_base};
+  static const Member sunlit[] = {&ssb200_canopy_flux::roof_sunlit_frac, &ssb200_canopy_flux::wall_sunlit_frac,
+                                  &ssb200_canopy_flux::veg_sunlit_frac};
+  if (!sum) {
+    for (ssb200_canopy_flux *f : {&b.f1, &b.f2}) {
+      for (Member m : spectral) add(out, f->*m, ns);
+      for (Member m : sunlit) add(out, f->*m, 1);
+    }
+    return elems;
   }
+  auto pair = [&](Member m, int w, unsigned char mode) {
+    double *sa = add(nullptr, b.f1.*m, w), *sb = add(nullptr, b.f2.*m, w);
+    if (!out || !sa || !sb || !(sum->*m)) return;
+    out->ref[out->n] = sum->*m;
+    out->staged[out->n] = sa;
+    out->staged2[out->n] = sb;
+    out->nspec[out->n] = w;
+    out->f32[out->n] = 0;
+    out->sum[out->n] = mode;
+    ++out->n;
+  };
+  for (Member m : spectral) pair(m, ns, kSumScaled);
+  for (Member m : sunlit) pair(m, 1, kSumPlain);
   return elems;
 }
 
@@ -254,6 +274,14 @@ struct Dispatcher {
   // the per-layer members of the call are the caller's float arrays, read and written through the
   // level-major staging only (ssb200_radsurf_device_sp; see all_layers_staged)
   bool f32_layers = false;
+  // summing scatter of each pass (ssb200_radsurf_fluxes_device; only valid when all_layers_staged holds):
+  // the per-layer members of f1 and f2 exist in the staging buffers of a chunk only, and the scatter
+  // writes their scaled sum into `out`.  The per-column members are left to the caller.
+  struct PassSum {
+    const ssb200_canopy_flux *out = nullptr;  // NULL: plain scatter into f1 and f2
+    const double *fa = nullptr, *fb = nullptr, *fb_minus = nullptr;
+  };
+  PassSum sum_sw, sum_lw;
   explicit Dispatcher(Backend &b) : be(b) {}
 
   static SolveCfg class_cfg(const ssb200_config &cfg, const ColumnClass &k, bool lw) {
@@ -369,7 +397,12 @@ struct Dispatcher {
       if (staged) {
         double *cursor = a.sweep + (rec ? scratch_doubles((size_t)r_op, (size_t)lmax, width)
                                         : scratch_doubles(es, (size_t)lmax + 1, width));
-        stage_plan(b, lw, (size_t)lmax * cnt, cursor, &sin.list, &sout.list, f32_layers);
+        const PassSum &ps = lw ? sum_lw : sum_sw;
+        stage_plan(b, lw, (size_t)lmax * cnt, cursor, &sin.list, &sout.list, f32_layers, ps.out);
+        sin.fa = sin.fb = sin.fb_minus = nullptr;
+        sout.fa = ps.fa;
+        sout.fb = ps.fb;
+        sout.fb_minus = ps.fb_minus;
         b.lstride = (int)cnt;
         sin.cols = sout.cols = a.cols;
         sin.nlay = sout.nlay = a.nlay;

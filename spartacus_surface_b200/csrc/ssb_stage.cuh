@@ -25,12 +25,38 @@ struct StageList {
   // 1: `ref` really holds float (ssb200_radsurf_device_sp): the gather widens exactly, the scatter
   // rounds to nearest, so the kernels see the same doubles as the double entry on widened inputs
   unsigned char f32[kStageMaxArrays];
+  // summing scatter (ssb200_radsurf_fluxes_device): `ref` is a member of the summed flux object and
+  // receives a combination of `staged` (the member of f1) and `staged2` (the same member of f2).
+  // kSumScaled: fa * a + (fb - fb_minus) * b per (interval, column); kSumPlain: a + b (sunlit fractions)
+  unsigned char sum[kStageMaxArrays];
+  double *staged2[kStageMaxArrays];
 };
+enum { kSumNone = 0, kSumScaled = 1, kSumPlain = 2 };
 struct StageArgs {
   StageList list;
   const int *cols, *nlay, *istartlay;
   int ncols, lmax;
+  // factors of the summing scatter, (nspec, ncol) in reference layout: fa NULL means 1, fb_minus
+  // non-NULL means fb - fb_minus (canopy_flux_type%scale followed by %sum, driver:250-261)
+  const double *fa, *fb, *fb_minus;
 };
+
+// One summed value, rounded as canopy_flux_type%scale (one product per object) followed by %sum
+// (radsurf/radsurf_canopy_flux.F90:212-282,399-460); `f` indexes the factors, g + nspec * col.
+// Written with explicit round-to-nearest operations so that no FMA contraction changes the bits.
+SSB_HDI double stage_sum(const StageArgs &s, int k, double a, double b, size_t f) {
+#if defined(__CUDA_ARCH__)
+  if (s.list.sum[k] == kSumPlain) return __dadd_rn(a, b);
+  const double xa = s.fa ? __dmul_rn(s.fa[f], a) : a;
+  const double fbk = s.fb_minus ? __dadd_rn(s.fb[f], -s.fb_minus[f]) : s.fb[f];
+  return __dadd_rn(xa, __dmul_rn(fbk, b));
+#else  // (the host check is compiled with -ffp-contract=off)
+  if (s.list.sum[k] == kSumPlain) return a + b;
+  const double xa = s.fa ? s.fa[f] * a : a;
+  const double fbk = s.fb_minus ? s.fb[f] - s.fb_minus[f] : s.fb[f];
+  return xa + fbk * b;
+#endif
+}
 
 // serial form (host check)
 inline void stage_host(const StageArgs &s, bool scatter) {
@@ -41,8 +67,11 @@ inline void stage_host(const StageArgs &s, bool scatter) {
       for (int lev = 0; lev < s.nlay[col]; ++lev)
         for (int g = 0; g < ns; ++g) {
           const size_t ri = (size_t)g + (size_t)ns * (size_t)(il1 + lev);
-          double &t = s.list.staged[k][(size_t)g + (size_t)ns * ((size_t)ic + (size_t)lev * (size_t)s.ncols)];
-          if (s.list.f32[k]) {
+          const size_t si = (size_t)g + (size_t)ns * ((size_t)ic + (size_t)lev * (size_t)s.ncols);
+          double &t = s.list.staged[k][si];
+          if (s.list.sum[k]) {  // (scatter only)
+            s.list.ref[k][ri] = stage_sum(s, k, t, s.list.staged2[k][si], (size_t)g + (size_t)ns * (size_t)col);
+          } else if (s.list.f32[k]) {
             float &r = reinterpret_cast<float *>(s.list.ref[k])[ri];
             if (scatter)
               r = (float)t;  // round to nearest even
@@ -69,7 +98,8 @@ __device__ __forceinline__ float stage_out(float *, double v) { return __double2
 
 // blockIdx.x: tile of `tc` chunk columns, blockIdx.y: array.  `lb` levels per pass of the tile.
 // R: element type of the caller's side (double, or float for the single-precision device entry).
-template <bool SCATTER, class R>
+// SUM: summing scatter (StageList::sum): the tile receives the combination of both staged objects.
+template <bool SCATTER, class R, bool SUM = false>
 __global__ void __launch_bounds__(kStageBlock) k_stage(StageArgs s, int tc, int lb) {
   __shared__ double tile[kStageTile + 2 * 64];
   const int k = blockIdx.y, ns = s.list.nspec[k];
@@ -98,8 +128,14 @@ __global__ void __launch_bounds__(kStageBlock) k_stage(StageArgs s, int tc, int 
     } else {
       for (int idx = threadIdx.x; idx < total; idx += kStageBlock) {
         const int l = idx / row, r = idx % row, c = r / ns;
-        if (l0 + l < s.nlay[s.cols[ic0 + c]])
-          tile[l * pitch + r] = stg[(size_t)(r % ns) + (size_t)ns * ((size_t)(ic0 + c) + (size_t)(l0 + l) * (size_t)s.ncols)];
+        const int col = s.cols[ic0 + c];
+        if (l0 + l < s.nlay[col]) {
+          const size_t si = (size_t)(r % ns) + (size_t)ns * ((size_t)(ic0 + c) + (size_t)(l0 + l) * (size_t)s.ncols);
+          if constexpr (SUM)
+            tile[l * pitch + r] = stage_sum(s, k, stg[si], s.list.staged2[k][si], (size_t)(r % ns) + (size_t)ns * (size_t)col);
+          else
+            tile[l * pitch + r] = stg[si];
+        }
       }
       __syncthreads();
       for (int idx = threadIdx.x; idx < total; idx += kStageBlock) {
@@ -116,8 +152,8 @@ __global__ void __launch_bounds__(kStageBlock) k_stage(StageArgs s, int tc, int 
 // Arrays with one value per layer (every array when nsw = nlw = 1): no tile needed.  A thread moves four
 // vertically adjacent layers of one column of every array: on the reference side that is one full 32-byte
 // sector per array (16 bytes for float), on the staged side four rows in which neighbouring threads are
-// neighbouring columns.
-template <bool SCATTER, class R>
+// neighbouring columns.  SUM: summing scatter, as in k_stage.
+template <bool SCATTER, class R, bool SUM = false>
 __global__ void __launch_bounds__(kStageBlock) k_stage1(StageArgs s) {
   // neighbouring threads take neighbouring groups of four layers of ONE column: on the reference side a
   // warp then covers whole 128-byte lines (8 columns x 16 layers when every column has 16 layers)
@@ -180,9 +216,16 @@ __global__ void __launch_bounds__(kStageBlock) k_stage1(StageArgs s) {
         for (int j = 0; j < 4; ++j)
           if (j < cnt) stg[j * pitch] = v[j];
       } else {
+        if constexpr (SUM) {
+          const double *stg2 = s.list.staged2[k] + sbase;
 #pragma unroll
-        for (int j = 0; j < 4; ++j)
-          if (j < cnt) v[j] = __ldcs(stg + j * pitch);
+          for (int j = 0; j < 4; ++j)
+            if (j < cnt) v[j] = stage_sum(s, k, __ldcs(stg + j * pitch), __ldcs(stg2 + j * pitch), (size_t)col);
+        } else {
+#pragma unroll
+          for (int j = 0; j < 4; ++j)
+            if (j < cnt) v[j] = __ldcs(stg + j * pitch);
+        }
         if (vec) {
           __stcs((double2 *)ref, make_double2(v[0], v[1]));
           __stcs((double2 *)ref + 1, make_double2(v[2], v[3]));
@@ -196,12 +239,12 @@ __global__ void __launch_bounds__(kStageBlock) k_stage1(StageArgs s) {
   }
 }
 
-template <bool SCATTER, class R>
+template <bool SCATTER, class R, bool SUM = false>
 inline void stage_launch_group(const StageArgs &g, int ns, cudaStream_t st) {
   if (ns == 1) {
     const long nthreads = (long)g.ncols * ((g.lmax + 3) / 4);
     const unsigned blocks = (unsigned)((nthreads + kStageBlock - 1) / kStageBlock);
-    k_stage1<SCATTER, R><<<blocks, kStageBlock, 0, st>>>(g);
+    k_stage1<SCATTER, R, SUM><<<blocks, kStageBlock, 0, st>>>(g);
     return;
   }
   int lb = g.lmax < 32 ? g.lmax : 32;
@@ -209,11 +252,12 @@ inline void stage_launch_group(const StageArgs &g, int ns, cudaStream_t st) {
   int tc = kStageTile / (lb * ns);
   tc = tc > 64 ? 64 : (tc < 1 ? 1 : tc);
   const dim3 grid((unsigned)((g.ncols + tc - 1) / tc), (unsigned)g.list.n);
-  k_stage<SCATTER, R><<<grid, kStageBlock, 0, st>>>(g, tc, lb);
+  k_stage<SCATTER, R, SUM><<<grid, kStageBlock, 0, st>>>(g, tc, lb);
 }
 
 // launches one grid per group of arrays with the same spectral width (the tile shape depends on it) and
-// the same element type on the caller's side
+// the same element type on the caller's side (a summing scatter sums every array of its list: its
+// scaled and plain members share the grid of their width)
 inline void stage_launch(const StageArgs &s, bool scatter, cudaStream_t st, long *launches) {
   if (s.list.n == 0 || s.ncols <= 0 || s.lmax <= 0) return;
   int done[kStageMaxArrays] = {0};
@@ -223,16 +267,21 @@ inline void stage_launch(const StageArgs &s, bool scatter, cudaStream_t st, long
     g.list.n = 0;
     const int ns = s.list.nspec[k0];
     const unsigned char f32 = s.list.f32[k0];
+    const bool sum = s.list.sum[k0] != kSumNone;
     for (int k = k0; k < s.list.n; ++k)
-      if (!done[k] && s.list.nspec[k] == ns && s.list.f32[k] == f32) {
+      if (!done[k] && s.list.nspec[k] == ns && s.list.f32[k] == f32 && (s.list.sum[k] != kSumNone) == sum) {
         g.list.ref[g.list.n] = s.list.ref[k];
         g.list.staged[g.list.n] = s.list.staged[k];
+        g.list.staged2[g.list.n] = s.list.staged2[k];
         g.list.nspec[g.list.n] = ns;
         g.list.f32[g.list.n] = f32;
+        g.list.sum[g.list.n] = s.list.sum[k];
         ++g.list.n;
         done[k] = 1;
       }
-    if (f32)
+    if (sum)  // (double caller side only: ssb200_radsurf_fluxes_device)
+      stage_launch_group<true, double, true>(g, ns, st);
+    else if (f32)
       scatter ? stage_launch_group<true, float>(g, ns, st) : stage_launch_group<false, float>(g, ns, st);
     else
       scatter ? stage_launch_group<true, double>(g, ns, st) : stage_launch_group<false, double>(g, ns, st);

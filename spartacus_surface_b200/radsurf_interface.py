@@ -2,7 +2,8 @@
 
 Same argument list and meaning as the reference subroutine; the body is the
 B200 library (ssb200_radsurf for host arrays, ssb200_radsurf_device when the
-members are torch CUDA tensors; the _sp wrappers below take float32 arrays).  The reference aborts on error
+members are torch CUDA tensors; radsurf_fluxes likewise picks ssb200_radsurf_fluxes or
+ssb200_radsurf_fluxes_device; the _sp wrappers below take float32 arrays).  The reference aborts on error
 (utilities/radiation_io.F90:46-54); here errors raise RadsurfError.
 """
 import ctypes as C
@@ -72,19 +73,27 @@ def radsurf(config, canopy_props, sw_spectral_props, lw_spectral_props, bc_out,
 def radsurf_fluxes(config, canopy_props, sw_spectral_props, lw_spectral_props, bc_out, istartcol=None, iendcol=None,
                    sw_flux=None, lw_flux=None, top_flux_dn_sw=None, top_flux_dn_direct_sw=None, top_flux_dn_lw=None,
                    ground_temperature=None, roof_temperature=None, wall_temperature=None,
-                   clear_air_temperature=None, veg_temperature=None, veg_air_temperature=None):
+                   clear_air_temperature=None, veg_temperature=None, veg_air_temperature=None, stream=None):
     """The reference driver's sequence for a block of columns in one call
     (driver/spartacus_surface_driver.F90:206-261): calc_simple_spectrum_lw, radsurf,
     scale of the normalised fluxes by the top-of-canopy fluxes and sum into `sw_flux` / `lw_flux`.
-    The four normalised flux objects never leave the device; members of the spectral property
+    The four normalised flux objects are never returned; members of the spectral property
     objects that are None take read_input's defaults or are derived from the temperatures
-    (include/spartacus_b200.h: ssb200_radsurf_fluxes).  Host (numpy) arrays."""
+    (include/spartacus_b200.h: ssb200_radsurf_fluxes).  numpy members: ssb200_radsurf_fluxes (host
+    arrays).  torch CUDA float64 members, top-of-canopy fluxes and temperatures included:
+    ssb200_radsurf_fluxes_device, enqueued on `stream` (cudaStream_t as an int, None = default stream)
+    without synchronising.  A mix of numpy arrays and tensors, or a float32 tensor, raises RadsurfError."""
     from . import _abi
     lib = load()
-    structs = marshal(config, canopy_props, sw_spectral_props, lw_spectral_props, bc_out)
     keep = [np_ for np_ in (top_flux_dn_sw, top_flux_dn_direct_sw, top_flux_dn_lw, ground_temperature,
                             roof_temperature, wall_temperature, clear_air_temperature, veg_temperature,
                             veg_air_temperature)]
+    members = list(_float_members(canopy_props, sw_spectral_props, lw_spectral_props, bc_out, sw_flux, lw_flux))
+    members += [a for a in keep if a is not None]
+    if any(is_torch(v) for v in members):
+        return _radsurf_fluxes_device(lib, members, keep, config, canopy_props, sw_spectral_props,
+                                      lw_spectral_props, bc_out, istartcol, iendcol, sw_flux, lw_flux, stream)
+    structs = marshal(config, canopy_props, sw_spectral_props, lw_spectral_props, bc_out)
     drv = _abi.DriverInputs(*[_abi.dptr(a) for a in keep])
     fsw = sw_flux.as_struct() if sw_flux is not None else None
     flw = lw_flux.as_struct() if lw_flux is not None else None
@@ -94,6 +103,40 @@ def radsurf_fluxes(config, canopy_props, sw_spectral_props, lw_spectral_props, b
     if rc < 0:
         raise RadsurfError(f"ssb200_radsurf_fluxes failed (rc={rc}): {last_error()}")
     return rc
+
+
+def _radsurf_fluxes_device(lib, members, keep, config, canopy_props, sw_spectral_props, lw_spectral_props, bc_out,
+                           istartcol, iendcol, sw_flux, lw_flux, stream):
+    from . import _abi
+    if not all(is_torch(v) for v in members):
+        raise RadsurfError("radsurf_fluxes: members mix numpy arrays and torch tensors")
+    ptr = f64_cuda_ptr("radsurf_fluxes")
+    structs = marshal(config, canopy_props, sw_spectral_props, lw_spectral_props, bc_out, ptr=ptr)
+    drv = _abi.DriverInputs(*[ptr(a) for a in keep])
+    fsw = sw_flux.as_struct(ptr) if sw_flux is not None else None
+    flw = lw_flux.as_struct(ptr) if lw_flux is not None else None
+    s = structs
+    rc = lib.ssb200_radsurf_fluxes_device(_ref(s["config"]), _ref(s["canopy"]), _ref(s["sw"]), _ref(s["lw"]),
+                                          C.byref(drv), _ref(s["bc"]), int(istartcol or 0), int(iendcol or 0),
+                                          _ref(fsw), _ref(flw), C.c_void_p(stream or 0), None)
+    if rc < 0:
+        raise RadsurfError(f"ssb200_radsurf_fluxes_device failed (rc={rc}): {last_error()}")
+    return rc
+
+
+def f64_cuda_ptr(where):
+    """Address function for the double-precision device entries that check their members: contiguous float64
+    torch CUDA tensors only; anything else raises RadsurfError."""
+    _dp = C.POINTER(C.c_double)
+
+    def ptr(a):
+        if a is None:
+            return C.cast(None, _dp)
+        import torch
+        if is_torch(a) and a.is_cuda and a.dtype == torch.float64 and a.is_contiguous():
+            return C.cast(a.data_ptr(), _dp)
+        raise RadsurfError(f"{where}: every real member must be a contiguous float64 CUDA tensor")
+    return ptr
 
 
 def _float_members(*objs):
