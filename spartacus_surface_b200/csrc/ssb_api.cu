@@ -257,6 +257,27 @@ struct DevBuf {
   }
 };
 
+// Grow-only pool over one of the context's buffer vectors: the i-th request of a call reuses the i-th
+// buffer.  The first allocation error is kept in `rc` (message prefixed by `what`); later requests
+// return NULL.
+struct Pool {
+  std::vector<DevBuf> &bufs;
+  const char *what;
+  size_t next = 0;
+  int rc = 0;
+  template <class T>
+  T *get(size_t n) {
+    if (rc) return nullptr;
+    if (next >= bufs.size()) bufs.resize(next + 16);
+    const cudaError_t e = bufs[next++].reserve(std::max(n, (size_t)1) * sizeof(T));
+    if (e != cudaSuccess) {
+      rc = fail(SSB200_ERR_CUDA, std::string(what) + cudaGetErrorString(e));
+      return nullptr;
+    }
+    return (T *)bufs[next - 1].p;
+  }
+};
+
 struct Context {
   ssb::Plan plan;
   bool plan_uploaded = false;
@@ -658,6 +679,17 @@ int finish_device_call(Context &cx, cudaStream_t stream, int32_t *status_out) {
   return 0;
 }
 
+// Synchronises `s` on scope exit unless disarmed: an error return of a device entry after its first
+// launch must not leave work queued on the context's buffers (a later call on another stream, or
+// ssb200_release, would not wait for it).
+struct Drain {
+  cudaStream_t s;
+  bool armed = true;
+  ~Drain() {
+    if (armed) cudaStreamSynchronize(s);
+  }
+};
+
 // Core of both entry points; all double arrays are device pointers here.
 // `blocks`: when non-null the call only prepares (plan, status, budget) and returns the
 // clamped 1-based column range in blocks[0..1]; the caller then dispatches column
@@ -748,52 +780,142 @@ int ensure_lay2col(Context &cx, size_t ncol, size_t ntot, cudaStream_t st) {
   return 0;
 }
 
+// The members of `o` that k_scale / k_sum / k_scale_sum visit.  with_sunlit: also the non-spectral
+// members (sunlit fractions); with_layers: also the per-layer ones.  Given `a`, a member that `a` or `b`
+// lacks is left out.
 static int collect_fields(ssb200_canopy_flux *o, const ssb200_canopy_flux *a, const ssb200_canopy_flux *b,
-                          FieldList &fl, bool with_sunlit) {
+                          FieldList &fl, bool with_sunlit, bool with_layers = true) {
   fl.n = 0;
-  auto add = [&](double *p, const double *pa, const double *pb, int per_layer, int spectral) {
-    if (!p) return;
-    if (a && (!pa || !pb)) return;
+  for (const ssb::FluxMember &m : ssb::kFluxMembers) {
+    double *p = o->*m.ptr;
+    const double *pa = a ? a->*m.ptr : nullptr, *pb = b ? b->*m.ptr : nullptr;
+    if (!p || (!m.spectral && !with_sunlit) || (m.per_layer && !with_layers) || (a && (!pa || !pb))) continue;
     fl.p[fl.n] = p;
     fl.a[fl.n] = pa;
     fl.b[fl.n] = pb;
-    fl.per_layer[fl.n] = per_layer;
-    fl.spectral[fl.n] = spectral;
+    fl.per_layer[fl.n] = m.per_layer;
+    fl.spectral[fl.n] = m.spectral;
     ++fl.n;
-  };
-#define F(m, pl, sp) add(o->m, a ? a->m : nullptr, b ? b->m : nullptr, pl, sp)
-  F(ground_dn, 0, 1);
-  F(ground_net, 0, 1);
-  F(ground_vertical_diff, 0, 1);
-  F(top_dn, 0, 1);
-  F(top_net, 0, 1);
-  F(ground_dn_dir, 0, 1);
-  F(top_dn_dir, 0, 1);
-  F(roof_in, 1, 1);
-  F(roof_net, 1, 1);
-  F(wall_in, 1, 1);
-  F(wall_net, 1, 1);
-  F(roof_in_dir, 1, 1);
-  F(wall_in_dir, 1, 1);
-  F(clear_air_abs, 1, 1);
-  F(veg_abs, 1, 1);
-  F(veg_air_abs, 1, 1);
-  F(veg_abs_dir, 1, 1);
-  F(flux_dn_layer_top, 1, 1);
-  F(flux_up_layer_top, 1, 1);
-  F(flux_dn_layer_base, 1, 1);
-  F(flux_up_layer_base, 1, 1);
-  F(flux_dn_dir_layer_top, 1, 1);
-  F(flux_dn_dir_layer_base, 1, 1);
-  if (with_sunlit) {
-    F(ground_sunlit_frac, 0, 0);
-    F(roof_sunlit_frac, 1, 0);
-    F(wall_sunlit_frac, 1, 0);
-    F(veg_sunlit_frac, 1, 0);
   }
-#undef F
   return fl.n;
 }
+
+// Packed layers [l0, l1) of the non-Flat columns in [c0, c1) (0-based).  contiguous: the layers of each
+// such column follow those of the previous one.  ok = false: some column's layers lie outside
+// 1..ntotlay (that column is left out of the range).
+struct LayerSpan {
+  size_t l0 = 0, l1 = 0;
+  bool contiguous = true, ok = true;
+};
+LayerSpan layer_span(const ssb200_canopy_properties &cp, size_t c0, size_t c1) {
+  LayerSpan r;
+  const size_t ntot = (size_t)cp.ntotlay;
+  size_t lo = ntot, hi = 0, expect = 0;
+  bool first = true;
+  for (size_t j = c0; j < c1; ++j) {
+    if (cp.i_representation[j] == SSB200_TILE_FLAT || cp.nlay[j] <= 0) continue;
+    const size_t s = (size_t)cp.istartlay[j] - 1, e = s + (size_t)cp.nlay[j];
+    if (cp.istartlay[j] < 1 || e > ntot) {
+      r.ok = false;
+      continue;
+    }
+    if (!first && s != expect) r.contiguous = false;
+    first = false;
+    expect = e;
+    lo = std::min(lo, s);
+    hi = std::max(hi, e);
+  }
+  if (hi > lo) {
+    r.l0 = lo;
+    r.l1 = hi;
+  }
+  return r;
+}
+
+// What the driver sequence derives for the members the caller leaves NULL: read_input's defaults and
+// sigma T^4 emission from the temperatures.  Both driver-sequence entries plan it here; each launches
+// fill() over the call's layers and derive() per column window of its own schedule.
+struct DriverStage {
+  struct Fill {  // constant, per packed layer
+    double *p;
+    double v;
+    size_t width;
+  };
+  struct Emis {  // out = sigma [emissivity] T^4, interval 1
+    double *out;
+    const double *emissivity, *temperature;
+    bool per_layer;
+  };
+  std::vector<Fill> fills;
+  std::vector<Emis> emis;
+  double *vcf = nullptr;  // default veg_contact_fraction (per packed layer)
+
+  // Points the NULL members of the device-array structs cp / sw / lw at buffers of `pool`.  The
+  // temperatures of `emis` are those of `drv`.  Returns 0 or a negative SSB200_ERR_* code.
+  int plan(const ssb200_config &cfg, const ssb200_driver_inputs &drv, size_t ncol, size_t ntot,
+           ssb200_canopy_properties &cp, ssb200_sw_spectral_properties &sw, ssb200_lw_spectral_properties &lw,
+           Pool &pool) {
+    if (!cp.veg_contact_fraction && cp.veg_fraction && cp.building_fraction) {
+      vcf = pool.get<double>(ntot);  // driver/spartacus_surface_read_input.F90:155-166
+      cp.veg_contact_fraction = vcf;
+    }
+    auto filled = [&](const double *&slot, size_t width, double v) {
+      slot = pool.get<double>(ntot * width);
+      fills.push_back(Fill{const_cast<double *>(slot), v, width});
+    };
+    if (cfg.do_sw) {  // driver/spartacus_surface_read_input.F90:258-269,335-344 (roof_albedo_dir NULL: the kernels use roof_albedo)
+      const size_t g = (size_t)cfg.nsw;
+      if (!sw.air_ext) filled(sw.air_ext, g, 1.0e-5);
+      if (!sw.air_ssa) filled(sw.air_ssa, g, 0.999);
+      if (!sw.wall_specular_frac && sw.wall_albedo) filled(sw.wall_specular_frac, g, 0.0);
+    }
+    if (cfg.do_lw) {  // driver/spartacus_surface_read_input.F90:362-365; radsurf_simple_spectrum.F90:41-66
+      const size_t g = (size_t)cfg.nlw;
+      if (!lw.air_ext) filled(lw.air_ext, g, 1.0e-5);
+      if (!lw.air_ssa) filled(lw.air_ssa, g, 0.0);
+      const bool need_t = !lw.ground_emission || !lw.roof_emission || !lw.wall_emission || !lw.clear_air_planck ||
+                          !lw.veg_planck || !lw.veg_air_planck;
+      if (need_t && g != 1)
+        return fail(SSB200_ERR_ARG, "Simple longwave spectrum only possible with one input spectral interval");
+      auto emission = [&](const double *&slot, const double *emissivity, const double *t, bool per_layer) {
+        if (slot || !t) return;
+        slot = pool.get<double>(per_layer ? ntot : ncol);
+        emis.push_back(Emis{const_cast<double *>(slot), emissivity, t, per_layer});
+      };
+      emission(lw.ground_emission, lw.ground_emissivity, drv.ground_temperature, false);
+      emission(lw.roof_emission, lw.roof_emissivity, drv.roof_temperature, true);
+      emission(lw.wall_emission, lw.wall_emissivity, drv.wall_temperature, true);
+      emission(lw.clear_air_planck, nullptr, drv.clear_air_temperature, true);
+      emission(lw.veg_planck, nullptr, drv.veg_temperature, true);
+      emission(lw.veg_air_planck, nullptr, drv.veg_air_temperature, true);
+    }
+    return pool.rc;
+  }
+  void fill(size_t l0, size_t l1, cudaStream_t st) const {
+    for (const Fill &f : fills) {
+      const long i0 = (long)(l0 * f.width), i1 = (long)(l1 * f.width);
+      if (i1 <= i0) continue;
+      k_fill<<<(unsigned)((i1 - i0 + 255) / 256), 256, 0, st>>>(f.p, f.v, i0, i1);
+      ++g_launches;
+    }
+  }
+  // default contact fraction and emission of columns [c0, c1) and packed layers [l0, l1); cp: the
+  // device arrays of the call
+  void derive(const ssb200_canopy_properties &cp, double min_veg, size_t c0, size_t c1, size_t l0, size_t l1,
+              cudaStream_t st) const {
+    if (vcf && l1 > l0) {
+      k_vcf_default<<<(unsigned)((l1 - l0 + 255) / 256), 256, 0, st>>>(vcf, cp.veg_fraction, cp.building_fraction,
+                                                                        min_veg, (long)l0, (long)l1);
+      ++g_launches;
+    }
+    for (const Emis &e : emis) {
+      const long i0 = (long)(e.per_layer ? l0 : c0), i1 = (long)(e.per_layer ? l1 : c1);
+      if (i1 <= i0) continue;
+      k_sigma_t4<<<(unsigned)((i1 - i0 + 255) / 256), 256, 0, st>>>(e.out, e.emissivity, e.temperature, 1, i0, i1);
+      ++g_launches;
+    }
+  }
+};
 
 // widen every array of `v` (round = false) or round its outputs back (true) on `st`, kConvMax arrays per launch
 int convert_arrays(const std::vector<ConvArray> &v, bool round, cudaStream_t st) {
@@ -830,10 +952,7 @@ int convert_arrays(const std::vector<ConvArray> &v, bool round, cudaStream_t st)
 
 // --- host-pointer staging --------------------------------------------------
 struct Stager {
-  Context &cx;
-  cudaStream_t stream;
-  int next = 0;
-  int rc = 0;
+  Pool pool;  // device mirrors and device-only arrays of the call
   struct Arr {
     double *host;    // (sp: really float *)
     double *dev;
@@ -845,43 +964,15 @@ struct Stager {
   // single-precision storage (ssb200_radsurf_sp): the caller's arrays hold float; they cross PCIe as
   // float and are widened / rounded on the device, the kernels see double mirrors as always
   bool sp = false;
-  Stager(Context &c, cudaStream_t s, bool sp_ = false) : cx(c), stream(s), sp(sp_) {}
+  Stager(Context &c, bool sp_) : pool{c.stage, "staging allocation: "}, sp(sp_) {}
   // device mirror of `host` (total = rows * width doubles); copies are issued per window
   double *mirror(const double *host, size_t rows, size_t width, bool per_layer, bool upload, bool download) {
-    if (!host || rc) return nullptr;
-    if ((size_t)next >= cx.stage.size()) cx.stage.resize((size_t)next + 16);
-    DevBuf &b = cx.stage[next++];
-    const size_t total = rows * width;
-    cudaError_t e = b.reserve((total > 0 ? total : 1) * sizeof(double));
-    if (e != cudaSuccess) {
-      rc = fail(SSB200_ERR_CUDA, std::string("staging allocation: ") + cudaGetErrorString(e));
-      return nullptr;
-    }
-    float *d32 = nullptr;
-    if (sp) {
-      if ((size_t)next >= cx.stage.size()) cx.stage.resize((size_t)next + 16);
-      DevBuf &b32 = cx.stage[next++];
-      e = b32.reserve((total > 0 ? total : 1) * sizeof(float));
-      if (e != cudaSuccess) {
-        rc = fail(SSB200_ERR_CUDA, std::string("staging allocation: ") + cudaGetErrorString(e));
-        return nullptr;
-      }
-      d32 = (float *)b32.p;
-    }
-    arrs.push_back(Arr{const_cast<double *>(host), (double *)cx.stage[next - (sp ? 2 : 1)].p, d32, width, per_layer, upload, download});
-    return arrs.back().dev;
-  }
-  // device-only array (no host counterpart: never copied)
-  double *device_only(size_t total) {
-    if (rc) return nullptr;
-    if ((size_t)next >= cx.stage.size()) cx.stage.resize((size_t)next + 16);
-    DevBuf &b = cx.stage[next++];
-    cudaError_t e = b.reserve((total > 0 ? total : 1) * sizeof(double));
-    if (e != cudaSuccess) {
-      rc = fail(SSB200_ERR_CUDA, std::string("staging allocation: ") + cudaGetErrorString(e));
-      return nullptr;
-    }
-    return (double *)b.p;
+    if (!host) return nullptr;
+    double *dev = pool.get<double>(rows * width);
+    float *dev32 = sp ? pool.get<float>(rows * width) : nullptr;
+    if (pool.rc) return nullptr;
+    arrs.push_back(Arr{const_cast<double *>(host), dev, dev32, width, per_layer, upload, download});
+    return dev;
   }
   // copy the slices of columns [c0, c1) / packed layers [l0, l1) on stream `st`
   int copy_window(bool to_device, size_t c0, size_t c1, size_t l0, size_t l1, cudaStream_t st) {
@@ -1042,42 +1133,29 @@ static int radsurf_device_sp_locked(Context &cx, const ssb::CallArgs &ca, int32_
   const bool staged = route.all_layers_staged(ca, cx.plan);
   const size_t ncol = (size_t)cp.ncol, ntot = (size_t)cp.ntotlay;
   const size_t c0 = (size_t)range[0] - 1, c1 = (size_t)range[1];
-  size_t l0 = ntot, l1 = 0;  // packed layers of the call's columns (fallback route)
-  if (!staged)
-    for (size_t j = c0; j < c1; ++j)
-      if (cp.i_representation[j] != SSB200_TILE_FLAT && cp.nlay[j] > 0) {
-        l0 = std::min(l0, (size_t)cp.istartlay[j] - 1);
-        l1 = std::max(l1, (size_t)cp.istartlay[j] - 1 + (size_t)cp.nlay[j]);
-      }
-  if (l1 < l0) l0 = l1 = 0;
+  LayerSpan span;  // packed layers of the call's columns (fallback route)
+  if (!staged) span = layer_span(cp, c0, c1);
   std::vector<ConvArray> conv;
-  size_t next = 0;
-  int err_rc = 0;
+  Pool pool{cx.wide, "double copies: "};
   // double buffer for the float array p of `rows` x `width` values; rows [r0, r1) are converted
   auto wide = [&](const void *p, size_t rows, size_t width, size_t r0, size_t r1, bool out) -> double * {
-    if (!p || err_rc) return nullptr;
-    if (next >= cx.wide.size()) cx.wide.resize(next + 16);
-    DevBuf &b = cx.wide[next++];
-    const cudaError_t e = b.reserve(std::max(rows * width, (size_t)1) * sizeof(double));
-    if (e != cudaSuccess) {
-      err_rc = fail(SSB200_ERR_CUDA, std::string("double copies: ") + cudaGetErrorString(e));
-      return nullptr;
-    }
-    conv.push_back(ConvArray{(float *)p, (double *)b.p, (long)(r0 * width), (long)(r1 * width), out});
-    return (double *)b.p;
+    if (!p) return nullptr;
+    double *d = pool.get<double>(rows * width);
+    if (d) conv.push_back(ConvArray{(float *)p, d, (long)(r0 * width), (long)(r1 * width), out});
+    return d;
   };
-  auto C = [&](const void *p, size_t w, bool out) { return wide(p, ncol, w, c0, c1, out); };
-  auto L = [&](const void *p, size_t w, bool out) { return staged ? (double *)p : wide(p, ntot, w, l0, l1, out); };
+  // the members of `d` as the kernels see them: per-column members widened over the call's columns,
+  // per-layer members passed to the staging (staged route) or widened over the call's layers
+  auto widen = [&](auto &d, const auto &table, size_t nspec, bool out) {
+    for (const auto &m : table) {
+      const size_t w = ssb::member_width(m, nspec);
+      const void *p = d.*m.ptr;
+      d.*m.ptr = !m.per_layer ? wide(p, ncol, w, c0, c1, out)
+                              : staged ? (double *)p : wide(p, ntot, w, span.l0, span.l1, out);
+    }
+  };
   ssb200_canopy_properties dcp = cp;
-  dcp.cos_sza = C(cp.cos_sza, 1, false);
-  dcp.dz = L(cp.dz, 1, false);
-  dcp.building_fraction = L(cp.building_fraction, 1, false);
-  dcp.building_scale = L(cp.building_scale, 1, false);
-  dcp.veg_fraction = L(cp.veg_fraction, 1, false);
-  dcp.veg_scale = L(cp.veg_scale, 1, false);
-  dcp.veg_ext = L(cp.veg_ext, 1, false);
-  dcp.veg_fsd = L(cp.veg_fsd, 1, false);
-  dcp.veg_contact_fraction = L(cp.veg_contact_fraction, 1, false);
+  widen(dcp, ssb::kCanopyMembers, 1, false);
   ssb200_sw_spectral_properties dsw;
   ssb200_lw_spectral_properties dlw;
   ssb200_boundary_conds_out dbc;
@@ -1085,70 +1163,19 @@ static int radsurf_device_sp_locked(Context &cx, const ssb::CallArgs &ca, int32_
   memset(&dlw, 0, sizeof(dlw));
   memset(&dbc, 0, sizeof(dbc));
   if (cfg.do_sw) {
-    const ssb200_sw_spectral_properties &sw = *ca.sw;
-    const size_t g = (size_t)cfg.nsw;
-    dsw.nspec = sw.nspec;
-    dsw.air_ext = L(sw.air_ext, g, false);
-    dsw.air_ssa = L(sw.air_ssa, g, false);
-    dsw.veg_ssa = L(sw.veg_ssa, g, false);
-    dsw.ground_albedo = C(sw.ground_albedo, g, false);
-    dsw.roof_albedo = L(sw.roof_albedo, g, false);
-    dsw.wall_albedo = L(sw.wall_albedo, g, false);
-    dsw.wall_specular_frac = L(sw.wall_specular_frac, g, false);
-    dsw.ground_albedo_dir = C(sw.ground_albedo_dir, g, false);
-    dsw.roof_albedo_dir = L(sw.roof_albedo_dir, g, false);
-    dbc.sw_albedo = C(ca.bc->sw_albedo, g, true);
-    dbc.sw_albedo_dir = C(ca.bc->sw_albedo_dir, g, true);
+    dsw = *ca.sw;
+    widen(dsw, ssb::kSwMembers, (size_t)cfg.nsw, false);
   }
   if (cfg.do_lw) {
-    const ssb200_lw_spectral_properties &lw = *ca.lw;
-    const size_t g = (size_t)cfg.nlw;
-    dlw.nspec = lw.nspec;
-    dlw.air_ext = L(lw.air_ext, g, false);
-    dlw.air_ssa = L(lw.air_ssa, g, false);
-    dlw.clear_air_planck = L(lw.clear_air_planck, g, false);
-    dlw.veg_ssa = L(lw.veg_ssa, g, false);
-    dlw.veg_planck = L(lw.veg_planck, g, false);
-    dlw.veg_air_planck = L(lw.veg_air_planck, g, false);
-    dlw.ground_emissivity = C(lw.ground_emissivity, g, false);
-    dlw.ground_emission = C(lw.ground_emission, g, false);
-    dlw.roof_emissivity = L(lw.roof_emissivity, g, false);
-    dlw.wall_emissivity = L(lw.wall_emissivity, g, false);
-    dlw.roof_emission = L(lw.roof_emission, g, false);
-    dlw.wall_emission = L(lw.wall_emission, g, false);
-    dbc.lw_emissivity = C(ca.bc->lw_emissivity, g, true);
-    dbc.lw_emission = C(ca.bc->lw_emission, g, true);
+    dlw = *ca.lw;
+    widen(dlw, ssb::kLwMembers, (size_t)cfg.nlw, false);
   }
+  for (const ssb::BcMember &m : ssb::kBcMembers)
+    if (m.lw ? cfg.do_lw : cfg.do_sw)
+      dbc.*m.ptr = wide(ca.bc->*m.ptr, ncol, (size_t)(m.lw ? cfg.nlw : cfg.nsw), c0, c1, true);
   auto flux = [&](const ssb200_canopy_flux *h, ssb200_canopy_flux &d) {
     d = *h;
-    const size_t g = (size_t)h->nspec;
-    d.ground_dn = C(h->ground_dn, g, true);
-    d.ground_net = C(h->ground_net, g, true);
-    d.ground_vertical_diff = C(h->ground_vertical_diff, g, true);
-    d.top_dn = C(h->top_dn, g, true);
-    d.top_net = C(h->top_net, g, true);
-    d.ground_dn_dir = C(h->ground_dn_dir, g, true);
-    d.top_dn_dir = C(h->top_dn_dir, g, true);
-    d.ground_sunlit_frac = C(h->ground_sunlit_frac, 1, true);
-    d.roof_in = L(h->roof_in, g, true);
-    d.roof_net = L(h->roof_net, g, true);
-    d.wall_in = L(h->wall_in, g, true);
-    d.wall_net = L(h->wall_net, g, true);
-    d.roof_in_dir = L(h->roof_in_dir, g, true);
-    d.wall_in_dir = L(h->wall_in_dir, g, true);
-    d.roof_sunlit_frac = L(h->roof_sunlit_frac, 1, true);
-    d.wall_sunlit_frac = L(h->wall_sunlit_frac, 1, true);
-    d.clear_air_abs = L(h->clear_air_abs, g, true);
-    d.veg_abs = L(h->veg_abs, g, true);
-    d.veg_air_abs = L(h->veg_air_abs, g, true);
-    d.veg_abs_dir = L(h->veg_abs_dir, g, true);
-    d.veg_sunlit_frac = L(h->veg_sunlit_frac, 1, true);
-    d.flux_dn_layer_top = L(h->flux_dn_layer_top, g, true);
-    d.flux_up_layer_top = L(h->flux_up_layer_top, g, true);
-    d.flux_dn_layer_base = L(h->flux_dn_layer_base, g, true);
-    d.flux_up_layer_base = L(h->flux_up_layer_base, g, true);
-    d.flux_dn_dir_layer_top = L(h->flux_dn_dir_layer_top, g, true);
-    d.flux_dn_dir_layer_base = L(h->flux_dn_dir_layer_base, g, true);
+    widen(d, ssb::kFluxMembers, (size_t)h->nspec, true);
   };
   ssb200_canopy_flux d1, d2, d3, d4;
   if (cfg.do_sw) {
@@ -1159,19 +1186,11 @@ static int radsurf_device_sp_locked(Context &cx, const ssb::CallArgs &ca, int32_
     flux(ca.lw_int, d3);
     flux(ca.lw_norm, d4);
   }
-  if (err_rc) return err_rc;
+  if (pool.rc) return pool.rc;
   ssb::CallArgs wca{ca.config, &dcp, cfg.do_sw ? &dsw : nullptr, cfg.do_lw ? &dlw : nullptr, &dbc,
                     cfg.do_sw ? &d1 : nullptr, cfg.do_sw ? &d2 : nullptr,
                     cfg.do_lw ? &d3 : nullptr, cfg.do_lw ? &d4 : nullptr};
-  // an error return after the first launch must not leave work queued on the context's buffers (a later
-  // call on another stream, or ssb200_release, would not wait for it)
-  struct Drain {
-    cudaStream_t s;
-    bool armed = true;
-    ~Drain() {
-      if (armed) cudaStreamSynchronize(s);
-    }
-  } drain{stream};
+  Drain drain{stream};
   if ((rc = convert_arrays(conv, false, stream))) return rc;
   if ((rc = dispatch_call(cx, wca, staged))) return rc;
   if ((rc = convert_arrays(conv, true, stream))) return rc;
@@ -1214,95 +1233,25 @@ static int radsurf_fluxes_device_locked(Context &cx, const ssb200_config *config
   if (c1 > c2) return 0;
   const size_t c0 = (size_t)c1 - 1, cN = (size_t)c2;  // 0-based column window [c0, cN)
   // packed layers [l0, lN) spanned by the call's columns (ranges outside 1..ntotlay are refused by the plan)
-  size_t l0 = ntot, lN = 0;
-  for (size_t j = c0; j < cN; ++j) {
-    if (cp->i_representation[j] == SSB200_TILE_FLAT || cp->nlay[j] <= 0 || cp->istartlay[j] < 1) continue;
-    const size_t s = (size_t)cp->istartlay[j] - 1, e = s + (size_t)cp->nlay[j];
-    if (e > ntot) continue;
-    l0 = std::min(l0, s);
-    lN = std::max(lN, e);
-  }
-  if (lN < l0) l0 = lN = 0;
-  size_t next = 0;
-  int err_rc = 0;
-  auto buffer = [&](size_t n) -> double * {
-    if (err_rc) return nullptr;
-    if (next >= cx.drv.size()) cx.drv.resize(next + 16);
-    DevBuf &b = cx.drv[next++];
-    const cudaError_t e = b.reserve(std::max(n, (size_t)1) * sizeof(double));
-    if (e != cudaSuccess) {
-      err_rc = fail(SSB200_ERR_CUDA, std::string("context buffers: ") + cudaGetErrorString(e));
-      return nullptr;
-    }
-    return (double *)b.p;
-  };
-  // read_input's defaults and the emission stage, as in radsurf_host
-  struct Fill {
-    double *p;
-    double v;
-    long i0, i1;
-  };
-  struct Emis {
-    double *out;
-    const double *emissivity, *temperature;
-    long i0, i1;
-  };
-  std::vector<Fill> fills;
-  std::vector<Emis> emis;
-  auto filled = [&](size_t width, double v) -> const double * {
-    double *p = buffer(ntot * width);
-    fills.push_back(Fill{p, v, (long)(l0 * width), (long)(lN * width)});
-    return p;
-  };
+  const LayerSpan span = layer_span(*cp, c0, cN);
+  const size_t l0 = span.l0, lN = span.l1;
+  Pool pool{cx.drv, "context buffers: "};
   ssb200_canopy_properties dcp = *cp;
-  double *vcf_default = nullptr;
-  if (!cp->veg_contact_fraction && cp->veg_fraction && cp->building_fraction) {
-    vcf_default = buffer(ntot);
-    dcp.veg_contact_fraction = vcf_default;
-  }
   ssb200_sw_spectral_properties dsw;
   ssb200_lw_spectral_properties dlw;
   memset(&dsw, 0, sizeof(dsw));
   memset(&dlw, 0, sizeof(dlw));
-  if (config->do_sw) {  // driver/spartacus_surface_read_input.F90:258-269,335-344
-    const size_t g = (size_t)config->nsw;
-    dsw = *sw;
-    if (!sw->air_ext) dsw.air_ext = filled(g, 1.0e-5);
-    if (!sw->air_ssa) dsw.air_ssa = filled(g, 0.999);
-    if (!sw->wall_specular_frac && sw->wall_albedo) dsw.wall_specular_frac = filled(g, 0.0);
-  }
-  if (config->do_lw) {  // driver/spartacus_surface_read_input.F90:362-365; radsurf_simple_spectrum.F90:41-66
-    const size_t g = (size_t)config->nlw;
-    dlw = *lw;
-    if (!lw->air_ext) dlw.air_ext = filled(g, 1.0e-5);
-    if (!lw->air_ssa) dlw.air_ssa = filled(g, 0.0);
-    const bool need_t = !lw->ground_emission || !lw->roof_emission || !lw->wall_emission || !lw->clear_air_planck ||
-                        !lw->veg_planck || !lw->veg_air_planck;
-    if (need_t && g != 1)
-      return fail(SSB200_ERR_ARG, "Simple longwave spectrum only possible with one input spectral interval");
-    if (!lw->ground_emission && drv->ground_temperature) {
-      dlw.ground_emission = buffer(ncol);
-      emis.push_back(Emis{const_cast<double *>(dlw.ground_emission), dlw.ground_emissivity, drv->ground_temperature,
-                          (long)c0, (long)cN});
-    }
-    auto layer_emis = [&](const double *given, const double *&slot, const double *emissivity, const double *t) {
-      if (given || !t) return;
-      slot = buffer(ntot);
-      emis.push_back(Emis{const_cast<double *>(slot), emissivity, t, (long)l0, (long)lN});
-    };
-    layer_emis(lw->roof_emission, dlw.roof_emission, dlw.roof_emissivity, drv->roof_temperature);
-    layer_emis(lw->wall_emission, dlw.wall_emission, dlw.wall_emissivity, drv->wall_temperature);
-    layer_emis(lw->clear_air_planck, dlw.clear_air_planck, nullptr, drv->clear_air_temperature);
-    layer_emis(lw->veg_planck, dlw.veg_planck, nullptr, drv->veg_temperature);
-    layer_emis(lw->veg_air_planck, dlw.veg_air_planck, nullptr, drv->veg_air_temperature);
-  }
-  if (err_rc) return err_rc;
+  if (config->do_sw) dsw = *sw;
+  if (config->do_lw) dlw = *lw;
+  DriverStage ds;
+  int rc = ds.plan(*config, *drv, ncol, ntot, dcp, dsw, dlw, pool);
+  if (rc) return rc;
   // plan, argument checks, ordering against the previous call, status reset (the summed objects stand in
   // for the normalised ones, whose shape they have)
   ssb::CallArgs ca{config, &dcp, config->do_sw ? &dsw : nullptr, config->do_lw ? &dlw : nullptr, bc,
                    sw_flux, sw_flux, lw_flux, lw_flux};
   int range[2] = {1, 0};
-  int rc = radsurf_device_locked(cx, ca, c1, c2, stream, nullptr, range);
+  rc = radsurf_device_locked(cx, ca, c1, c2, stream, nullptr, range);
   if (rc || range[0] > range[1]) return rc;
   CudaBackend probe(cx);
   ssb::Dispatcher<CudaBackend> route(probe);
@@ -1313,23 +1262,13 @@ static int radsurf_fluxes_device_locked(Context &cx, const ssb200_config *config
   std::vector<std::pair<double *, size_t>> zeroed;
   auto normalised = [&](const ssb200_canopy_flux *sum, ssb200_canopy_flux &d) {
     d = *sum;
-    const size_t g = (size_t)sum->nspec;
-    auto make = [&](double *&m, bool per_layer, size_t w) {
-      if (!m || (per_layer && staged)) return;
-      double *p = buffer((per_layer ? ntot : ncol) * w);
-      if (p) zeroed.push_back({p + (per_layer ? l0 : c0) * w, ((per_layer ? lN - l0 : cN - c0)) * w});
-      m = p;
-    };
-    make(d.ground_dn, false, g); make(d.ground_net, false, g); make(d.ground_vertical_diff, false, g);
-    make(d.top_dn, false, g); make(d.top_net, false, g); make(d.ground_dn_dir, false, g); make(d.top_dn_dir, false, g);
-    make(d.ground_sunlit_frac, false, 1);
-    make(d.roof_in, true, g); make(d.roof_net, true, g); make(d.wall_in, true, g); make(d.wall_net, true, g);
-    make(d.roof_in_dir, true, g); make(d.wall_in_dir, true, g);
-    make(d.roof_sunlit_frac, true, 1); make(d.wall_sunlit_frac, true, 1);
-    make(d.clear_air_abs, true, g); make(d.veg_abs, true, g); make(d.veg_air_abs, true, g); make(d.veg_abs_dir, true, g);
-    make(d.veg_sunlit_frac, true, 1);
-    make(d.flux_dn_layer_top, true, g); make(d.flux_up_layer_top, true, g); make(d.flux_dn_layer_base, true, g);
-    make(d.flux_up_layer_base, true, g); make(d.flux_dn_dir_layer_top, true, g); make(d.flux_dn_dir_layer_base, true, g);
+    for (const ssb::FluxMember &m : ssb::kFluxMembers) {
+      double *&member = d.*m.ptr;
+      if (!member || (m.per_layer && staged)) continue;
+      const size_t w = ssb::member_width(m, (size_t)sum->nspec);
+      member = pool.get<double>((m.per_layer ? ntot : ncol) * w);
+      if (member) zeroed.push_back({member + (m.per_layer ? l0 : c0) * w, (m.per_layer ? lN - l0 : cN - c0) * w});
+    }
   };
   ssb200_canopy_flux d1, d2, d3, d4;
   PassSum sum_sw, sum_lw;
@@ -1347,35 +1286,14 @@ static int radsurf_fluxes_device_locked(Context &cx, const ssb200_config *config
     sum_lw.fb = drv->top_flux_dn_lw;
     if (staged) sum_lw.out = lw_flux;
   }
-  if (err_rc) return err_rc;
+  if (pool.rc) return pool.rc;
   const ssb::CallArgs nca{config, &dcp, ca.sw, ca.lw, bc, config->do_sw ? &d1 : nullptr, config->do_sw ? &d2 : nullptr,
                           config->do_lw ? &d3 : nullptr, config->do_lw ? &d4 : nullptr};
-  // an error return after the first launch must not leave work queued on the context's buffers
-  struct Drain {
-    cudaStream_t s;
-    bool armed = true;
-    ~Drain() {
-      if (armed) cudaStreamSynchronize(s);
-    }
-  } drain{stream};
+  Drain drain{stream};
   CudaBackend be(cx);  // (profiling: the stages around the solve are booked with family 4)
   be.tick(4, true);
-  for (const Fill &f : fills)
-    if (f.i1 > f.i0) {
-      k_fill<<<(unsigned)((f.i1 - f.i0 + 255) / 256), 256, 0, stream>>>(f.p, f.v, f.i0, f.i1);
-      ++g_launches;
-    }
-  if (vcf_default && lN > l0) {
-    k_vcf_default<<<(unsigned)((lN - l0 + 255) / 256), 256, 0, stream>>>(
-        vcf_default, cp->veg_fraction, cp->building_fraction, config->min_vegetation_fraction, (long)l0, (long)lN);
-    ++g_launches;
-  }
-  for (const Emis &e : emis)
-    if (e.i1 > e.i0) {
-      k_sigma_t4<<<(unsigned)((e.i1 - e.i0 + 255) / 256), 256, 0, stream>>>(e.out, e.emissivity, e.temperature, 1,
-                                                                              e.i0, e.i1);
-      ++g_launches;
-    }
+  ds.fill(l0, lN, stream);
+  ds.derive(dcp, config->min_vegetation_fraction, c0, cN, l0, lN, stream);
   for (const auto &z : zeroed)
     if (z.second > 0) SSB_CUDA(cudaMemsetAsync(z.first, 0, z.second * sizeof(double), stream));
   SSB_CUDA(cudaGetLastError());
@@ -1387,18 +1305,8 @@ static int radsurf_fluxes_device_locked(Context &cx, const ssb200_config *config
   const long cnt = (long)std::max(cN - c0, staged ? (size_t)0 : lN - l0);
   auto scale_sum = [&](ssb200_canopy_flux *o, const ssb200_canopy_flux &x, const ssb200_canopy_flux &y,
                        const double *fa, const double *fb, const double *fbm, int nspec) {
-    FieldList all, fl;
-    collect_fields(o, &x, &y, all, true);
-    fl.n = 0;
-    for (int f = 0; f < all.n; ++f)
-      if (!staged || !all.per_layer[f]) {
-        fl.p[fl.n] = all.p[f];
-        fl.a[fl.n] = all.a[f];
-        fl.b[fl.n] = all.b[f];
-        fl.per_layer[fl.n] = all.per_layer[f];
-        fl.spectral[fl.n] = all.spectral[f];
-        ++fl.n;
-      }
+    FieldList fl;
+    collect_fields(o, &x, &y, fl, true, !staged);
     const long nthr = cnt * nspec;
     if (fl.n == 0 || nthr <= 0) return;
     k_scale_sum<<<(unsigned)((nthr + 255) / 256), 256, 0, stream>>>(fl, fa, fb, fbm, (const int *)cx.d_lay2col.p,
@@ -1448,133 +1356,46 @@ static int radsurf_host(const ssb200_config *config, const ssb200_canopy_propert
   if (c2 > cp->ncol) c2 = cp->ncol;
   if (c1 > c2) return 0;
   const size_t ncol = (size_t)cp->ncol, ntot = (size_t)cp->ntotlay;
-  // packed layer range touched by the columns of this call; check that it is
-  // contiguous so that per-layer outputs need no upload
-  size_t l1 = ntot, l2 = 0;
-  bool contiguous = true;
-  size_t expect = 0;
-  bool first = true;
-  for (int j = c1 - 1; j < c2; ++j) {
-    if (cp->i_representation[j] == SSB200_TILE_FLAT || cp->nlay[j] <= 0) continue;
-    const size_t s = (size_t)cp->istartlay[j] - 1, e = s + (size_t)cp->nlay[j];
-    if (cp->istartlay[j] < 1 || e > ntot) return fail(SSB200_ERR_SHAPE, "layer range outside 1..ntotlay");
-    if (!first && s != expect) contiguous = false;
-    first = false;
-    expect = e;
-    if (s < l1) l1 = s;
-    if (e > l2) l2 = e;
-  }
-  if (l2 < l1) l1 = l2 = 0;
-  const size_t cO = (size_t)(c1 - 1), cN = (size_t)(c2 - c1 + 1), lN = l2 - l1;
+  // packed layer range touched by the columns of this call: per-layer outputs need no upload when it is
+  // contiguous
+  const LayerSpan span = layer_span(*cp, (size_t)c1 - 1, (size_t)c2);
+  if (!span.ok) return fail(SSB200_ERR_SHAPE, "layer range outside 1..ntotlay");
+  const bool contiguous = span.contiguous;
+  const size_t l1 = span.l0, l2 = span.l1, cN = (size_t)(c2 - c1 + 1), lN = l2 - l1;
   if (drv && !contiguous)
     return fail(SSB200_ERR_UNSUPPORTED, "radsurf_fluxes needs the packed layers of the selected columns to be contiguous");
-  Stager sg(cx, st, sp);
-  ssb200_canopy_properties dcp = *cp;
-  auto lay1 = [&](const double *h) { return (const double *)sg.mirror(h, ntot, 1, true, true, false); };
-  dcp.cos_sza = sg.mirror(cp->cos_sza, ncol, 1, false, true, false);
-  dcp.dz = lay1(cp->dz);
-  dcp.building_fraction = lay1(cp->building_fraction);
-  dcp.building_scale = lay1(cp->building_scale);
-  dcp.veg_fraction = lay1(cp->veg_fraction);
-  dcp.veg_scale = lay1(cp->veg_scale);
-  dcp.veg_ext = lay1(cp->veg_ext);
-  dcp.veg_fsd = lay1(cp->veg_fsd);
-  dcp.veg_contact_fraction = lay1(cp->veg_contact_fraction);
-  // read_input's defaults for members the caller leaves NULL (ssb200_radsurf_fluxes only)
-  struct Fill {
-    double *p;
-    double v;
-    size_t n;
+  Stager sg(cx, sp);
+  // inputs: mirrors uploaded per window
+  auto inputs = [&](auto &d, const auto &h, const auto &table, size_t nspec) {
+    d = h;
+    for (const auto &m : table)
+      d.*m.ptr = sg.mirror(h.*m.ptr, m.per_layer ? ntot : ncol, ssb::member_width(m, nspec), m.per_layer, true, false);
   };
-  struct Emis {  // out = sigma [emissivity] T^4 on the device, per window
-    double *out;
-    const double *emissivity, *temperature;
-    bool per_layer;
-  };
-  std::vector<Emis> emis;
-  std::vector<Fill> fills;
-  auto filled = [&](size_t width, double v) -> const double * {
-    double *p = sg.device_only(ntot * width);
-    fills.push_back(Fill{p, v, ntot * width});
-    return p;
-  };
-  double *d_vcf_default = nullptr;
-  if (drv && !cp->veg_contact_fraction && cp->veg_fraction && cp->building_fraction) {
-    d_vcf_default = sg.device_only(ntot);
-    dcp.veg_contact_fraction = d_vcf_default;
-  }
+  ssb200_canopy_properties dcp;
   ssb200_sw_spectral_properties dsw;
   ssb200_lw_spectral_properties dlw;
   memset(&dsw, 0, sizeof(dsw));
   memset(&dlw, 0, sizeof(dlw));
-  if (config->do_sw) {
-    const size_t g = (size_t)config->nsw;
-    auto L = [&](const double *h) { return (const double *)sg.mirror(h, ntot, g, true, true, false); };
-    auto Cc = [&](const double *h) { return (const double *)sg.mirror(h, ncol, g, false, true, false); };
-    dsw.nspec = sw->nspec;
-    dsw.air_ext = L(sw->air_ext);
-    dsw.air_ssa = L(sw->air_ssa);
-    dsw.veg_ssa = L(sw->veg_ssa);
-    dsw.ground_albedo = Cc(sw->ground_albedo);
-    dsw.roof_albedo = L(sw->roof_albedo);
-    dsw.wall_albedo = L(sw->wall_albedo);
-    dsw.wall_specular_frac = L(sw->wall_specular_frac);
-    dsw.ground_albedo_dir = Cc(sw->ground_albedo_dir);
-    dsw.roof_albedo_dir = L(sw->roof_albedo_dir);
-    if (drv) {  // driver/spartacus_surface_read_input.F90:258-269,335-344 (roof_albedo_dir NULL: the kernels use roof_albedo)
-      if (!sw->air_ext) dsw.air_ext = filled(g, 1.0e-5);
-      if (!sw->air_ssa) dsw.air_ssa = filled(g, 0.999);
-      if (!sw->wall_specular_frac && sw->wall_albedo) dsw.wall_specular_frac = filled(g, 0.0);
-    }
-  }
-  if (config->do_lw) {
-    const size_t g = (size_t)config->nlw;
-    auto L = [&](const double *h) { return (const double *)sg.mirror(h, ntot, g, true, true, false); };
-    auto Cc = [&](const double *h) { return (const double *)sg.mirror(h, ncol, g, false, true, false); };
-    dlw.nspec = lw->nspec;
-    dlw.air_ext = L(lw->air_ext);
-    dlw.air_ssa = L(lw->air_ssa);
-    dlw.clear_air_planck = L(lw->clear_air_planck);
-    dlw.veg_ssa = L(lw->veg_ssa);
-    dlw.veg_planck = L(lw->veg_planck);
-    dlw.veg_air_planck = L(lw->veg_air_planck);
-    dlw.ground_emissivity = Cc(lw->ground_emissivity);
-    dlw.ground_emission = Cc(lw->ground_emission);
-    dlw.roof_emissivity = L(lw->roof_emissivity);
-    dlw.wall_emissivity = L(lw->wall_emissivity);
-    dlw.roof_emission = L(lw->roof_emission);
-    dlw.wall_emission = L(lw->wall_emission);
-    if (drv) {  // driver/spartacus_surface_read_input.F90:362-365; radsurf_simple_spectrum.F90:41-66
-      if (!lw->air_ext) dlw.air_ext = filled(g, 1.0e-5);
-      if (!lw->air_ssa) dlw.air_ssa = filled(g, 0.0);
-      // (the same host array given for several temperatures - the driver passes one air temperature
-      // for clear air, vegetation and the air in vegetation - is uploaded once)
-      std::vector<std::pair<const double *, const double *>> t_seen;
-      auto T1 = [&](const double *h, size_t rows, bool per_layer) {
-        for (const auto &s : t_seen)
-          if (s.first == h) return s.second;
-        const double *d = (const double *)sg.mirror(h, rows, 1, per_layer, true, false);
-        t_seen.push_back({h, d});
-        return d;
-      };
-      const bool need_t = !lw->ground_emission || !lw->roof_emission || !lw->wall_emission ||
-                          !lw->clear_air_planck || !lw->veg_planck || !lw->veg_air_planck;
-      if (need_t && g != 1)
-        return fail(SSB200_ERR_ARG, "Simple longwave spectrum only possible with one input spectral interval");
-      if (!lw->ground_emission && drv->ground_temperature) {
-        emis.push_back(Emis{sg.device_only(ncol), dlw.ground_emissivity, T1(drv->ground_temperature, ncol, false), false});
-        dlw.ground_emission = emis.back().out;
+  inputs(dcp, *cp, ssb::kCanopyMembers, 1);
+  if (config->do_sw) inputs(dsw, *sw, ssb::kSwMembers, (size_t)config->nsw);
+  if (config->do_lw) inputs(dlw, *lw, ssb::kLwMembers, (size_t)config->nlw);
+  // read_input's defaults and the emission for members the caller leaves NULL (ssb200_radsurf_fluxes only)
+  DriverStage ds;
+  if (drv) {
+    if (sg.pool.rc) return sg.pool.rc;
+    if ((rc = ds.plan(*config, *drv, ncol, ntot, dcp, dsw, dlw, sg.pool))) return rc;
+    // (the same host array given for several temperatures - the driver passes one air temperature
+    // for clear air, vegetation and the air in vegetation - is uploaded once)
+    std::vector<std::pair<const double *, const double *>> t_seen;
+    for (DriverStage::Emis &e : ds.emis) {
+      const double *h = e.temperature;
+      e.temperature = nullptr;
+      for (const auto &s : t_seen)
+        if (s.first == h) e.temperature = s.second;
+      if (!e.temperature) {
+        e.temperature = sg.mirror(h, e.per_layer ? ntot : ncol, 1, e.per_layer, true, false);
+        t_seen.push_back({h, e.temperature});
       }
-      auto layer_emis = [&](const double *host_out, const double *&slot, const double *emissivity, const double *t) {
-        if (host_out || !t) return;
-        emis.push_back(Emis{sg.device_only(ntot), emissivity, T1(t, ntot, true), true});
-        slot = emis.back().out;
-      };
-      layer_emis(lw->roof_emission, dlw.roof_emission, dlw.roof_emissivity, drv->roof_temperature);
-      layer_emis(lw->wall_emission, dlw.wall_emission, dlw.wall_emissivity, drv->wall_temperature);
-      layer_emis(lw->clear_air_planck, dlw.clear_air_planck, nullptr, drv->clear_air_temperature);
-      layer_emis(lw->veg_planck, dlw.veg_planck, nullptr, drv->veg_temperature);
-      layer_emis(lw->veg_air_planck, dlw.veg_air_planck, nullptr, drv->veg_air_temperature);
     }
   }
   // outputs: per-column members are uploaded first (Flat tiles and night-time
@@ -1582,78 +1403,27 @@ static int radsurf_host(const ssb200_config *config, const ssb200_canopy_propert
   // rewritten by the kernels when the layer range is contiguous
   ssb200_boundary_conds_out dbc;
   memset(&dbc, 0, sizeof(dbc));
-  {
-    const size_t gs = (size_t)config->nsw, gl = (size_t)config->nlw;
-    if (config->do_sw) {
-      dbc.sw_albedo = sg.mirror(bc->sw_albedo, ncol, gs, false, true, true);
-      dbc.sw_albedo_dir = sg.mirror(bc->sw_albedo_dir, ncol, gs, false, true, true);
-    }
-    if (config->do_lw) {
-      dbc.lw_emissivity = sg.mirror(bc->lw_emissivity, ncol, gl, false, true, true);
-      dbc.lw_emission = sg.mirror(bc->lw_emission, ncol, gl, false, true, true);
-    }
-  }
+  for (const ssb::BcMember &m : ssb::kBcMembers)
+    if (m.lw ? config->do_lw : config->do_sw)
+      dbc.*m.ptr = sg.mirror(bc->*m.ptr, ncol, (size_t)(m.lw ? config->nlw : config->nsw), false, true, true);
   auto stage_flux = [&](const ssb200_canopy_flux *h, ssb200_canopy_flux &d) {
     d = *h;
-    const size_t g = (size_t)h->nspec;
-    auto Cc = [&](double *p) { return sg.mirror(p, ncol, g, false, true, true); };
-    auto L = [&](double *p) { return sg.mirror(p, ntot, g, true, !contiguous, true); };
-    auto C1 = [&](double *p) { return sg.mirror(p, ncol, 1, false, true, true); };
-    auto L1 = [&](double *p) { return sg.mirror(p, ntot, 1, true, !contiguous, true); };
-    d.ground_dn = Cc(h->ground_dn);
-    d.ground_net = Cc(h->ground_net);
-    d.ground_vertical_diff = Cc(h->ground_vertical_diff);
-    d.top_dn = Cc(h->top_dn);
-    d.top_net = Cc(h->top_net);
-    d.ground_dn_dir = Cc(h->ground_dn_dir);
-    d.top_dn_dir = Cc(h->top_dn_dir);
-    d.ground_sunlit_frac = C1(h->ground_sunlit_frac);
-    d.roof_in = L(h->roof_in);
-    d.roof_net = L(h->roof_net);
-    d.wall_in = L(h->wall_in);
-    d.wall_net = L(h->wall_net);
-    d.roof_in_dir = L(h->roof_in_dir);
-    d.wall_in_dir = L(h->wall_in_dir);
-    d.roof_sunlit_frac = L1(h->roof_sunlit_frac);
-    d.wall_sunlit_frac = L1(h->wall_sunlit_frac);
-    d.clear_air_abs = L(h->clear_air_abs);
-    d.veg_abs = L(h->veg_abs);
-    d.veg_air_abs = L(h->veg_air_abs);
-    d.veg_abs_dir = L(h->veg_abs_dir);
-    d.veg_sunlit_frac = L1(h->veg_sunlit_frac);
-    d.flux_dn_layer_top = L(h->flux_dn_layer_top);
-    d.flux_up_layer_top = L(h->flux_up_layer_top);
-    d.flux_dn_layer_base = L(h->flux_dn_layer_base);
-    d.flux_up_layer_base = L(h->flux_up_layer_base);
-    d.flux_dn_dir_layer_top = L(h->flux_dn_dir_layer_top);
-    d.flux_dn_dir_layer_base = L(h->flux_dn_dir_layer_base);
+    for (const ssb::FluxMember &m : ssb::kFluxMembers)
+      d.*m.ptr = sg.mirror(h->*m.ptr, m.per_layer ? ntot : ncol, ssb::member_width(m, (size_t)h->nspec), m.per_layer,
+                           !m.per_layer || !contiguous, true);
   };
-  // a normalised flux object that lives on the device only, with the members of `tmpl`
+  // a normalised flux object that lives on the device only, with the members of `tmpl`; members the
+  // kernels may leave untouched start from zero (canopy_flux_type%zero_all, driver:184)
   std::vector<std::pair<double *, size_t>> zeroed;
   auto device_flux = [&](const ssb200_canopy_flux *tmpl, ssb200_canopy_flux &d) {
     d = *tmpl;
-    const size_t g = (size_t)tmpl->nspec;
-    auto make = [&](double *present, size_t total, bool always_zero) -> double * {
-      if (!present) return nullptr;
-      double *p = sg.device_only(total);
-      // members the kernels may leave untouched start from zero (canopy_flux_type%zero_all, driver:184)
-      if (always_zero || !contiguous) zeroed.push_back({p, total});
-      return p;
-    };
-#define SSB_DC(m) d.m = make(tmpl->m, ncol * g, true)
-#define SSB_DL(m) d.m = make(tmpl->m, ntot * g, false)
-    SSB_DC(ground_dn); SSB_DC(ground_net); SSB_DC(ground_vertical_diff); SSB_DC(top_dn); SSB_DC(top_net);
-    SSB_DC(ground_dn_dir); SSB_DC(top_dn_dir);
-    d.ground_sunlit_frac = make(tmpl->ground_sunlit_frac, ncol, true);
-    SSB_DL(roof_in); SSB_DL(roof_net); SSB_DL(wall_in); SSB_DL(wall_net); SSB_DL(roof_in_dir); SSB_DL(wall_in_dir);
-    d.roof_sunlit_frac = make(tmpl->roof_sunlit_frac, ntot, false);
-    d.wall_sunlit_frac = make(tmpl->wall_sunlit_frac, ntot, false);
-    SSB_DL(clear_air_abs); SSB_DL(veg_abs); SSB_DL(veg_air_abs); SSB_DL(veg_abs_dir);
-    d.veg_sunlit_frac = make(tmpl->veg_sunlit_frac, ntot, false);
-    SSB_DL(flux_dn_layer_top); SSB_DL(flux_up_layer_top); SSB_DL(flux_dn_layer_base); SSB_DL(flux_up_layer_base);
-    SSB_DL(flux_dn_dir_layer_top); SSB_DL(flux_dn_dir_layer_base);
-#undef SSB_DC
-#undef SSB_DL
+    for (const ssb::FluxMember &m : ssb::kFluxMembers) {
+      double *&member = d.*m.ptr;
+      if (!member) continue;
+      const size_t total = (m.per_layer ? ntot : ncol) * ssb::member_width(m, (size_t)tmpl->nspec);
+      member = sg.pool.get<double>(total);
+      if (!m.per_layer || !contiguous) zeroed.push_back({member, total});
+    }
   };
   ssb200_canopy_flux d1, d2, d3, d4, dsum_sw, dsum_lw;
   const double *d_top_sw = nullptr, *d_top_dir = nullptr, *d_top_lw = nullptr;
@@ -1681,12 +1451,8 @@ static int radsurf_host(const ssb200_config *config, const ssb200_canopy_propert
       stage_flux(lw_norm, d4);
     }
   }
-  if (sg.rc) return sg.rc;
-  for (const Fill &f : fills)
-    if (f.n > 0) {
-      k_fill<<<(unsigned)((f.n + 255) / 256), 256, 0, st>>>(f.p, f.v, 0, (long)f.n);
-      ++g_launches;
-    }
+  if (sg.pool.rc) return sg.pool.rc;
+  ds.fill(l1, l2, st);
   for (const auto &z : zeroed) SSB_CUDA(cudaMemsetAsync(z.first, 0, z.second * sizeof(double), st));
   ssb::CallArgs ca{config, &dcp, config->do_sw ? &dsw : nullptr, config->do_lw ? &dlw : nullptr, &dbc,
                    config->do_sw ? &d1 : nullptr, config->do_sw ? &d2 : nullptr,
@@ -1747,19 +1513,8 @@ static int radsurf_host(const ssb200_config *config, const ssb200_canopy_propert
       SSB_CUDA(cudaEventRecord(cx.blk_events[2 * b], s_up));
       SSB_CUDA(cudaStreamWaitEvent(s_run, cx.blk_events[2 * b], 0));
     }
-    if (drv) {  // input stage of the window: default contact fraction, emission from temperatures
-      if (d_vcf_default && lb1 > lb0) {
-        k_vcf_default<<<(unsigned)((lb1 - lb0 + 255) / 256), 256, 0, s_run>>>(
-            d_vcf_default, dcp.veg_fraction, dcp.building_fraction, config->min_vegetation_fraction, (long)lb0, (long)lb1);
-        ++g_launches;
-      }
-      for (const Emis &e : emis) {
-        const long i0 = e.per_layer ? (long)lb0 : (long)cb0, i1 = e.per_layer ? (long)lb1 : (long)cb1;
-        if (i1 <= i0) continue;
-        k_sigma_t4<<<(unsigned)((i1 - i0 + 255) / 256), 256, 0, s_run>>>(e.out, e.emissivity, e.temperature, 1, i0, i1);
-        ++g_launches;
-      }
-    }
+    // input stage of the window: default contact fraction, emission from temperatures
+    ds.derive(dcp, config->min_vegetation_fraction, (size_t)cb0, (size_t)cb1, lb0, lb1, s_run);
     rc = run_window(cx, ca, 1, cx.budget_doubles, cb0, cb1);
     if (rc) return rc;
     if (drv) {  // scale + sum of the window (driver:250-261), still on the kernel lane

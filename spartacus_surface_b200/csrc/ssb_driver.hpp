@@ -10,6 +10,7 @@
 // exercised by CPU tests.
 #pragma once
 #include <algorithm>
+#include <cstddef>
 #include <cstdio>
 #include <cstring>
 #include <string>
@@ -19,6 +20,110 @@
 #include "ssb_stage.cuh"
 
 namespace ssb {
+
+// The array members of the ABI structs (include/spartacus_b200.h), in declaration order.  Every entry
+// marshals its arrays by looping over these tables, so a member is described once: its extent (per
+// column, (nspec, ncol), or per packed layer, (nspec, ntotlay)) and whether it is spectral (nspec values
+// per column or layer) or not (one).  Members of ssb200_boundary_conds_out belong to the shortwave
+// (width nsw) or the longwave band (width nlw).
+template <class S, class P>
+struct Member {
+  P S::*ptr;
+  bool per_layer;
+  bool spectral;
+  bool lw;  // ssb200_boundary_conds_out: longwave member
+};
+typedef Member<ssb200_canopy_properties, const double *> CanopyMember;
+typedef Member<ssb200_sw_spectral_properties, const double *> SwMember;
+typedef Member<ssb200_lw_spectral_properties, const double *> LwMember;
+typedef Member<ssb200_boundary_conds_out, double *> BcMember;
+typedef Member<ssb200_canopy_flux, double *> FluxMember;
+
+constexpr bool kCol = false, kLay = true, kSpec = true, kOne = false;
+
+inline constexpr CanopyMember kCanopyMembers[] = {
+    {&ssb200_canopy_properties::cos_sza, kCol, kOne},
+    {&ssb200_canopy_properties::dz, kLay, kOne},
+    {&ssb200_canopy_properties::building_fraction, kLay, kOne},
+    {&ssb200_canopy_properties::building_scale, kLay, kOne},
+    {&ssb200_canopy_properties::veg_fraction, kLay, kOne},
+    {&ssb200_canopy_properties::veg_scale, kLay, kOne},
+    {&ssb200_canopy_properties::veg_ext, kLay, kOne},
+    {&ssb200_canopy_properties::veg_fsd, kLay, kOne},
+    {&ssb200_canopy_properties::veg_contact_fraction, kLay, kOne}};
+inline constexpr SwMember kSwMembers[] = {
+    {&ssb200_sw_spectral_properties::air_ext, kLay, kSpec},
+    {&ssb200_sw_spectral_properties::air_ssa, kLay, kSpec},
+    {&ssb200_sw_spectral_properties::veg_ssa, kLay, kSpec},
+    {&ssb200_sw_spectral_properties::ground_albedo, kCol, kSpec},
+    {&ssb200_sw_spectral_properties::roof_albedo, kLay, kSpec},
+    {&ssb200_sw_spectral_properties::wall_albedo, kLay, kSpec},
+    {&ssb200_sw_spectral_properties::wall_specular_frac, kLay, kSpec},
+    {&ssb200_sw_spectral_properties::ground_albedo_dir, kCol, kSpec},
+    {&ssb200_sw_spectral_properties::roof_albedo_dir, kLay, kSpec}};
+inline constexpr LwMember kLwMembers[] = {
+    {&ssb200_lw_spectral_properties::air_ext, kLay, kSpec},
+    {&ssb200_lw_spectral_properties::air_ssa, kLay, kSpec},
+    {&ssb200_lw_spectral_properties::clear_air_planck, kLay, kSpec},
+    {&ssb200_lw_spectral_properties::veg_ssa, kLay, kSpec},
+    {&ssb200_lw_spectral_properties::veg_planck, kLay, kSpec},
+    {&ssb200_lw_spectral_properties::veg_air_planck, kLay, kSpec},
+    {&ssb200_lw_spectral_properties::ground_emissivity, kCol, kSpec},
+    {&ssb200_lw_spectral_properties::ground_emission, kCol, kSpec},
+    {&ssb200_lw_spectral_properties::roof_emissivity, kLay, kSpec},
+    {&ssb200_lw_spectral_properties::wall_emissivity, kLay, kSpec},
+    {&ssb200_lw_spectral_properties::roof_emission, kLay, kSpec},
+    {&ssb200_lw_spectral_properties::wall_emission, kLay, kSpec}};
+inline constexpr BcMember kBcMembers[] = {
+    {&ssb200_boundary_conds_out::sw_albedo, kCol, kSpec, false},
+    {&ssb200_boundary_conds_out::sw_albedo_dir, kCol, kSpec, false},
+    {&ssb200_boundary_conds_out::lw_emissivity, kCol, kSpec, true},
+    {&ssb200_boundary_conds_out::lw_emission, kCol, kSpec, true}};
+inline constexpr FluxMember kFluxMembers[] = {
+    {&ssb200_canopy_flux::ground_dn, kCol, kSpec},
+    {&ssb200_canopy_flux::ground_net, kCol, kSpec},
+    {&ssb200_canopy_flux::ground_vertical_diff, kCol, kSpec},
+    {&ssb200_canopy_flux::top_dn, kCol, kSpec},
+    {&ssb200_canopy_flux::top_net, kCol, kSpec},
+    {&ssb200_canopy_flux::ground_dn_dir, kCol, kSpec},
+    {&ssb200_canopy_flux::top_dn_dir, kCol, kSpec},
+    {&ssb200_canopy_flux::ground_sunlit_frac, kCol, kOne},
+    {&ssb200_canopy_flux::roof_in, kLay, kSpec},
+    {&ssb200_canopy_flux::roof_net, kLay, kSpec},
+    {&ssb200_canopy_flux::wall_in, kLay, kSpec},
+    {&ssb200_canopy_flux::wall_net, kLay, kSpec},
+    {&ssb200_canopy_flux::roof_in_dir, kLay, kSpec},
+    {&ssb200_canopy_flux::wall_in_dir, kLay, kSpec},
+    {&ssb200_canopy_flux::roof_sunlit_frac, kLay, kOne},
+    {&ssb200_canopy_flux::wall_sunlit_frac, kLay, kOne},
+    {&ssb200_canopy_flux::clear_air_abs, kLay, kSpec},
+    {&ssb200_canopy_flux::veg_abs, kLay, kSpec},
+    {&ssb200_canopy_flux::veg_air_abs, kLay, kSpec},
+    {&ssb200_canopy_flux::veg_abs_dir, kLay, kSpec},
+    {&ssb200_canopy_flux::veg_sunlit_frac, kLay, kOne},
+    {&ssb200_canopy_flux::flux_dn_layer_top, kLay, kSpec},
+    {&ssb200_canopy_flux::flux_up_layer_top, kLay, kSpec},
+    {&ssb200_canopy_flux::flux_dn_layer_base, kLay, kSpec},
+    {&ssb200_canopy_flux::flux_up_layer_base, kLay, kSpec},
+    {&ssb200_canopy_flux::flux_dn_dir_layer_top, kLay, kSpec},
+    {&ssb200_canopy_flux::flux_dn_dir_layer_base, kLay, kSpec}};
+
+// The array members follow the integer header members and fill the rest of the struct: a member added to
+// the header without a row above fails here.
+#define SSB_TABLE_COVERS(S, first, table) \
+  static_assert(offsetof(S, first) + sizeof(table) / sizeof(table[0]) * sizeof(double *) == sizeof(S), #table)
+SSB_TABLE_COVERS(ssb200_canopy_properties, cos_sza, kCanopyMembers);
+SSB_TABLE_COVERS(ssb200_sw_spectral_properties, air_ext, kSwMembers);
+SSB_TABLE_COVERS(ssb200_lw_spectral_properties, air_ext, kLwMembers);
+SSB_TABLE_COVERS(ssb200_boundary_conds_out, sw_albedo, kBcMembers);
+SSB_TABLE_COVERS(ssb200_canopy_flux, ground_dn, kFluxMembers);
+#undef SSB_TABLE_COVERS
+
+// values per column or packed layer of a member of a struct with `nspec` spectral intervals
+template <class M>
+inline size_t member_width(const M &m, size_t nspec) {
+  return m.spectral ? nspec : 1;
+}
 
 // Lists the per-layer arrays of a pass and redirects the members of `b` to their level-major staging
 // buffers (ssb_stage.cuh), carved from `cursor` (NULL: only count).  Returns doubles per (level, column).
@@ -47,70 +152,36 @@ inline size_t stage_plan(ClassArgs &b, bool lw, size_t per_elem, double *cursor,
     cursor += (size_t)ns * per_elem;
     return staged;
   };
-  auto cin = [&](const double *&member, int ns) { add(in, const_cast<double *&>(member), ns); };
+  // per-layer inputs of the canopy and of the pass's spectral properties
+  auto inputs = [&](auto &obj, const auto &table) {
+    for (const auto &m : table)
+      if (m.per_layer) add(in, const_cast<double *&>(obj.*m.ptr), (int)member_width(m, b.cfg.nspec));
+  };
   if (in) in->n = 0;
   if (out) out->n = 0;
-  const int ns = b.cfg.nspec;
-  cin(b.cp.dz, 1);
-  cin(b.cp.building_fraction, 1);
-  cin(b.cp.building_scale, 1);
-  cin(b.cp.veg_fraction, 1);
-  cin(b.cp.veg_scale, 1);
-  cin(b.cp.veg_ext, 1);
-  cin(b.cp.veg_fsd, 1);
-  cin(b.cp.veg_contact_fraction, 1);
-  if (lw) {
-    cin(b.lw.air_ext, ns);
-    cin(b.lw.air_ssa, ns);
-    cin(b.lw.clear_air_planck, ns);
-    cin(b.lw.veg_ssa, ns);
-    cin(b.lw.veg_planck, ns);
-    cin(b.lw.veg_air_planck, ns);
-    cin(b.lw.roof_emissivity, ns);
-    cin(b.lw.wall_emissivity, ns);
-    cin(b.lw.roof_emission, ns);
-    cin(b.lw.wall_emission, ns);
-  } else {
-    cin(b.sw.air_ext, ns);
-    cin(b.sw.air_ssa, ns);
-    cin(b.sw.veg_ssa, ns);
-    cin(b.sw.roof_albedo, ns);
-    cin(b.sw.wall_albedo, ns);
-    cin(b.sw.wall_specular_frac, ns);
-    cin(b.sw.roof_albedo_dir, ns);
-  }
-  typedef double *ssb200_canopy_flux::*Member;
-  static const Member spectral[] = {
-      &ssb200_canopy_flux::roof_in,           &ssb200_canopy_flux::roof_net,
-      &ssb200_canopy_flux::wall_in,           &ssb200_canopy_flux::wall_net,
-      &ssb200_canopy_flux::roof_in_dir,       &ssb200_canopy_flux::wall_in_dir,
-      &ssb200_canopy_flux::clear_air_abs,     &ssb200_canopy_flux::veg_abs,
-      &ssb200_canopy_flux::veg_air_abs,       &ssb200_canopy_flux::veg_abs_dir,
-      &ssb200_canopy_flux::flux_dn_layer_top, &ssb200_canopy_flux::flux_up_layer_top,
-      &ssb200_canopy_flux::flux_dn_layer_base, &ssb200_canopy_flux::flux_up_layer_base,
-      &ssb200_canopy_flux::flux_dn_dir_layer_top, &ssb200_canopy_flux::flux_dn_dir_layer_base};
-  static const Member sunlit[] = {&ssb200_canopy_flux::roof_sunlit_frac, &ssb200_canopy_flux::wall_sunlit_frac,
-                                  &ssb200_canopy_flux::veg_sunlit_frac};
-  if (!sum) {
-    for (ssb200_canopy_flux *f : {&b.f1, &b.f2}) {
-      for (Member m : spectral) add(out, f->*m, ns);
-      for (Member m : sunlit) add(out, f->*m, 1);
+  inputs(b.cp, kCanopyMembers);
+  if (lw)
+    inputs(b.lw, kLwMembers);
+  else
+    inputs(b.sw, kSwMembers);
+  for (const FluxMember &m : kFluxMembers) {
+    if (!m.per_layer) continue;
+    const int w = (int)member_width(m, b.cfg.nspec);
+    if (!sum) {
+      add(out, b.f1.*m.ptr, w);
+      add(out, b.f2.*m.ptr, w);
+      continue;
     }
-    return elems;
-  }
-  auto pair = [&](Member m, int w, unsigned char mode) {
-    double *sa = add(nullptr, b.f1.*m, w), *sb = add(nullptr, b.f2.*m, w);
-    if (!out || !sa || !sb || !(sum->*m)) return;
-    out->ref[out->n] = sum->*m;
+    double *sa = add(nullptr, b.f1.*m.ptr, w), *sb = add(nullptr, b.f2.*m.ptr, w);
+    if (!out || !sa || !sb || !(sum->*m.ptr)) continue;
+    out->ref[out->n] = sum->*m.ptr;
     out->staged[out->n] = sa;
     out->staged2[out->n] = sb;
     out->nspec[out->n] = w;
     out->f32[out->n] = 0;
-    out->sum[out->n] = mode;
+    out->sum[out->n] = m.spectral ? kSumScaled : kSumPlain;
     ++out->n;
-  };
-  for (Member m : spectral) pair(m, ns, kSumScaled);
-  for (Member m : sunlit) pair(m, 1, kSumPlain);
+  }
   return elems;
 }
 
