@@ -492,6 +492,13 @@ struct CudaBackend {
     }
     launch(ssb::launch_layer_lw<NS>, a, nt, 2);
   }
+  // The planner sizes the interface scratch of a staged chunk by the register-resident state alone
+  // (run_class); the generic sweeps need their larger one and must never run on a smaller area.
+  static bool generic_sweep_scratch(const ssb::ClassArgs &a, bool lw) {
+    const ssb::SolveCfg &c = a.cfg;
+    const int n = c.nreg * c.ns, d = c.nreg, nrb = c.urban ? c.nreg + 1 : c.nreg, m = nrb * c.ns;
+    return a.ne_sweep >= (lw ? ssb::lw_sweep_elems(n, m, c.nreg, nrb) : ssb::sw_sweep_elems(n, d, m, nrb, c.nreg, nrb));
+  }
   template <int NS>
   void sweeps_sw(const ssb::ClassArgs &a, long nt) {
     // the register-resident sweeps read what the partition pass of the layer kernels prepared
@@ -502,7 +509,7 @@ struct CudaBackend {
       tick(1, false);
       if (done) return;
     }
-    if (a.lstride) {
+    if (a.lstride || !generic_sweep_scratch(a, false)) {
       if (cx.first_error == cudaSuccess) cx.first_error = cudaErrorNotSupported;
       return;
     }
@@ -517,7 +524,7 @@ struct CudaBackend {
       tick(3, false);
       if (done) return;
     }
-    if (a.lstride) {
+    if (a.lstride || !generic_sweep_scratch(a, true)) {
       if (cx.first_error == cudaSuccess) cx.first_error = cudaErrorNotSupported;
       return;
     }

@@ -395,7 +395,6 @@ struct Dispatcher {
     const SolveCfg &c = a.cfg;
     const int n = c.nreg * c.ns, d = c.nreg, nrb = c.urban ? c.nreg + 1 : c.nreg, m = nrb * c.ns;
     const size_t el = lw ? lw_layer_elems(n, c.nreg) : sw_layer_elems(n, d);
-    const size_t es = lw ? lw_sweep_elems(n, m, c.nreg, nrb) : sw_sweep_elems(n, d, m, nrb, c.nreg, nrb);
     const size_t budget = be.scratch_budget_doubles();
     // column-resident path where the backend has it (1 and 2 streams): one private tile per
     // resident thread block plus one operator record per (problem, level)
@@ -408,6 +407,12 @@ struct Dispatcher {
     const bool rec = !fused && be.records_shape(c, lw, &r_op);
     // level-major staging of the per-layer arrays (ssb_stage.cuh): register-resident kernels only
     const bool stage = !fused && be.stage_supported(c);
+    // interface scratch per level: staged arrays are read by the register-resident sweeps alone (the
+    // generic ones refuse them), which keep only a_above and d_above / source_above.  This holds because
+    // every shape stage_supported() accepts has a register-resident sweep kernel; should one ever lack
+    // it, the backend refuses the generic sweeps on the smaller area instead of overrunning it.
+    const size_t es = stage ? (size_t)(lw ? fast_lw_sweep_elems(n) : fast_sw_sweep_elems(n, d))
+                            : (size_t)(lw ? lw_sweep_elems(n, m, c.nreg, nrb) : sw_sweep_elems(n, d, m, nrb, c.nreg, nrb));
     size_t stage_elems = 0;
     if (stage) {
       ClassArgs probe = a;

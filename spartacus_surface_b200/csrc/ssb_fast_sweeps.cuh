@@ -4,8 +4,9 @@
 // Same recurrences and outputs as column_sweeps_sw/_lw of ssb_solver.cuh
 // (radsurf_urban_sw.F90:591-984, radsurf_urban_lw.F90:552-858 and the forest
 // equivalents), organised around HBM traffic, which bounds these kernels:
-//  * only a_above, d_above (or source_above) and the LU factors of the
-//    denominator I - a_above R are kept per interface; the "below" albedo
+//  * only a_above and d_above (or source_above) are kept per interface (the
+//    LU factors of the denominator I - a_above R are rebuilt in the downward
+//    pass from a_above and R, which it loads anyway); the "below" albedo
 //    matrices (which carry the extra roof region) are never formed in the
 //    downward pass - their action on a flux vector is evaluated as
 //      a_below x = R x + T D^-1 (a_above (T x))   (+ the roof block),
@@ -138,57 +139,6 @@ SSB_HDI void smv1(const Scr &S, int e0, int lev, const double *x, double *y,
       y[i] = fma(a, x[j], y[i]);
     }
   }
-}
-
-// One step of the upward adding sweep shared by SW and LW: given a_above (in
-// `st`, n x n at offset 0) and the layer's R, T in scratch, produce
-//   LU  = factors of I - a_above R           (returned in registers, stored to scratch at oLU)
-//   X   = D^-1 (a_above T)                   (n x n)
-//   Wx  = D^-1 (a_above Wa + Wb)             (n x NW extra right-hand sides supplied by the caller
-//                                             through `rhs_extra`, already holding Wb on entry;
-//                                             Wa is streamed from the layer scratch at oWa)
-template <int n, int NW, int NS, int WKIND>
-SSB_HDI void adding_core(const StateMem &st, const Scr &L, const Scr &W, int jl, int oR, int oT, int oWa, int oLU,
-                         double *LU, double *X, double *rhs_extra, const SegKeep &sk) {
-  double Aa[n * n];
-  SSB_UNROLL
-  for (int i = 0; i < n * n; ++i) Aa[i] = st(i);
-  SSB_UNROLL
-  for (int j = 0; j < n; ++j) {
-    SSB_UNROLL
-    for (int i = 0; i < n; ++i) LU[i + n * j] = (i == j) ? 1.0 : 0.0;
-    SSB_UNROLL
-    for (int k = 0; k < n; ++k) {
-      const double r = L.ldp(oR + k + n * j, jl, sk.k[seg_class<0, NS>(k, j)]);
-      SSB_UNROLL
-      for (int i = 0; i < n; ++i) LU[i + n * j] = fma(-Aa[i + n * k], r, LU[i + n * j]);
-    }
-  }
-  sm_lu<n>(LU);
-  SSB_UNROLL
-  for (int i = 0; i < n * n; ++i) W.st(oLU + i, jl, LU[i]);
-  SSB_UNROLL
-  for (int j = 0; j < n; ++j) {
-    SSB_UNROLL
-    for (int i = 0; i < n; ++i) X[i + n * j] = 0.0;
-    SSB_UNROLL
-    for (int k = 0; k < n; ++k) {
-      const double t = L.ldp(oT + k + n * j, jl, sk.k[seg_class<0, NS>(k, j)]);
-      SSB_UNROLL
-      for (int i = 0; i < n; ++i) X[i + n * j] = fma(Aa[i + n * k], t, X[i + n * j]);
-    }
-  }
-  SSB_UNROLL
-  for (int j = 0; j < NW; ++j) {
-    SSB_UNROLL
-    for (int k = 0; k < n; ++k) {
-      const double w = L.ldp(oWa + k + n * j, jl, sk.k[seg_class<WKIND, NS>(k, j)]);
-      SSB_UNROLL
-      for (int i = 0; i < n; ++i) rhs_extra[i + n * j] = fma(Aa[i + n * k], w, rhs_extra[i + n * j]);
-    }
-  }
-  sm_lu_solve_left<n, n>(LU, X);
-  sm_lu_solve_left<n, NW>(LU, rhs_extra);
 }
 
 // overlap matrices of the interface above layer jl of the column starting at packed layer il1
@@ -333,9 +283,9 @@ struct SwSweepLayout {
   static constexpr int oR = 0, oT = n * n, oIdiff = 2 * n * n, oSup = 3 * n * n, oSdn = oSup + n * d,
                        oIdd = oSdn + n * d, oE = oIdd + n * d, oIdir = oE + d * d;
   static constexpr int oGeo = oIdir + d * d;                      // geometry block (fast_prepare_level)
-  static constexpr int oAa = 0, oDa = n * n, oLU = oDa + n * d;  // interface scratch of the fast path
+  static constexpr int oAa = 0, oDa = n * n;  // interface scratch of the fast path (state_doubles per level)
   static constexpr int NRB = URBAN ? NREG + 1 : NREG, m = NRB * NS;
-  static constexpr int state_doubles = n * n + n * d;
+  static constexpr int state_doubles = fast_sw_sweep_elems(n, d);
   // block of a layer that solves only its vegetated regions (segment 2)
   static constexpr int vegNA = NREG > 1 ? n - NS : n, vegI0 = NREG > 1 ? NS : 0;
 };
@@ -420,11 +370,11 @@ SSB_HD inline void fast_column_sweeps_sw(const ClassArgs &a, int q, const StateM
     }
     double Ab[n * n], Db[n * d];
     if (NREG == 1 || seg == 0)
-      sw_up_block<Lay, NREG, NS, n, 0>(st, L, W, jl, Ab, Db);
+      sw_up_block<Lay, NREG, NS, n, 0>(st, L, jl, Ab, Db);
     else if (seg == 1)
-      sw_up_block<Lay, NREG, NS, NS, 0>(st, L, W, jl, Ab, Db);
+      sw_up_block<Lay, NREG, NS, NS, 0>(st, L, jl, Ab, Db);
     else
-      sw_up_block<Lay, NREG, NS, Lay::vegNA, Lay::vegI0>(st, L, W, jl, Ab, Db);
+      sw_up_block<Lay, NREG, NS, Lay::vegNA, Lay::vegI0>(st, L, jl, Ab, Db);
     double rb[NS], rd[NS];
     SSB_UNROLL
     for (int js = 0; js < NS; ++js) rb[js] = rd[js] = 0.0;
@@ -548,7 +498,6 @@ SSB_HD inline void fast_column_sweeps_sw(const ClassArgs &a, int q, const StateM
       if (NREG == 1 || sn == 0) {
         prefetch_block<n, n, 0>(L, Lay::oT, jl - 1);
         prefetch_block<n, n, 0>(L, Lay::oR, jl - 1);
-        prefetch_block<n, n, 0>(W, Lay::oLU, jl - 1);
       } else if (sn == 1) {
         prefetch_block<n, NS, 0>(L, Lay::oT, jl - 1);
         prefetch_block<n, NS, 0>(L, Lay::oR, jl - 1);
@@ -746,9 +695,9 @@ struct LwSweepLayout {
   static constexpr int n = NREG * NS, d = NREG;
   static constexpr int oR = 0, oT = n * n, oIF = 2 * n * n, oSrc = 3 * n * n, oIsrc = oSrc + n, oBook = oIsrc + n;
   static constexpr int oGeo = oBook + 3 * d + 1;  // geometry block (fast_prepare_level)
-  static constexpr int oAa = 0, oSa = n * n, oLU = oSa + n;
+  static constexpr int oAa = 0, oSa = n * n;
   static constexpr int NRB = URBAN ? NREG + 1 : NREG, m = NRB * NS;
-  static constexpr int state_doubles = n * n + n;
+  static constexpr int state_doubles = fast_lw_sweep_elems(n);
   static constexpr int vegNA = NREG > 1 ? n - NS : n, vegI0 = NREG > 1 ? NS : 0;
 };
 
@@ -804,11 +753,11 @@ SSB_HD inline void fast_column_sweeps_lw(const ClassArgs &a, int q, const StateM
     const int seg = (int)L.ld(Lay::oGeo + 7, jl);
     double Ab[n * n], Sb[n];
     if (NREG == 1 || seg == 0)
-      lw_up_block<Lay, NREG, NS, n, 0>(st, L, W, jl, Ab, Sb);
+      lw_up_block<Lay, NREG, NS, n, 0>(st, L, jl, Ab, Sb);
     else if (seg == 1)
-      lw_up_block<Lay, NREG, NS, NS, 0>(st, L, W, jl, Ab, Sb);
+      lw_up_block<Lay, NREG, NS, NS, 0>(st, L, jl, Ab, Sb);
     else
-      lw_up_block<Lay, NREG, NS, Lay::vegNA, Lay::vegI0>(st, L, W, jl, Ab, Sb);
+      lw_up_block<Lay, NREG, NS, Lay::vegNA, Lay::vegI0>(st, L, jl, Ab, Sb);
     double rb[NS], rs[NS];
     SSB_UNROLL
     for (int js = 0; js < NS; ++js) rb[js] = rs[js] = 0.0;

@@ -113,6 +113,10 @@ SSB_HDI int sw_sweep_elems(int n, int d, int m, int db, int nreg, int nrb) {
   return 2 * n * n + n * d + m * m + m * db + 2 * nreg * nrb;
 }
 SSB_HDI int lw_sweep_elems(int n, int m, int nreg, int nrb) { return 2 * n * n + n + m * m + m + 2 * nreg * nrb; }
+// interface scratch of the register-resident sweeps: a_above and d_above / source_above per level
+// (SwSweepLayout / LwSweepLayout::state_doubles, ssb_fast_sweeps.cuh)
+SSB_HD constexpr int fast_sw_sweep_elems(int n, int d) { return n * n + n * d; }
+SSB_HD constexpr int fast_lw_sweep_elems(int n) { return n * n + n; }
 
 #define SSB_LAY(arr, g, il) (arr[(size_t)(g) + (size_t)nspec * (size_t)(il)])
 

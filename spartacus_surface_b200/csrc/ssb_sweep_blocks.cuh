@@ -12,8 +12,9 @@
 //     a_below = R + T D^-1 a_above T = [R_AA + T_AA D_AA^-1 a_AA T_AA, 0; 0, 0]   (likewise d_below, source_below).
 // Half of the layers of the benchmark canopy are clear-only (order 2 instead of 6): with the columns of
 // a launch ordered by segment pattern the switch below is uniform per warp, and those layers execute a
-// tenth of the arithmetic of a full one instead of multiplying structural zeros.  Only the LU factors
-// of D_AA go to the interface scratch (NA^2 instead of n^2 doubles per level).
+// tenth of the arithmetic of a full one instead of multiplying structural zeros.  The LU factors of
+// D_AA never go to the interface scratch: the downward step rebuilds them from the a_AA and R_AA it
+// loads for its own products (denominator_lu), bit for bit the factors of the upward step.
 // Same recurrences as radsurf_urban_sw.F90:603-984 / radsurf_urban_lw.F90:548-858 (and the forest
 // equivalents); NA = n, I0 = 0 is the unrestricted step.
 #pragma once
@@ -47,8 +48,26 @@ SSB_HDI void interface_store_pruned(const StateMem &st, const ScrT &W, int lev) 
 // Shortwave
 // ---------------------------------------------------------------------------------------------
 // upward: Ab (n x n) = a_below street part, Db (n x d) = d_below street part (zeros outside the block)
+// D_AA = I - a_AA R_AA factored in place into LU, with the operation order of the upward steps
+// (sw_up_block / lw_up_block build the same matrix interleaved with a_AA T_AA): the downward steps
+// call this on the same a_AA and R_AA and so solve with exactly the factors of the upward step.
+template <int NA>
+SSB_HDI void denominator_lu(const double *Aa, const double *Ra, double *LU) {
+  SSB_UNROLL
+  for (int j = 0; j < NA; ++j) {
+    SSB_UNROLL
+    for (int i = 0; i < NA; ++i) LU[i + NA * j] = (i == j) ? 1.0 : 0.0;
+    SSB_UNROLL
+    for (int k = 0; k < NA; ++k) {
+      SSB_UNROLL
+      for (int i = 0; i < NA; ++i) LU[i + NA * j] = fma(-Aa[i + NA * k], Ra[k + NA * j], LU[i + NA * j]);
+    }
+  }
+  sm_lu<NA>(LU);
+}
+
 template <class Lay, int NREG, int NS, int NA, int I0, class ScrT>
-SSB_HDI void sw_up_block(const StateMem &st, const ScrT &L, const ScrT &W, int jl, double *Ab, double *Db) {
+SSB_HDI void sw_up_block(const StateMem &st, const ScrT &L, int jl, double *Ab, double *Db) {
   constexpr int n = NREG * NS, d = NREG, DA = NA / NS, R0 = I0 / NS;
   double Aa[NA * NA], X[NA * NA], Wd[NA * DA];
   SSB_UNROLL
@@ -95,8 +114,6 @@ SSB_HDI void sw_up_block(const StateMem &st, const ScrT &L, const ScrT &W, int j
       }
     }
     sm_lu<NA>(LU);
-    SSB_UNROLL
-    for (int i = 0; i < NA * NA; ++i) W.st(Lay::oLU + i, jl, LU[i]);
     sm_lu_solve_left<NA, NA>(LU, X);
     sm_lu_solve_left<NA, DA>(LU, Wd);
   }
@@ -188,12 +205,15 @@ SSB_HDI void sw_down_block(const ScrT &L, const ScrT &W, int jl, const double *x
   }
   SSB_UNROLL
   for (int i = 0; i < n; ++i) ub_d[i] = ub_f[i] = 0.0;
+  double Aa[NA * NA], Ra[NA * NA];
   SSB_UNROLL
   for (int j = 0; j < NA; ++j) {
     SSB_UNROLL
     for (int i = 0; i < NA; ++i) {
       const double a = W.ld(Lay::oAa + (I0 + i) + n * (I0 + j), jl);
       const double r = L.ld(Lay::oR + (I0 + i) + n * (I0 + j), jl);
+      Aa[i + NA * j] = a;
+      Ra[i + NA * j] = r;
       z1_d[i] = fma(a, y_d[j], z1_d[i]);
       z1_f[i] = fma(a, y_f[j], z1_f[i]);
       z2_d[i] = fma(r, refl[I0 + j], z2_d[i]);
@@ -203,8 +223,7 @@ SSB_HDI void sw_down_block(const ScrT &L, const ScrT &W, int jl, const double *x
   }
   {
     double LU[NA * NA];
-    SSB_UNROLL
-    for (int i = 0; i < NA * NA; ++i) LU[i] = W.ld(Lay::oLU + i, jl);
+    denominator_lu<NA>(Aa, Ra, LU);
     sm_lu_solve_left<NA, 1>(LU, z1_d);
     sm_lu_solve_left<NA, 1>(LU, z1_f);
     sm_lu_solve_left<NA, 1>(LU, z2_d);
@@ -313,7 +332,7 @@ SSB_HDI void sw_down_block(const ScrT &L, const ScrT &W, int jl, const double *x
 // Longwave (suffix i: internal emission pass, f: incoming-flux pass)
 // ---------------------------------------------------------------------------------------------
 template <class Lay, int NREG, int NS, int NA, int I0, class ScrT>
-SSB_HDI void lw_up_block(const StateMem &st, const ScrT &L, const ScrT &W, int jl, double *Ab, double *Sb) {
+SSB_HDI void lw_up_block(const StateMem &st, const ScrT &L, int jl, double *Ab, double *Sb) {
   constexpr int n = NREG * NS;
   double Aa[NA * NA], X[NA * NA], v1[NA], src[NA];
   SSB_UNROLL
@@ -352,8 +371,6 @@ SSB_HDI void lw_up_block(const StateMem &st, const ScrT &L, const ScrT &W, int j
       }
     }
     sm_lu<NA>(LU);
-    SSB_UNROLL
-    for (int i = 0; i < NA * NA; ++i) W.st(Lay::oLU + i, jl, LU[i]);
     sm_lu_solve_left<NA, NA>(LU, X);
     sm_lu_solve_left<NA, 1>(LU, v1);
   }
@@ -415,12 +432,15 @@ SSB_HDI void lw_down_block(const ScrT &L, const ScrT &W, int jl, const double *x
   for (int i = 0; i < n; ++i) ub_i[i] = ub_f[i] = 0.0;
   SSB_UNROLL
   for (int i = 0; i < NA; ++i) ub_i[I0 + i] = src[i];
+  double Aa[NA * NA], Ra[NA * NA];
   SSB_UNROLL
   for (int j = 0; j < NA; ++j) {
     SSB_UNROLL
     for (int i = 0; i < NA; ++i) {
       const double a = W.ld(Lay::oAa + (I0 + i) + n * (I0 + j), jl);
       const double r = L.ld(Lay::oR + (I0 + i) + n * (I0 + j), jl);
+      Aa[i + NA * j] = a;
+      Ra[i + NA * j] = r;
       z1_i[i] = fma(a, y_i[j], z1_i[i]);
       z1_f[i] = fma(a, y_f[j], z1_f[i]);
       z2_i[i] = fma(r, sa[I0 + j], z2_i[i]);
@@ -430,8 +450,7 @@ SSB_HDI void lw_down_block(const ScrT &L, const ScrT &W, int jl, const double *x
   }
   {
     double LU[NA * NA];
-    SSB_UNROLL
-    for (int i = 0; i < NA * NA; ++i) LU[i] = W.ld(Lay::oLU + i, jl);
+    denominator_lu<NA>(Aa, Ra, LU);
     sm_lu_solve_left<NA, 1>(LU, z1_i);
     sm_lu_solve_left<NA, 1>(LU, z1_f);
     sm_lu_solve_left<NA, 1>(LU, z2_i);
