@@ -393,6 +393,31 @@ int ssb200_radsurf_fluxes_device(const ssb200_config *config,
                                  ssb200_canopy_flux *sw_flux, ssb200_canopy_flux *lw_flux,
                                  void *stream, int32_t *status_out);
 
+/* ssb200_radsurf_fluxes_device for float (single-precision) HBM arrays, as a -DSINGLE_PRECISION host
+ * model holds them: every real array, the members of `driver_inputs` included, is a float DEVICE pointer;
+ * nlay, istartlay and i_representation stay HOST arrays.  Stream, ordering against other streams,
+ * `status_out`, the columns and layers written and the return convention are those of
+ * ssb200_radsurf_fluxes_device, and non-contiguous packed layers are accepted.
+ * The solve, the emission, the defaults of NULL members and the scale + sum run in FP64 on the float
+ * inputs widened exactly, and every output is rounded once to nearest float: it equals the output of
+ * ssb200_radsurf_fluxes_device on the widened inputs, cast to float, and on contiguous layouts that of
+ * ssb200_radsurf_fluxes_sp on the same arrays.  read_input's defaults, sigma T^4 and the default
+ * veg_contact_fraction are held as doubles in buffers of the context, never rounded to float.
+ * The per-column members, bc_out and the top-of-canopy fluxes are widened into double buffers of the
+ * context for the call's columns (bc_out is rounded back).  When every per-layer access of the call goes
+ * through the level-major staging (same condition as ssb200_radsurf_fluxes_device), the staging widens the
+ * per-layer inputs as it gathers them and its summing scatter rounds into sw_flux / lw_flux; otherwise
+ * the per-layer inputs of the call's packed layers are widened into double buffers too. */
+int ssb200_radsurf_fluxes_device_sp(const ssb200_config *config,
+                                    const ssb200_canopy_properties_sp *canopy_props,
+                                    const ssb200_sw_spectral_properties_sp *sw_spectral_props,
+                                    const ssb200_lw_spectral_properties_sp *lw_spectral_props,
+                                    const ssb200_driver_inputs_sp *driver_inputs,
+                                    ssb200_boundary_conds_out_sp *bc_out,
+                                    int32_t istartcol, int32_t iendcol,
+                                    ssb200_canopy_flux_sp *sw_flux, ssb200_canopy_flux_sp *lw_flux,
+                                    void *stream, int32_t *status_out);
+
 /* Number of kernels launched by this process through the library so far
  * (bench.py reports the per-step delta as `gpu_launches`). */
 int64_t ssb200_kernel_launch_count(void);

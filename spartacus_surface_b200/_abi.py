@@ -122,7 +122,8 @@ EXPORTED_SYMBOLS = [
     "ssb200_version", "ssb200_abi_sizes", "ssb200_last_error", "ssb200_device_count", "ssb200_set_device",
     "ssb200_legendre_gauss_init", "ssb200_radsurf", "ssb200_radsurf_device", "ssb200_radsurf_fluxes",
     "ssb200_radsurf_sp", "ssb200_radsurf_fluxes_sp", "ssb200_radsurf_device_sp", "ssb200_radsurf_fluxes_device",
-    "ssb200_kernel_launch_count", "ssb200_set_profiling", "ssb200_last_kernel_times_ms", "ssb200_last_kernel_counts",
+    "ssb200_radsurf_fluxes_device_sp", "ssb200_kernel_launch_count", "ssb200_set_profiling",
+    "ssb200_last_kernel_times_ms", "ssb200_last_kernel_counts",
     "ssb200_release", "ssb200_set_option", "ssb200_canopy_flux_scale_device", "ssb200_canopy_flux_sum_device",
     "ssb200_canopy_flux_check_device", "ssb200_calc_simple_spectrum_lw_device", "ssb200_measure_fp64_peak_tflops",
 ]

@@ -47,6 +47,8 @@ def _declare(lib):
     lib.ssb200_radsurf_device_sp.restype = C.c_int
     lib.ssb200_radsurf_fluxes_device.argtypes = lib.ssb200_radsurf_fluxes.argtypes + [C.c_void_p, P(C.c_int32)]
     lib.ssb200_radsurf_fluxes_device.restype = C.c_int
+    lib.ssb200_radsurf_fluxes_device_sp.argtypes = lib.ssb200_radsurf_fluxes_device.argtypes
+    lib.ssb200_radsurf_fluxes_device_sp.restype = C.c_int
     lib.ssb200_kernel_launch_count.restype = C.c_int64
     lib.ssb200_set_profiling.argtypes = [C.c_int]
     lib.ssb200_last_kernel_times_ms.argtypes = [P(C.c_double)]

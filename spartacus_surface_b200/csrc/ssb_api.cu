@@ -122,14 +122,16 @@ __global__ void k_check(ssb200_canopy_flux f, const int *nlay, const int *istart
   residual[col] = ground_net + clear + wall + roof + veg + vegair - top_net;
 }
 
-// sigma * emissivity * T^4 (emissivity NULL: 1) for elements [i0, i1) of (nspec, .) arrays, interval 1
-__global__ void k_sigma_t4(double *out, const double *emissivity, const double *temperature, int nspec, long i0,
-                           long i1) {
+// sigma * emissivity * T^4 (emissivity NULL: 1) for elements [i0, i1) of (nspec, .) arrays, interval 1.
+// T: element type of the temperatures and emissivities (float inputs are widened exactly; the output and
+// the arithmetic stay FP64, so a float caller gets the emission of the double entry on widened inputs).
+template <class T>
+__global__ void k_sigma_t4(double *out, const T *emissivity, const T *temperature, int nspec, long i0, long i1) {
   const long i = i0 + blockIdx.x * (long)blockDim.x + threadIdx.x;
   if (i >= i1) return;
-  const double t = temperature[i], t2 = t * t;
+  const double t = (double)temperature[i], t2 = t * t;
   const double sb = 5.67037321e-8;  // radtool/radiation_constants.F90:26
-  out[(size_t)nspec * i] = emissivity ? (sb * emissivity[(size_t)nspec * i]) * (t2 * t2) : sb * (t2 * t2);
+  out[(size_t)nspec * i] = emissivity ? (sb * (double)emissivity[(size_t)nspec * i]) * (t2 * t2) : sb * (t2 * t2);
 }
 
 // ---- single-precision storage variant: float <-> double on the device (ssb200_radsurf_sp) ----
@@ -176,10 +178,12 @@ __global__ void k_fill(double *p, double v, long i0, long i1) {
   const long i = i0 + blockIdx.x * (long)blockDim.x + threadIdx.x;
   if (i < i1) p[i] = v;
 }
-// read_input's default veg_contact_fraction (driver/spartacus_surface_read_input.F90:155-166)
-__global__ void k_vcf_default(double *vcf, const double *vf, const double *bf, double min_veg, long i0, long i1) {
+// read_input's default veg_contact_fraction (driver/spartacus_surface_read_input.F90:155-166); T: element
+// type of the fractions (float: widened exactly, the result stays FP64)
+template <class T>
+__global__ void k_vcf_default(double *vcf, const T *vf, const T *bf, double min_veg, long i0, long i1) {
   const long i = i0 + blockIdx.x * (long)blockDim.x + threadIdx.x;
-  if (i < i1) vcf[i] = fmin(1.0, vf[i] / fmax(min_veg, 1.0 - bf[i]));
+  if (i < i1) vcf[i] = fmin(1.0, (double)vf[i] / fmax(min_veg, 1.0 - (double)bf[i]));
 }
 __global__ void k_lay2col(const int *nlay, const int *istartlay, const int *irep, int ncol, int *lay2col) {
   const int j = blockIdx.x * blockDim.x + threadIdx.x;
@@ -193,6 +197,11 @@ __global__ void k_lay2col(const int *nlay, const int *istartlay, const int *irep
 // Non-spectral members (sunlit fractions) are summed unscaled.  Window: columns [c0, c1), layers [l0, l1);
 // a layer of the window is skipped unless a column of [c0, c1) owns it (lay2col: -1 for the layers of no
 // non-Flat column), so packed layouts whose layers are not contiguous leave other columns' layers alone.
+// R: element type of the summed object (float: ssb200_radsurf_fluxes_device_sp; the FP64 result is rounded
+// once to nearest).
+__device__ __forceinline__ void store_rounded(double *p, double v) { *p = v; }
+__device__ __forceinline__ void store_rounded(float *p, double v) { *p = __double2float_rn(v); }
+template <class R>
 __global__ void k_scale_sum(FieldList fl, const double *fa, const double *fb, const double *fb_minus,
                             const int *lay2col, int nspec, long c0, long c1, long l0, long l1) {
   const long t = blockIdx.x * (long)blockDim.x + threadIdx.x;
@@ -205,15 +214,16 @@ __global__ void k_scale_sum(FieldList fl, const double *fa, const double *fb, co
     const long col = fl.per_layer[f] ? lay2col[idx] : idx;
     if (col < c0 || col >= c1) continue;
     const double a = fl.a[f][i], b = fl.b[f][i];
+    R *p = reinterpret_cast<R *>(fl.p[f]) + i;
     if (!fl.spectral[f]) {
-      fl.p[f][i] = __dadd_rn(a, b);
+      store_rounded(p, __dadd_rn(a, b));
       continue;
     }
     const int g = (int)(i % nspec);
     const size_t k = (size_t)g + (size_t)nspec * (size_t)col;
     const double xa = fa ? __dmul_rn(fa[k], a) : a;
     const double fbk = fb_minus ? __dadd_rn(fb[k], -fb_minus[k]) : fb[k];
-    fl.p[f][i] = __dadd_rn(xa, __dmul_rn(fbk, b));
+    store_rounded(p, __dadd_rn(xa, __dmul_rn(fbk, b)));
   }
 }
 
@@ -342,7 +352,7 @@ struct CudaBackend {
   bool forked = false;
   size_t budget;
   bool layer_was_fast = false;  // the chunk's layer kernels were the register-resident ones
-  bool f32_layers = false;      // per-layer members are the caller's float arrays (ssb200_radsurf_device_sp)
+  bool f32_layers = false;      // per-layer members are the caller's float arrays (single-precision device entries)
   explicit CudaBackend(Context &c, int lane_ = 0, size_t budget_ = 0)
       : cx(c), lane(lane_), pass_lane(lane_), main_stream(c.stream), budget(budget_ ? budget_ : c.budget_doubles) {}
   // Shortwave pass on the stream of the call, longwave pass on an auxiliary stream with its own
@@ -400,6 +410,8 @@ struct CudaBackend {
     int gbits = 0;
     for (size_t ngroups = (n + (size_t)group - 1) / (size_t)group; ((size_t)1 << gbits) < ngroups; ++gbits) {
     }
+    // (the key reads building_fraction and veg_fraction only, which the driver-sequence entries never
+    // replace by a double default: with float layers they are always the caller's float arrays)
     if (f32_layers)
       k_column_keys<float><<<(unsigned)((n + 127) / 128), 128, 0, cx.stream>>>(a, keys, group, lbits);
     else
@@ -655,16 +667,17 @@ int upload_plan(Context &cx, const ssb200_canopy_properties &cp) {
 
 typedef ssb::Dispatcher<CudaBackend>::PassSum PassSum;
 
-// Runs the prepared plan on cx.stream.  f32_layers: the per-layer members of `ca` are float arrays that
-// only the level-major staging touches (ssb200_radsurf_device_sp, staged route).  sum_sw / sum_lw:
-// summing scatter of each pass (ssb200_radsurf_fluxes_device, staged route).
-int dispatch_call(Context &cx, const ssb::CallArgs &ca, bool f32_layers, const PassSum &sum_sw = PassSum(),
-                  const PassSum &sum_lw = PassSum()) {
+// Runs the prepared plan on cx.stream.  prec.f32: the per-layer members of `ca` are float arrays that
+// only the level-major staging touches (single-precision device entries, staged route), apart from the
+// double buffers in prec.f64.  sum_sw / sum_lw: summing scatter of each pass (ssb200_radsurf_fluxes_device
+// and _sp, staged route).
+int dispatch_call(Context &cx, const ssb::CallArgs &ca, const ssb::StagePrecision &prec = ssb::StagePrecision(),
+                  const PassSum &sum_sw = PassSum(), const PassSum &sum_lw = PassSum()) {
   std::string err;
   CudaBackend be(cx);
-  be.f32_layers = f32_layers;
+  be.f32_layers = prec.f32;
   ssb::Dispatcher<CudaBackend> disp(be);
-  disp.f32_layers = f32_layers;
+  disp.precision = prec;
   disp.sum_sw = sum_sw;
   disp.sum_lw = sum_lw;
   const int rc = disp.run(ca, cx.plan, err);
@@ -752,7 +765,7 @@ int radsurf_device_locked(Context &cx, const ssb::CallArgs &ca, int istartcol, i
     blocks[1] = c2;
     return 0;
   }
-  rc = dispatch_call(cx, ca, false);
+  rc = dispatch_call(cx, ca);
   if (rc) return rc;
   return finish_device_call(cx, stream, status_out);
 }
@@ -907,18 +920,38 @@ struct DriverStage {
     }
   }
   // default contact fraction and emission of columns [c0, c1) and packed layers [l0, l1); cp: the
-  // device arrays of the call
+  // caller's device arrays.  f32: the fractions, temperatures and emissivities read here are float
+  // (ssb200_radsurf_fluxes_device_sp); the results stay FP64 either way.
   void derive(const ssb200_canopy_properties &cp, double min_veg, size_t c0, size_t c1, size_t l0, size_t l1,
-              cudaStream_t st) const {
+              cudaStream_t st, bool f32 = false) const {
+    if (f32)
+      derive_as<float>(cp, min_veg, c0, c1, l0, l1, st);
+    else
+      derive_as<double>(cp, min_veg, c0, c1, l0, l1, st);
+  }
+  // the buffers of the plan: double whatever the precision of the caller's arrays
+  std::vector<const void *> buffers() const {
+    std::vector<const void *> v;
+    if (vcf) v.push_back(vcf);
+    for (const Fill &f : fills) v.push_back(f.p);
+    for (const Emis &e : emis) v.push_back(e.out);
+    return v;
+  }
+
+ private:
+  template <class T>
+  void derive_as(const ssb200_canopy_properties &cp, double min_veg, size_t c0, size_t c1, size_t l0, size_t l1,
+                 cudaStream_t st) const {
     if (vcf && l1 > l0) {
-      k_vcf_default<<<(unsigned)((l1 - l0 + 255) / 256), 256, 0, st>>>(vcf, cp.veg_fraction, cp.building_fraction,
-                                                                        min_veg, (long)l0, (long)l1);
+      k_vcf_default<T><<<(unsigned)((l1 - l0 + 255) / 256), 256, 0, st>>>(
+          vcf, (const T *)cp.veg_fraction, (const T *)cp.building_fraction, min_veg, (long)l0, (long)l1);
       ++g_launches;
     }
     for (const Emis &e : emis) {
       const long i0 = (long)(e.per_layer ? l0 : c0), i1 = (long)(e.per_layer ? l1 : c1);
       if (i1 <= i0) continue;
-      k_sigma_t4<<<(unsigned)((i1 - i0 + 255) / 256), 256, 0, st>>>(e.out, e.emissivity, e.temperature, 1, i0, i1);
+      k_sigma_t4<T><<<(unsigned)((i1 - i0 + 255) / 256), 256, 0, st>>>(e.out, (const T *)e.emissivity,
+                                                                         (const T *)e.temperature, 1, i0, i1);
       ++g_launches;
     }
   }
@@ -1199,16 +1232,18 @@ static int radsurf_device_sp_locked(Context &cx, const ssb::CallArgs &ca, int32_
                     cfg.do_lw ? &d3 : nullptr, cfg.do_lw ? &d4 : nullptr};
   Drain drain{stream};
   if ((rc = convert_arrays(conv, false, stream))) return rc;
-  if ((rc = dispatch_call(cx, wca, staged))) return rc;
+  ssb::StagePrecision prec;
+  prec.f32 = staged;
+  if ((rc = dispatch_call(cx, wca, prec))) return rc;
   if ((rc = convert_arrays(conv, true, stream))) return rc;
   drain.armed = false;
   return finish_device_call(cx, stream, status_out);
 }
 
-// Body of ssb200_radsurf_fluxes_device: the sequence of radsurf_host with drv != NULL on device arrays.
-// Inputs the caller leaves NULL are filled in context buffers (read_input's defaults, sigma T^4 from the
-// temperatures) over the call's columns and packed layers.  The four normalised flux objects take one of
-// two routes, chosen per call from the plan:
+// Body of ssb200_radsurf_fluxes_device and, with sp, ssb200_radsurf_fluxes_device_sp: the sequence of
+// radsurf_host with drv != NULL on device arrays.  Inputs the caller leaves NULL are filled in context
+// buffers (read_input's defaults, sigma T^4 from the temperatures) over the call's columns and packed layers.
+// The four normalised flux objects take one of two routes, chosen per call from the plan:
 //   staged:   every per-layer write goes through the level-major staging, whose scatter writes
 //             fa * f1 + fb * f2 straight into sw_flux / lw_flux (StageList::sum): the per-layer members of
 //             the normalised objects exist in the staging buffers of a chunk only.  Their per-column
@@ -1218,16 +1253,26 @@ static int radsurf_device_sp_locked(Context &cx, const ssb::CallArgs &ca, int32_
 //             the four objects are materialised in zeroed context buffers for the call's columns and
 //             layers, and scaled and summed per column and per owned layer after the solve.
 // Both give the bits of ssb200_radsurf_fluxes: the same products and sums, each rounded once.
+// sp: every real array of the caller, driver_inputs included, holds float.  The defaults, the emission
+// and the default contact fraction stay in double context buffers, computed from the float inputs widened
+// exactly.  The caller's per-column members, bc_out and the top-of-canopy fluxes are widened into context
+// buffers for the call's columns (bc_out is rounded back after the solve).  On the staged route the
+// staging widens the caller's per-layer inputs and its summing scatter rounds into the float summed
+// objects; on the fallback route the per-layer inputs are widened over the call's layers.  Either way the
+// scale + sum rounds the FP64 result once into the summed objects, so every output is the double entry's
+// on widened inputs, rounded to nearest.
 static int radsurf_fluxes_device_locked(Context &cx, const ssb200_config *config, const ssb200_canopy_properties *cp,
                                         const ssb200_sw_spectral_properties *sw, const ssb200_lw_spectral_properties *lw,
                                         const ssb200_driver_inputs *drv, ssb200_boundary_conds_out *bc,
                                         int32_t istartcol, int32_t iendcol, ssb200_canopy_flux *sw_flux,
-                                        ssb200_canopy_flux *lw_flux, cudaStream_t stream, int32_t *status_out) {
+                                        ssb200_canopy_flux *lw_flux, cudaStream_t stream, int32_t *status_out,
+                                        bool sp = false) {
+  const char *name = sp ? "radsurf_fluxes_device_sp" : "radsurf_fluxes_device";
   if (!config || !cp || !bc || !drv)
     return fail(SSB200_ERR_ARG, "config, canopy_props, driver_inputs and bc_out must not be NULL");
   if ((config->do_sw && (!sw_flux || !drv->top_flux_dn_sw || !drv->top_flux_dn_direct_sw)) ||
       (config->do_lw && (!lw_flux || !drv->top_flux_dn_lw)))
-    return fail(SSB200_ERR_ARG, "radsurf_fluxes_device: flux object or top-of-canopy flux missing");
+    return fail(SSB200_ERR_ARG, std::string(name) + ": flux object or top-of-canopy flux missing");
   {
     ssb::CallArgs probe{config, cp, sw, lw, bc, sw_flux, sw_flux, lw_flux, lw_flux};
     std::string err;
@@ -1246,6 +1291,7 @@ static int radsurf_fluxes_device_locked(Context &cx, const ssb200_config *config
   ssb200_canopy_properties dcp = *cp;
   ssb200_sw_spectral_properties dsw;
   ssb200_lw_spectral_properties dlw;
+  ssb200_boundary_conds_out dbc = *bc;
   memset(&dsw, 0, sizeof(dsw));
   memset(&dlw, 0, sizeof(dlw));
   if (config->do_sw) dsw = *sw;
@@ -1255,7 +1301,7 @@ static int radsurf_fluxes_device_locked(Context &cx, const ssb200_config *config
   if (rc) return rc;
   // plan, argument checks, ordering against the previous call, status reset (the summed objects stand in
   // for the normalised ones, whose shape they have)
-  ssb::CallArgs ca{config, &dcp, config->do_sw ? &dsw : nullptr, config->do_lw ? &dlw : nullptr, bc,
+  ssb::CallArgs ca{config, &dcp, config->do_sw ? &dsw : nullptr, config->do_lw ? &dlw : nullptr, &dbc,
                    sw_flux, sw_flux, lw_flux, lw_flux};
   int range[2] = {1, 0};
   rc = radsurf_device_locked(cx, ca, c1, c2, stream, nullptr, range);
@@ -1263,6 +1309,44 @@ static int radsurf_fluxes_device_locked(Context &cx, const ssb200_config *config
   CudaBackend probe(cx);
   ssb::Dispatcher<CudaBackend> route(probe);
   const bool staged = route.all_layers_staged(ca, cx.plan);
+  ssb::StagePrecision prec;  // (the staging reaches the caller's float arrays on the staged route only)
+  prec.f32 = sp && staged;
+  prec.f64 = ds.buffers();
+  // sp: double copies of the caller's float arrays, widened over rows [r0, r1) before the solve; `out`
+  // ones (bc_out) are rounded back after it
+  std::vector<ConvArray> conv;
+  auto wide = [&](const void *p, size_t rows, size_t width, size_t r0, size_t r1, bool out) -> double * {
+    if (!p) return nullptr;
+    double *d = pool.get<double>(rows * width);
+    if (d) conv.push_back(ConvArray{(float *)p, d, (long)(r0 * width), (long)(r1 * width), out});
+    return d;
+  };
+  // the caller's members of `d`: per-column ones over the call's columns; per-layer ones over its layers on
+  // the fallback route (the staging widens them on the staged route).  DriverStage's buffers are double.
+  auto widen = [&](auto &d, const auto &table, size_t nspec) {
+    for (const auto &m : table) {
+      auto &member = d.*m.ptr;
+      if (!member || (m.per_layer && staged)) continue;
+      if (std::find(prec.f64.begin(), prec.f64.end(), (const void *)member) != prec.f64.end()) continue;
+      const size_t w = ssb::member_width(m, nspec);
+      member = m.per_layer ? wide(member, ntot, w, l0, lN, false) : wide(member, ncol, w, c0, cN, false);
+    }
+  };
+  const double *top_sw = drv->top_flux_dn_sw, *top_dir = drv->top_flux_dn_direct_sw, *top_lw = drv->top_flux_dn_lw;
+  if (sp) {
+    widen(dcp, ssb::kCanopyMembers, 1);
+    if (config->do_sw) widen(dsw, ssb::kSwMembers, (size_t)config->nsw);
+    if (config->do_lw) widen(dlw, ssb::kLwMembers, (size_t)config->nlw);
+    for (const ssb::BcMember &m : ssb::kBcMembers)
+      dbc.*m.ptr = (m.lw ? config->do_lw : config->do_sw)
+                       ? wide(bc->*m.ptr, ncol, (size_t)(m.lw ? config->nlw : config->nsw), c0, cN, true)
+                       : nullptr;
+    if (config->do_sw) {
+      top_sw = wide(top_sw, ncol, (size_t)config->nsw, c0, cN, false);
+      top_dir = wide(top_dir, ncol, (size_t)config->nsw, c0, cN, false);
+    }
+    if (config->do_lw) top_lw = wide(top_lw, ncol, (size_t)config->nlw, c0, cN, false);
+  }
   // the normalised objects: context buffers shaped like the summed object, zeroed over the call's window
   // (canopy_flux_type%zero_all, driver:184).  Staged route: per-column members only; the per-layer members
   // keep the summed object's pointers, which only mark them present (stage_plan redirects them).
@@ -1282,32 +1366,34 @@ static int radsurf_fluxes_device_locked(Context &cx, const ssb200_config *config
   if (config->do_sw) {
     normalised(sw_flux, d1);
     normalised(sw_flux, d2);
-    sum_sw.fa = drv->top_flux_dn_direct_sw;
-    sum_sw.fb = drv->top_flux_dn_sw;
-    sum_sw.fb_minus = drv->top_flux_dn_direct_sw;
+    sum_sw.fa = top_dir;
+    sum_sw.fb = top_sw;
+    sum_sw.fb_minus = top_dir;
     if (staged) sum_sw.out = sw_flux;
   }
   if (config->do_lw) {
     normalised(lw_flux, d3);
     normalised(lw_flux, d4);
-    sum_lw.fb = drv->top_flux_dn_lw;
+    sum_lw.fb = top_lw;
     if (staged) sum_lw.out = lw_flux;
   }
   if (pool.rc) return pool.rc;
-  const ssb::CallArgs nca{config, &dcp, ca.sw, ca.lw, bc, config->do_sw ? &d1 : nullptr, config->do_sw ? &d2 : nullptr,
+  const ssb::CallArgs nca{config, &dcp, ca.sw, ca.lw, &dbc, config->do_sw ? &d1 : nullptr, config->do_sw ? &d2 : nullptr,
                           config->do_lw ? &d3 : nullptr, config->do_lw ? &d4 : nullptr};
   Drain drain{stream};
   CudaBackend be(cx);  // (profiling: the stages around the solve are booked with family 4)
   be.tick(4, true);
+  if ((rc = convert_arrays(conv, false, stream))) return rc;
   ds.fill(l0, lN, stream);
-  ds.derive(dcp, config->min_vegetation_fraction, c0, cN, l0, lN, stream);
+  ds.derive(*cp, config->min_vegetation_fraction, c0, cN, l0, lN, stream, sp);
   for (const auto &z : zeroed)
     if (z.second > 0) SSB_CUDA(cudaMemsetAsync(z.first, 0, z.second * sizeof(double), stream));
   SSB_CUDA(cudaGetLastError());
   be.tick(4, false);
-  if ((rc = dispatch_call(cx, nca, false, sum_sw, sum_lw))) return rc;
+  if ((rc = dispatch_call(cx, nca, prec, sum_sw, sum_lw))) return rc;
   // scale + sum (driver:250-261) of what the solve left in the normalised objects: the per-column members
-  // (staged route), or every member over the call's columns and owned layers (fallback route)
+  // (staged route), or every member over the call's columns and owned layers (fallback route), rounded
+  // once into float summed objects (sp)
   if (!staged && (rc = ensure_lay2col(cx, ncol, ntot, stream))) return rc;
   const long cnt = (long)std::max(cN - c0, staged ? (size_t)0 : lN - l0);
   auto scale_sum = [&](ssb200_canopy_flux *o, const ssb200_canopy_flux &x, const ssb200_canopy_flux &y,
@@ -1316,14 +1402,19 @@ static int radsurf_fluxes_device_locked(Context &cx, const ssb200_config *config
     collect_fields(o, &x, &y, fl, true, !staged);
     const long nthr = cnt * nspec;
     if (fl.n == 0 || nthr <= 0) return;
-    k_scale_sum<<<(unsigned)((nthr + 255) / 256), 256, 0, stream>>>(fl, fa, fb, fbm, (const int *)cx.d_lay2col.p,
-                                                                     nspec, (long)c0, (long)cN, (long)l0, (long)lN);
+    const unsigned blocks = (unsigned)((nthr + 255) / 256);
+    const int *lay2col = (const int *)cx.d_lay2col.p;
+    if (sp)
+      k_scale_sum<float><<<blocks, 256, 0, stream>>>(fl, fa, fb, fbm, lay2col, nspec, (long)c0, (long)cN, (long)l0, (long)lN);
+    else
+      k_scale_sum<double><<<blocks, 256, 0, stream>>>(fl, fa, fb, fbm, lay2col, nspec, (long)c0, (long)cN, (long)l0, (long)lN);
     ++g_launches;
   };
   be.tick(4, true);
   if (config->do_sw) scale_sum(sw_flux, d1, d2, sum_sw.fa, sum_sw.fb, sum_sw.fb_minus, config->nsw);
   if (config->do_lw) scale_sum(lw_flux, d3, d4, nullptr, sum_lw.fb, nullptr, config->nlw);
   SSB_CUDA(cudaGetLastError());
+  if ((rc = convert_arrays(conv, true, stream))) return rc;
   be.tick(4, false);
   drain.armed = false;
   return finish_device_call(cx, stream, status_out);
@@ -1532,7 +1623,7 @@ static int radsurf_host(const ssb200_config *config, const ssb200_canopy_propert
         collect_fields(&o, &x, &y, fl, true);
         const long nthr = cnt * nspec;
         if (fl.n == 0 || nthr <= 0) return;
-        k_scale_sum<<<(unsigned)((nthr + 255) / 256), 256, 0, s_run>>>(fl, fa, fb, fbm, (const int *)cx.d_lay2col.p, nspec,
+        k_scale_sum<double><<<(unsigned)((nthr + 255) / 256), 256, 0, s_run>>>(fl, fa, fb, fbm, (const int *)cx.d_lay2col.p, nspec,
                                                                        (long)cb0, (long)cb1, (long)lb0, (long)lb1);
         ++g_launches;
       };
@@ -1638,6 +1729,25 @@ int ssb200_radsurf_fluxes_device(const ssb200_config *config, const ssb200_canop
   std::lock_guard<std::mutex> lock(g_mutex);
   return radsurf_fluxes_device_locked(g_ctx, config, canopy_props, sw, lw, driver_inputs, bc_out, istartcol, iendcol,
                                       sw_flux, lw_flux, (cudaStream_t)stream, status_out);
+}
+
+int ssb200_radsurf_fluxes_device_sp(const ssb200_config *config, const ssb200_canopy_properties_sp *canopy_props,
+                                    const ssb200_sw_spectral_properties_sp *sw,
+                                    const ssb200_lw_spectral_properties_sp *lw,
+                                    const ssb200_driver_inputs_sp *driver_inputs, ssb200_boundary_conds_out_sp *bc_out,
+                                    int32_t istartcol, int32_t iendcol, ssb200_canopy_flux_sp *sw_flux,
+                                    ssb200_canopy_flux_sp *lw_flux, void *stream, int32_t *status_out) {
+  int rc = ensure_device();
+  if (rc) return rc;
+  std::lock_guard<std::mutex> lock(g_mutex);
+  return radsurf_fluxes_device_locked(g_ctx, config, reinterpret_cast<const ssb200_canopy_properties *>(canopy_props),
+                                      reinterpret_cast<const ssb200_sw_spectral_properties *>(sw),
+                                      reinterpret_cast<const ssb200_lw_spectral_properties *>(lw),
+                                      reinterpret_cast<const ssb200_driver_inputs *>(driver_inputs),
+                                      reinterpret_cast<ssb200_boundary_conds_out *>(bc_out), istartcol, iendcol,
+                                      reinterpret_cast<ssb200_canopy_flux *>(sw_flux),
+                                      reinterpret_cast<ssb200_canopy_flux *>(lw_flux), (cudaStream_t)stream, status_out,
+                                      true);
 }
 
 int64_t ssb200_kernel_launch_count(void) { return (int64_t)g_launches; }
@@ -1844,7 +1954,7 @@ int ssb200_calc_simple_spectrum_lw_device(ssb200_lw_spectral_properties *lw, int
     double *out = const_cast<double *>(out_c);
     if (!temp || i1 <= i0) return 0;
     if (!out || (need_emis && !emis)) return fail(SSB200_ERR_ARG, "temperature given but emission / emissivity array missing");
-    k_sigma_t4<<<(unsigned)((i1 - i0 + 255) / 256), 256, 0, st>>>(out, emis, temp, lw->nspec, i0, i1);
+    k_sigma_t4<double><<<(unsigned)((i1 - i0 + 255) / 256), 256, 0, st>>>(out, emis, temp, lw->nspec, i0, i1);
     ++g_launches;
     SSB_CUDA(cudaGetLastError());
     return 0;

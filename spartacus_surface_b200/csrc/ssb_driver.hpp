@@ -125,13 +125,25 @@ inline size_t member_width(const M &m, size_t nspec) {
   return m.spectral ? nspec : 1;
 }
 
+// Element type of the caller-side arrays that a pass stages, decided per array.  f32: the caller's arrays
+// hold float (ssb200_radsurf_device_sp, ssb200_radsurf_fluxes_device_sp).  The buffers listed in `f64` hold
+// double all the same: the context buffers the driver-sequence entries put in place of NULL members
+// (read_input's defaults, sigma T^4, the default contact fraction), which stay FP64 so that the single-
+// precision entry computes the bits of its double twin.
+struct StagePrecision {
+  bool f32 = false;
+  std::vector<const void *> f64;
+  bool is_f32(const void *p) const { return f32 && std::find(f64.begin(), f64.end(), p) == f64.end(); }
+};
+
 // Lists the per-layer arrays of a pass and redirects the members of `b` to their level-major staging
 // buffers (ssb_stage.cuh), carved from `cursor` (NULL: only count).  Returns doubles per (level, column).
-// f32: the members of `b` are the caller's float arrays (ssb200_radsurf_device_sp).
-// sum: summing scatter (ssb200_radsurf_fluxes_device): both normalised objects f1 and f2 are still staged
-// (the kernels write both), and `out` pairs the staging buffers of each member with that member of *sum.
+// prec: element type of each listed array, from its address before the redirection.
+// sum: summing scatter (ssb200_radsurf_fluxes_device and _sp): both normalised objects f1 and f2 are still
+// staged (the kernels write both), and `out` pairs the staging buffers of each member with that member of
+// *sum, which takes the summed object's precision.
 inline size_t stage_plan(ClassArgs &b, bool lw, size_t per_elem, double *cursor, StageList *in, StageList *out,
-                         bool f32 = false, const ssb200_canopy_flux *sum = nullptr) {
+                         const StagePrecision &prec = StagePrecision(), const ssb200_canopy_flux *sum = nullptr) {
   size_t elems = 0;
   // stages `member` (listed in `list` unless NULL); returns its staging buffer
   auto add = [&](StageList *list, double *&member, int ns) -> double * {
@@ -144,7 +156,7 @@ inline size_t stage_plan(ClassArgs &b, bool lw, size_t per_elem, double *cursor,
       list->staged[list->n] = cursor;
       list->staged2[list->n] = nullptr;
       list->nspec[list->n] = ns;
-      list->f32[list->n] = f32 ? 1 : 0;
+      list->f32[list->n] = prec.is_f32(member) ? 1 : 0;
       list->sum[list->n] = kSumNone;
       ++list->n;
     }
@@ -178,7 +190,7 @@ inline size_t stage_plan(ClassArgs &b, bool lw, size_t per_elem, double *cursor,
     out->staged[out->n] = sa;
     out->staged2[out->n] = sb;
     out->nspec[out->n] = w;
-    out->f32[out->n] = 0;
+    out->f32[out->n] = prec.is_f32(sum->*m.ptr) ? 1 : 0;
     out->sum[out->n] = m.spectral ? kSumScaled : kSumPlain;
     ++out->n;
   }
@@ -342,10 +354,11 @@ struct Dispatcher {
   // optional window of global column indices [col_lo, col_hi): lets the host entry
   // pipeline transfers and kernels over blocks of columns without rebuilding the plan
   int col_lo = 0, col_hi = 0x7fffffff;
-  // the per-layer members of the call are the caller's float arrays, read and written through the
-  // level-major staging only (ssb200_radsurf_device_sp; see all_layers_staged)
-  bool f32_layers = false;
-  // summing scatter of each pass (ssb200_radsurf_fluxes_device; only valid when all_layers_staged holds):
+  // element type of the staged arrays: precision.f32 when the per-layer members of the call are the
+  // caller's float arrays, read and written through the level-major staging only (the single-precision
+  // device entries; see all_layers_staged), except the double buffers listed in precision.f64
+  StagePrecision precision;
+  // summing scatter of each pass (ssb200_radsurf_fluxes_device and _sp; only valid when all_layers_staged holds):
   // the per-layer members of f1 and f2 exist in the staging buffers of a chunk only, and the scatter
   // writes their scaled sum into `out`.  The per-column members are left to the caller.
   struct PassSum {
@@ -474,7 +487,7 @@ struct Dispatcher {
         double *cursor = a.sweep + (rec ? scratch_doubles((size_t)r_op, (size_t)lmax, width)
                                         : scratch_doubles(es, (size_t)lmax + 1, width));
         const PassSum &ps = lw ? sum_lw : sum_sw;
-        stage_plan(b, lw, (size_t)lmax * cnt, cursor, &sin.list, &sout.list, f32_layers, ps.out);
+        stage_plan(b, lw, (size_t)lmax * cnt, cursor, &sin.list, &sout.list, precision, ps.out);
         sin.fa = sin.fb = sin.fb_minus = nullptr;
         sout.fa = ps.fa;
         sout.fb = ps.fb;

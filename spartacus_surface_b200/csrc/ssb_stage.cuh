@@ -22,11 +22,13 @@ struct StageList {
   double *ref[kStageMaxArrays];     // the caller's array, reference layout (inputs are not written)
   double *staged[kStageMaxArrays];  // [lev][ic][g] buffer of the chunk
   int nspec[kStageMaxArrays];
-  // 1: `ref` really holds float (ssb200_radsurf_device_sp): the gather widens exactly, the scatter
-  // rounds to nearest, so the kernels see the same doubles as the double entry on widened inputs
+  // 1: `ref` really holds float (ssb200_radsurf_device_sp, ssb200_radsurf_fluxes_device_sp): the gather
+  // widens exactly, the scatter rounds to nearest, so the kernels see the same doubles as the double entry
+  // on widened inputs.  Set per array: one list may mix the caller's float arrays with double buffers.
   unsigned char f32[kStageMaxArrays];
-  // summing scatter (ssb200_radsurf_fluxes_device): `ref` is a member of the summed flux object and
-  // receives a combination of `staged` (the member of f1) and `staged2` (the same member of f2).
+  // summing scatter (ssb200_radsurf_fluxes_device and _sp): `ref` is a member of the summed flux object and
+  // receives a combination of `staged` (the member of f1) and `staged2` (the same member of f2), summed in
+  // FP64 and, when f32 is set, rounded once to float.
   // kSumScaled: fa * a + (fb - fb_minus) * b per (interval, column); kSumPlain: a + b (sunlit fractions)
   unsigned char sum[kStageMaxArrays];
   double *staged2[kStageMaxArrays];
@@ -70,7 +72,11 @@ inline void stage_host(const StageArgs &s, bool scatter) {
           const size_t si = (size_t)g + (size_t)ns * ((size_t)ic + (size_t)lev * (size_t)s.ncols);
           double &t = s.list.staged[k][si];
           if (s.list.sum[k]) {  // (scatter only)
-            s.list.ref[k][ri] = stage_sum(s, k, t, s.list.staged2[k][si], (size_t)g + (size_t)ns * (size_t)col);
+            const double v = stage_sum(s, k, t, s.list.staged2[k][si], (size_t)g + (size_t)ns * (size_t)col);
+            if (s.list.f32[k])
+              reinterpret_cast<float *>(s.list.ref[k])[ri] = (float)v;  // round to nearest even
+            else
+              s.list.ref[k][ri] = v;
           } else if (s.list.f32[k]) {
             float &r = reinterpret_cast<float *>(s.list.ref[k])[ri];
             if (scatter)
@@ -190,9 +196,16 @@ __global__ void __launch_bounds__(kStageBlock) k_stage1(StageArgs s) {
         for (int j = 0; j < 4; ++j)
           if (j < cnt) stg[j * pitch] = v[j];
       } else {
+        if constexpr (SUM) {  // summed in FP64, then rounded once
+          const double *stg2 = s.list.staged2[k] + sbase;
 #pragma unroll
-        for (int j = 0; j < 4; ++j)
-          if (j < cnt) v[j] = __ldcs(stg + j * pitch);
+          for (int j = 0; j < 4; ++j)
+            if (j < cnt) v[j] = stage_sum(s, k, __ldcs(stg + j * pitch), __ldcs(stg2 + j * pitch), (size_t)col);
+        } else {
+#pragma unroll
+          for (int j = 0; j < 4; ++j)
+            if (j < cnt) v[j] = __ldcs(stg + j * pitch);
+        }
         if (vec4) {
           __stcs((float4 *)ref, make_float4(__double2float_rn(v[0]), __double2float_rn(v[1]), __double2float_rn(v[2]),
                                             __double2float_rn(v[3])));
@@ -279,8 +292,8 @@ inline void stage_launch(const StageArgs &s, bool scatter, cudaStream_t st, long
         ++g.list.n;
         done[k] = 1;
       }
-    if (sum)  // (double caller side only: ssb200_radsurf_fluxes_device)
-      stage_launch_group<true, double, true>(g, ns, st);
+    if (sum)  // (ssb200_radsurf_fluxes_device / _sp: the summed object's precision)
+      f32 ? stage_launch_group<true, float, true>(g, ns, st) : stage_launch_group<true, double, true>(g, ns, st);
     else if (f32)
       scatter ? stage_launch_group<true, float>(g, ns, st) : stage_launch_group<false, float>(g, ns, st);
     else

@@ -3,7 +3,8 @@
 Same argument list and meaning as the reference subroutine; the body is the
 B200 library (ssb200_radsurf for host arrays, ssb200_radsurf_device when the
 members are torch CUDA tensors; radsurf_fluxes likewise picks ssb200_radsurf_fluxes or
-ssb200_radsurf_fluxes_device; the _sp wrappers below take float32 arrays).  The reference aborts on error
+ssb200_radsurf_fluxes_device; the _sp wrappers below take float32 arrays and pick the host or device
+single-precision entry the same way).  The reference aborts on error
 (utilities/radiation_io.F90:46-54); here errors raise RadsurfError.
 """
 import ctypes as C
@@ -222,27 +223,38 @@ def radsurf_sp(config, canopy_props, sw_spectral_props, lw_spectral_props, bc_ou
 def radsurf_fluxes_sp(config, canopy_props, sw_spectral_props, lw_spectral_props, bc_out, istartcol=None,
                       iendcol=None, sw_flux=None, lw_flux=None, top_flux_dn_sw=None, top_flux_dn_direct_sw=None,
                       top_flux_dn_lw=None, ground_temperature=None, roof_temperature=None, wall_temperature=None,
-                      clear_air_temperature=None, veg_temperature=None, veg_air_temperature=None):
-    """radsurf_fluxes for single-precision (float32) host arrays: ssb200_radsurf_fluxes_sp.  Same arguments
-    and defaults as radsurf_fluxes; every real member, top-of-canopy flux and temperature must be a float32
-    numpy array.  The arrays cross PCIe as float32, the solve, emission and scale + sum run in FP64 and
-    every output is the FP64 result rounded to float32."""
+                      clear_air_temperature=None, veg_temperature=None, veg_air_temperature=None, stream=None):
+    """radsurf_fluxes for single-precision (float32) arrays.  Same arguments and defaults as radsurf_fluxes;
+    every real member, top-of-canopy flux and temperature must be float32.  numpy arrays:
+    ssb200_radsurf_fluxes_sp (the arrays cross PCIe as float32).  torch CUDA tensors:
+    ssb200_radsurf_fluxes_device_sp, enqueued on `stream` (cudaStream_t as an int, None = default stream)
+    without synchronising.  The solve, emission and scale + sum run in FP64 and every output is the FP64
+    result rounded to float32.  A mix of numpy arrays and tensors, or a float64 member, raises RadsurfError."""
     from . import _abi
     lib = load()
-    ptr = f32_ptr(False, "radsurf_fluxes_sp")
+    keep = (top_flux_dn_sw, top_flux_dn_direct_sw, top_flux_dn_lw, ground_temperature, roof_temperature,
+            wall_temperature, clear_air_temperature, veg_temperature, veg_air_temperature)
     members = list(_float_members(canopy_props, sw_spectral_props, lw_spectral_props, bc_out, sw_flux, lw_flux))
+    members += [a for a in keep if a is not None]
+    device = any(is_torch(v) for v in members)
+    if device and not all(is_torch(v) for v in members):
+        raise RadsurfError("radsurf_fluxes_sp: members mix numpy arrays and torch tensors")
     if not all(_is_f32(v) for v in members):
         raise RadsurfError("radsurf_fluxes_sp: every real array member must be float32")
+    ptr = f32_ptr(device, "radsurf_fluxes_sp")
     structs = marshal(config, canopy_props, sw_spectral_props, lw_spectral_props, bc_out, ptr=ptr)
-    drv = _abi.DriverInputs(*[ptr(a) for a in (top_flux_dn_sw, top_flux_dn_direct_sw, top_flux_dn_lw,
-                                               ground_temperature, roof_temperature, wall_temperature,
-                                               clear_air_temperature, veg_temperature, veg_air_temperature)])
+    drv = _abi.DriverInputs(*[ptr(a) for a in keep])
     fsw = sw_flux.as_struct(ptr) if sw_flux is not None else None
     flw = lw_flux.as_struct(ptr) if lw_flux is not None else None
     s = structs
-    rc = lib.ssb200_radsurf_fluxes_sp(_ref(s["config"]), _ref(s["canopy"]), _ref(s["sw"]), _ref(s["lw"]),
-                                      C.byref(drv), _ref(s["bc"]), int(istartcol or 0), int(iendcol or 0),
-                                      _ref(fsw), _ref(flw))
+    args = (_ref(s["config"]), _ref(s["canopy"]), _ref(s["sw"]), _ref(s["lw"]), C.byref(drv), _ref(s["bc"]),
+            int(istartcol or 0), int(iendcol or 0), _ref(fsw), _ref(flw))
+    if device:
+        name = "ssb200_radsurf_fluxes_device_sp"
+        rc = lib.ssb200_radsurf_fluxes_device_sp(*args, C.c_void_p(stream or 0), None)
+    else:
+        name = "ssb200_radsurf_fluxes_sp"
+        rc = lib.ssb200_radsurf_fluxes_sp(*args)
     if rc < 0:
-        raise RadsurfError(f"ssb200_radsurf_fluxes_sp failed (rc={rc}): {last_error()}")
+        raise RadsurfError(f"{name} failed (rc={rc}): {last_error()}")
     return rc
